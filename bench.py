@@ -59,7 +59,14 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="N>1: skip the replica-checksum / averaged-gradient-vs-oracle block")
     ap.add_argument("--concurrent-hvp", action="store_true", help="run the two finite-difference passes of the Hessian-vector product as two graph branches (model | twin); measured 2 % slower than one after the other on B200, so off by default")
     ap.add_argument("--no-overlap", action="store_true", help="keep the weight-grad jobs on the main stream")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (loss, "
+                    "alphas / betas, BatchNorm running statistics, a fixed sample of the weights) as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200 only: the reference arm's CPU path is not the timed GPU path")
+    return a
 
 
 def workload(a, n):
@@ -100,6 +107,28 @@ def synth_batch(seed, B, V, img):
     qst[:, 0] = 2
     lbl = torch.randint(0, 1000, (B,), generator=g)
     return image, qst, lbl
+
+
+DUMP_WEIGHT_SAMPLE = 1 << 22        # 16 MB of float32; all weights are ~95 MB at V = 17858
+
+
+def dump_outputs(path, model, loss):
+    """What the timed step hands its caller, as float32 .npy files under `path`: the loss of the last step and the state
+    that step left behind (alphas / betas, BatchNorm running statistics, weights).  The weights are a sample: positions drawn
+    with a fixed seed from all parameters concatenated in model.parameters() order, so equal shapes give equal positions.
+    The inputs are seeded, but the kernels reduce BatchNorm sums and split-K products with atomics: two runs of one build
+    agree to that rounding as it grows over the steps, not bit for bit."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    with torch.no_grad():
+        out = {"loss": loss.reshape(1)}
+        out.update(zip(("alphas_normal", "alphas_reduce", "betas_normal", "betas_reduce"), model.arch_parameters()))
+        out["bn_running_stats"] = torch.cat([b.reshape(-1) for b in model.buffers() if b.is_floating_point()])
+        flat = torch.cat([p.reshape(-1) for p in model.parameters()])
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_WEIGHT_SAMPLE].sort().values
+        out["weights_sample"] = flat[idx.to(flat.device)]
+        for name, t in out.items():
+            np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -290,11 +319,13 @@ def run_b200(a):
         from search import GraphedSearchStep
         graphed = GraphedSearchStep(stepper, train, valid, 1e-3, unrolled=unrolled)
 
+    last_loss = [None]
+
     def step_resident():
         if graphed is not None:
-            graphed()
+            last_loss[0] = graphed()
         else:
-            stepper.step(train, valid, 1e-3, unrolled=unrolled)
+            last_loss[0] = stepper.step(train, valid, 1e-3, unrolled=unrolled)
 
     def step_e2e():
         if graphed is not None:
@@ -311,11 +342,13 @@ def run_b200(a):
     l0 = lib.pcd_launch_count()
     ms = timed(step_resident, a.steps)
     launches = lib.pcd_launch_count() - l0
+    clk = clocks.stop() if rank == 0 else None      # the clock record covers the timed steps only
+    if a.dump_outputs and rank == 0:        # before anything below steps the model again
+        dump_outputs(a.dump_outputs, model, last_loss[0])
     if graphed is not None:      # replays do not pass through the host launcher: count one eager step instead
         l0 = lib.pcd_launch_count()
         stepper.step(train, valid, 1e-3, unrolled=unrolled)
         launches = (lib.pcd_launch_count() - l0) * a.steps
-    clk = clocks.stop() if rank == 0 else None
     value = world * a.steps / (ms / 1e3)
 
     step_e2e()

@@ -1,6 +1,5 @@
 """Stand-alone candidate operations (SURVEY.md §8f-4) — the op kernels' SOURCES compiled with -DPCD_EMU, against the same
 layers in stock torch at float64, plus the pin of that stock path to the reference's own modules."""
-import os
 import sys
 
 import pytest
@@ -50,35 +49,64 @@ def test_unsupported_ops_raise():
         OPS["dil_conv_3x3"](8, 1, True).eval()(torch.randn(1, 8, 8, 8))    # eval-mode BatchNorm is out of scope
 
 
-REF = "/root/reference/darts_vqa"
+_STOCK_MIXED = {}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree only exists in the development container")
-@pytest.mark.parametrize("name,C,stride", [("sep_conv_3x3", 8, 2), ("sep_conv_5x5", 8, 1), ("sep_conv_7x7", 4, 1), ("dil_conv_3x3", 8, 1),
-                                           ("dil_conv_5x5", 8, 2), ("max_pool_3x3", 4, 2), ("avg_pool_3x3", 4, 1),
-                                           ("skip_connect", 8, 2), ("skip_connect", 8, 1), ("none", 4, 2)])
-def test_stock_forward_is_the_reference_module(name, C, stride):
-    """`stock_forward` (the yardstick of the op parity tests) against the reference's OPS[name] with the same state_dict:
-    bit-equal outputs and gradients (both are the same ATen calls)."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_operations", os.path.join(REF, "pcdarts", "operations.py"))
-    ref_ops = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_ops)
-    from pcdarts.operations import OPS
-    torch.manual_seed(3)
-    mine, ref = OPS[name](C, stride, True).train(), ref_ops.OPS[name](C, stride, True).train()
-    ref.load_state_dict(mine.state_dict())
-    x1 = torch.randn(2, C, 12, 12, requires_grad=True)
-    x2 = x1.detach().clone().requires_grad_(True)
-    y1 = mine.stock_forward(x1) if hasattr(mine, "stock_forward") else mine(x1)
-    y2 = ref(x2)
-    assert torch.equal(y1, y2)
-    if y1.requires_grad:
-        gy = torch.randn_like(y1)
-        g1 = torch.autograd.grad(y1, [x1] + list(mine.parameters()), gy)
-        g2 = torch.autograd.grad(y2, [x2] + list(ref.parameters()), gy)
-        for a, b in zip(g1, g2):
-            assert torch.equal(a, b)
+def _stock_mixed(name, C, stride):
+    """MixedOp of the reference (model_search.py:44-58) composed from this repo's OPS modules' `stock_forward`, with the
+    weights, input, arch weights and output gradient its golden generator used (tests/golden/make_golden.py mixed_case).
+    One thread, like the generator: the weight-gradient sums then come out in the same order."""
+    if name not in _STOCK_MIXED:
+        import config
+        from oracle import pcdarts_oracle as O
+        from pcdarts.model_search import MixedOp
+        from helpers import load_golden
+        config.DEVICE = torch.device("cpu")
+        g = load_golden("mixed_" + name)
+        m = MixedOp(C, stride).train()
+        P._fill(m, 100 + C + stride)
+        x = g["x"].clone().requires_grad_(True)
+        w = g["w"].clone().requires_grad_(True)
+        c = C // 4
+        threads = torch.get_num_threads()
+        torch.set_num_threads(1)
+        try:
+            acc = 0
+            for k, op in enumerate(m._ops):          # python sum() order of the reference: ((0 + w0 o0) + w1 o1) + ...
+                if isinstance(op, torch.nn.Sequential):      # pool candidate + BatchNorm2d(affine=False)
+                    o = op[1](op[0].stock_forward(x[:, :c]))
+                else:
+                    o = op.stock_forward(x[:, :c]) if hasattr(op, "stock_forward") else op(x[:, :c])
+                acc = acc + w[k] * o
+            rest = x[:, c:] if stride == 1 else torch.nn.functional.max_pool2d(x[:, c:], 2, 2)
+            y = O.channel_shuffle(torch.cat([acc, rest], dim=1))
+            (y * g["G"]).sum().backward()
+        finally:
+            torch.set_num_threads(threads)
+        _STOCK_MIXED[name] = (m, y.detach(), x.grad, w.grad, g)
+    return _STOCK_MIXED[name]
+
+
+@pytest.mark.parametrize("primitive", ["none", "max_pool_3x3", "avg_pool_3x3", "skip_connect", "sep_conv_3x3", "sep_conv_5x5",
+                                       "dil_conv_3x3", "dil_conv_5x5"])
+@pytest.mark.parametrize("name,C,stride", P.MIXED)
+def test_stock_forward_is_the_reference_module(name, C, stride, primitive):
+    """`stock_forward` (the yardstick of the op parity tests) against what the reference's own OPS[primitive] modules computed
+    inside its MixedOp (tests/golden/mixed_*.npz): the MixedOp output and input / arch-weight gradients, and this primitive's
+    weight gradients and BatchNorm buffers.  Bit-equal on the generator's thread count; 1e-6 leaves room for a CPU whose
+    vector width orders the weight-gradient sums differently."""
+    from pcdarts.genotypes import PRIMITIVES
+    from helpers import assert_close
+    m, y, dx, dw, g = _stock_mixed(name, C, stride)
+    for got, k in ((y, "y"), (dx, "dx"), (dw, "dw")):
+        assert_close(got, g[k], 1e-6, k)
+    pre = f"_ops.{PRIMITIVES.index(primitive)}."
+    for k, p in m.named_parameters():
+        if k.startswith(pre):
+            assert_close(p.grad, g["grad." + k], 1e-6, k)
+    for k, v in m.state_dict().items():
+        if k.startswith(pre) and ("running" in k or "tracked" in k):
+            assert_close(v.double(), g["buf." + k].double(), 1e-6, k)
 
 
 def test_derived_network_vs_stock_emulated():
