@@ -19,8 +19,9 @@
  *     only); the opt-in weight-gradient overlap (pcd_set_overlap: one library-owned low-priority stream + two events, set
  *     outside capture, used by one backward at a time); and the opt-in event profiler (pcd_profile_*: a single-threaded
  *     measurement mode).
- *   - BatchNorm is training-mode only (batch statistics, running stats updated in place,
- *     unbiased variance, num_batches_tracked += 1), eps/momentum as given.
+ *   - BatchNorm is training-mode (batch statistics, running stats updated in place,
+ *     unbiased variance, num_batches_tracked += 1), eps/momentum as given, except in the `*_eval`
+ *     entry points, which use the running statistics and write none of them.
  */
 #ifndef PCDARTS_SM100_H
 #define PCDARTS_SM100_H
@@ -321,6 +322,67 @@ int pcd_pool3x3_backward(const pcd_pool_args* a, void* stream);
  * preprocess kernels' normalised output */
 int pcd_channel_affine(const float* x, const float* scale, const float* shift, float* y, int batch, int channels, int hw,
                        void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Eval mode (module.eval(), BatchNorm from running statistics), forward only.
+ * Every BatchNorm is the per-channel affine map y = scale * z + shift with scale = gamma / sqrt(running_var + eps) and
+ * shift = beta - running_mean * scale (gamma = 1, beta = 0 without affine).  The calls read the same parameter and
+ * running-stat arenas, at the same offsets, as the training-mode calls above, and write nothing but their outputs
+ * (and `work`): no statistics, no running-stat updates, no num_batches_tracked, no saved activations.
+ * A node of a cell is ONE launch (every incoming edge, all 8 candidate ops, alpha / beta weighting, bypass channels and
+ * channel shuffle).  Shape envelope as in training mode.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct pcd_cell_eval_args {
+    pcd_cell_shape shape;
+    const float* s0;          /* (B, C_pp, H0, W0) contiguous */
+    const float* s1;          /* (B, C_p, H, W) contiguous */
+    const float* weights;     /* (14, 8) softmax(alphas) rows, device */
+    const float* weights2;    /* (14,) grouped softmax(betas), device */
+    const float* params;      /* param arena (pcd_cell_sizes_of) */
+    const float* running;     /* running-stat arena, read only */
+    float* out;               /* (B, 4C, Ho, Wo) contiguous */
+    float* work;              /* pcd_cell_eval_work_floats: the two preprocessed states */
+} pcd_cell_eval_args;
+
+int pcd_cell_eval_work_floats(const pcd_cell_shape* shape, int64_t* work_floats);
+int pcd_cell_forward_eval(const pcd_cell_eval_args* a, void* stream);
+
+typedef struct pcd_mixedop_eval_args {
+    pcd_mixedop_shape shape;
+    const float* x;           /* (B, C, H, W) contiguous */
+    const float* weights;     /* (8,) */
+    const float* params;
+    const float* running;     /* read only */
+    float* out;               /* (B, C, H/stride, W/stride) */
+} pcd_mixedop_eval_args;
+
+int pcd_mixedop_forward_eval(const pcd_mixedop_eval_args* a, void* stream);
+
+/* ReLUConvBN(C_in, C_out, 1, 1, 0) / FactorizedReduce: C_out a multiple of 16 (32 for FactorizedReduce) */
+typedef struct pcd_pre_eval_args {
+    int32_t batch, c_in, c_out, height, width;   /* input spatial size */
+    int32_t factorized;
+    float bn_eps;
+    const float* x;
+    const float* weight;      /* as pcd_pre_args.weight */
+    const float* running;     /* mean(C_out), var(C_out) */
+    const float* gamma;       /* NULL => 1 (affine=False) */
+    const float* beta;        /* NULL => 0 */
+    float* y;                 /* (B, C_out, Ho, Wo) */
+} pcd_pre_eval_args;
+
+int pcd_preprocess_forward_eval(const pcd_pre_eval_args* a, void* stream);
+
+typedef struct pcd_stem_eval_args {
+    int32_t batch, c_out, height, width;
+    float bn_eps;
+    const float* x;           /* (B,3,H,W) contiguous */
+    const float* params;      /* conv weight (Cout,3,3,3), bn weight (Cout), bn bias (Cout) */
+    const float* running;     /* mean(Cout), var(Cout) */
+    float* out;               /* (B,Cout,H,W) */
+} pcd_stem_eval_args;
+
+int pcd_stem_forward_eval(const pcd_stem_eval_args* a, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Network.global_pooling = AdaptiveAvgPool2d(7) followed by flatten

@@ -9,6 +9,7 @@
 #include "pcd_edge_v4.cuh"
 #include "pcd_edge_bwd4.cuh"
 #include "pcd_opk.cuh"
+#include "pcd_eval.cuh"
 #include "pcd_kernels.h"
 #include "pcd_launch.cuh"
 
@@ -939,6 +940,99 @@ int pcd_pool3x3_backward(const pcd_pool_args* a, void* stream) {
     PCD_TRY(pool_args(a, p));
     p.dy = a->grad_y; p.dx = a->grad_x;
     return launch_pool_bwd(p, stream);
+}
+
+// ---- eval mode (pcd_eval.cuh) --------------------------------------------------------------------------------------
+static int run_pre_eval(int B, int Cin, int Cout, int Hin, int Win, int fr, float eps, const float* x, const float* w,
+                        const float* running, const float* gamma, const float* beta, float* y, void* stream) {
+    if (B <= 0 || Cin <= 0 || Hin <= 0 || Win <= 0) return PCD_ERR_UNSUPPORTED;
+    if (fr && ((Hin | Win) & 1)) return PCD_ERR_UNSUPPORTED;
+    EvalPreArgs p;
+    memset(&p, 0, sizeof p);
+    p.B = B; p.Cin = Cin; p.Cout = Cout; p.Hin = Hin; p.Win = Win; p.fr = fr;
+    p.Ho = fr ? Hin / 2 : Hin; p.Wo = fr ? Win / 2 : Win;
+    p.eps = eps; p.x = x; p.w = w; p.running = running; p.gamma = gamma; p.beta = beta; p.y = y;
+    return launch_eval_pre(p, stream);
+}
+
+static int run_node_eval(int B, int c, int Ho, int Wo, float eps, float* out, long long out_ns, const EvalEdge* edges, int n,
+                         void* stream) {
+    if (n < 1 || n > kEvalMaxIn) return PCD_ERR_ARG;
+    EvalNodeArgs a;
+    memset(&a, 0, sizeof a);
+    a.B = B; a.Ho = Ho; a.Wo = Wo; a.TH = kEvalTH; a.nin = n; a.eps = eps; a.out = out; a.out_ns = out_ns; a.maxS = 1;
+    for (int i = 0; i < n; ++i) {
+        a.e[i] = edges[i];
+        if (edges[i].stride > a.maxS) a.maxS = edges[i].stride;
+    }
+    return launch_eval_node(a, c, stream);
+}
+
+int pcd_cell_eval_work_floats(const pcd_cell_shape* shape, int64_t* work_floats) {
+    if (!shape || !work_floats) return PCD_ERR_ARG;
+    CellLayout L;
+    PCD_TRY(cell_layout(*shape, L));
+    *work_floats = 2LL * L.B * L.C * L.Hs * L.Ws;
+    return PCD_OK;
+}
+
+int pcd_cell_forward_eval(const pcd_cell_eval_args* a, void* stream) {
+    if (!a || !a->s0 || !a->s1 || !a->weights || !a->weights2 || !a->params || !a->running || !a->out || !a->work)
+        return PCD_ERR_ARG;
+    CellLayout L;
+    PCD_TRY(cell_layout(a->shape, L));
+    const float eps = a->shape.bn_eps;
+    const long long state = (long long)L.C * L.Hs * L.Ws, node = (long long)L.C * L.Ho * L.Wo;
+    float* pre[2] = {a->work, a->work + L.B * state};
+    PCD_TRY(run_pre_eval(L.B, L.Cpp, L.C, L.H0, L.W0, L.redp, eps, a->s0, a->params + L.pre_par[0], a->running + L.pre_run[0],
+                         nullptr, nullptr, pre[0], stream));
+    PCD_TRY(run_pre_eval(L.B, L.Cp, L.C, L.Hs, L.Ws, 0, eps, a->s1, a->params + L.pre_par[1], a->running + L.pre_run[1],
+                         nullptr, nullptr, pre[1], stream));
+    for (int w = 0; w < 4; ++w) {
+        EvalEdge ev[kEvalMaxIn];
+        const int e0 = L.first_edge[w];
+        for (int j = 0; j < 2 + w; ++j) {
+            const int e = e0 + j;
+            EvalEdge& d = ev[j];
+            if (j < 2) { d.x = pre[j]; d.x_ns = state; d.Hs = L.Hs; d.Ws = L.Ws; }
+            else { d.x = a->out + (j - 2) * node; d.x_ns = 4 * node; d.Hs = L.Ho; d.Ws = L.Wo; }
+            d.stride = L.stride[e];
+            d.par = a->params + L.par[e];
+            d.running = a->running + L.run[e];
+            d.alpha = a->weights + e * PCD_NUM_PRIMITIVES;
+            d.beta = a->weights2 + e;
+        }
+        PCD_TRY(run_node_eval(L.B, L.c, L.Ho, L.Wo, eps, a->out + w * node, 4 * node, ev, 2 + w, stream));
+    }
+    return PCD_OK;
+}
+
+int pcd_mixedop_forward_eval(const pcd_mixedop_eval_args* a, void* stream) {
+    if (!a || !a->x || !a->weights || !a->params || !a->running || !a->out) return PCD_ERR_ARG;
+    EdgeGeom q;
+    PCD_TRY(mixedop_geom(a->shape, q));
+    EvalEdge d;
+    d.x = a->x; d.x_ns = 4LL * q.c * q.Hs * q.Ws; d.stride = q.S; d.Hs = q.Hs; d.Ws = q.Ws;
+    d.par = a->params; d.running = a->running; d.alpha = a->weights; d.beta = nullptr;
+    return run_node_eval(q.B, q.c, q.Ho, q.Wo, a->shape.bn_eps, a->out, 4LL * q.c * q.Ho * q.Wo, &d, 1, stream);
+}
+
+int pcd_preprocess_forward_eval(const pcd_pre_eval_args* a, void* stream) {
+    if (!a || !a->x || !a->weight || !a->running || !a->y) return PCD_ERR_ARG;
+    return run_pre_eval(a->batch, a->c_in, a->c_out, a->height, a->width, a->factorized, a->bn_eps, a->x, a->weight,
+                        a->running, a->gamma, a->beta, a->y, stream);
+}
+
+int pcd_stem_forward_eval(const pcd_stem_eval_args* a, void* stream) {
+    if (!a || !a->x || !a->params || !a->running || !a->out) return PCD_ERR_ARG;
+    if (a->batch <= 0 || a->c_out <= 0 || a->height <= 0 || a->width <= 0) return PCD_ERR_UNSUPPORTED;
+    EvalStemArgs s;
+    memset(&s, 0, sizeof s);
+    s.B = a->batch; s.Cout = a->c_out; s.H = a->height; s.W = a->width; s.eps = a->bn_eps;
+    s.rows = a->width >= 512 ? 1 : 512 / a->width;
+    if (s.rows > a->height) s.rows = a->height;
+    s.x = a->x; s.par = a->params; s.running = a->running; s.out = a->out;
+    return launch_eval_stem(s, stream);
 }
 
 int pcd_channel_affine(const float* x, const float* scale, const float* shift, float* y, int batch, int channels, int hw, void* stream) {

@@ -75,6 +75,25 @@ class PreArgs(C.Structure):
                     "x", "weight", "running", "nbt", "y", "stats", "grad_y", "grad_x", "grad_weight", "bstats")]
 
 
+class CellEvalArgs(C.Structure):
+    _fields_ = [("shape", CellShape)] + [(n, vp) for n in ("s0", "s1", "weights", "weights2", "params", "running", "out",
+                                                           "work")]
+
+
+class MixedEvalArgs(C.Structure):
+    _fields_ = [("shape", MixedShape)] + [(n, vp) for n in ("x", "weights", "params", "running", "out")]
+
+
+class PreEvalArgs(C.Structure):
+    _fields_ = [(n, i32) for n in ("batch", "c_in", "c_out", "height", "width", "factorized")] + [("bn_eps", f32)] + \
+        [(n, vp) for n in ("x", "weight", "running", "gamma", "beta", "y")]
+
+
+class StemEvalArgs(C.Structure):
+    _fields_ = [(n, i32) for n in ("batch", "c_out", "height", "width")] + [("bn_eps", f32)] + \
+        [(n, vp) for n in ("x", "params", "running", "out")]
+
+
 class DwConvArgs(C.Structure):
     _fields_ = [(n, i32) for n in ("batch", "channels", "height", "width", "kernel", "stride", "padding", "dilation",
                                    "relu_input")] + [(n, vp) for n in ("x", "weight", "out", "grad_out", "grad_x", "grad_weight")]
@@ -105,7 +124,9 @@ EXPORTS = ("pcd_launch_count", "pcd_profile_enable", "pcd_profile_num_kernels", 
            "pcd_decode_work_floats", "pcd_decode_greedy", "pcd_flat_max_runs", "pcd_flat_axpy", "pcd_flat_scale",
            "pcd_flat_sumsq", "pcd_flat_sumsq_work", "pcd_flat_adam", "pcd_gemm_small_f32",
            "pcd_dwconv_forward", "pcd_dwconv_backward", "pcd_pwconv_forward", "pcd_pwconv_backward", "pcd_bn_apply",
-           "pcd_bn_backward_stats", "pcd_pool3x3_forward", "pcd_pool3x3_backward", "pcd_channel_affine")
+           "pcd_bn_backward_stats", "pcd_pool3x3_forward", "pcd_pool3x3_backward", "pcd_channel_affine",
+           "pcd_cell_eval_work_floats", "pcd_cell_forward_eval", "pcd_mixedop_forward_eval", "pcd_preprocess_forward_eval",
+           "pcd_stem_forward_eval")
 
 
 def _declare(lib):
@@ -158,6 +179,10 @@ def _declare(lib):
                    ("pcd_pool3x3_forward", PoolArgs), ("pcd_pool3x3_backward", PoolArgs)):
         getattr(lib, fn).argtypes = [C.POINTER(st), vp]
     lib.pcd_channel_affine.argtypes = [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp]
+    lib.pcd_cell_eval_work_floats.argtypes = [C.POINTER(CellShape), C.POINTER(C.c_int64)]
+    for fn, st in (("pcd_cell_forward_eval", CellEvalArgs), ("pcd_mixedop_forward_eval", MixedEvalArgs),
+                   ("pcd_preprocess_forward_eval", PreEvalArgs), ("pcd_stem_forward_eval", StemEvalArgs)):
+        getattr(lib, fn).argtypes = [C.POINTER(st), vp]
     return lib
 
 

@@ -8,14 +8,15 @@ they are called on their own, and what a network derived from a genotype is buil
     affine_apply    gamma * yhat + beta behind the preprocess kernels' normalised output (ReLUConvBN / FactorizedReduce with
                     affine=True, operations.py:22-33,90-104)
 
-Training-mode BatchNorm only (batch statistics; running statistics updated like nn.BatchNorm2d); everything else raises.
+BatchNorm in training mode (batch statistics; running statistics updated like nn.BatchNorm2d) or, in eval mode under
+torch.no_grad(), from the running statistics (forward only, nothing written).
 """
 import ctypes as C
 
 import torch
 
 import pcd_native as N
-from pcd_ops import BN_EPS, BN_MOMENTUM, _empty, _empty_like, _f32c
+from pcd_ops import BN_EPS, BN_MOMENTUM, _empty, _empty_like, _f32c, autograd_records
 
 
 def _bn_running(bn):
@@ -91,22 +92,64 @@ class UnitFunction(torch.autograd.Function):
 
 
 def _check(x, bn, what):
-    if not bn.training:
-        raise NotImplementedError(f"{what}: the native path implements training-mode BatchNorm (batch statistics) only")
     if not bn.track_running_stats or bn.momentum is None or abs(bn.momentum - BN_MOMENTUM) > 1e-12 or abs(bn.eps - BN_EPS) > 1e-12:
         raise NotImplementedError(f"{what}: BatchNorm2d(eps={BN_EPS}, momentum={BN_MOMENTUM}, track_running_stats=True) expected")
     if x.dim() != 4 or x.dtype != torch.float32:
         raise NotImplementedError(f"{what}: float32 NCHW input expected")
 
 
+def _eval_guard(tensors, bn, what):
+    """True in eval mode (BatchNorm from running statistics: forward only); raises if autograd would record that forward."""
+    if bn.training:
+        return False
+    if autograd_records(tensors):
+        raise NotImplementedError(f"{what} in eval mode (BatchNorm from running statistics) is forward-only: wrap the call in "
+                                  "torch.no_grad() or torch.inference_mode(), or call .train() to differentiate")
+    return True
+
+
+def _unit_eval(x, dw, pw, bn):
+    """Eval-mode unit: dwconv -> pwconv (its batch sums go to a scratch buffer, unused) -> per-channel running-stat affine."""
+    lib = N.lib_for(x)
+    xc = _f32c(x)
+    ks, stride, pad, dil = dw.kernel_size[0], dw.stride[0], dw.padding[0], dw.dilation[0]
+    B, cin, H, W = xc.shape
+    cout = pw.out_channels
+    ho = (H + 2 * pad - dil * (ks - 1) - 1) // stride + 1
+    wo = (W + 2 * pad - dil * (ks - 1) - 1) // stride + 1
+    dev, st = xc.device, N.stream_for(xc)
+    t = _empty((B, cin, ho, wo), torch.float32, dev)
+    a = N.DwConvArgs(B, cin, H, W, ks, stride, pad, dil, 1, N.ptr(xc), N.ptr(_f32c(dw.weight)), N.ptr(t), None, None, None)
+    N.check(lib, lib.pcd_dwconv_forward(C.byref(a), st), "pcd_dwconv_forward")
+    z = _empty((B, cout, ho, wo), torch.float32, dev)
+    scratch = _empty(2 * cout, torch.float64, dev)
+    p = N.PwConvArgs(B, cin, cout, ho * wo, BN_EPS, N.ptr(t), N.ptr(_f32c(pw.weight)), N.ptr(z), N.ptr(scratch), None, None, None,
+                     None, None)
+    N.check(lib, lib.pcd_pwconv_forward(C.byref(p), st), "pcd_pwconv_forward")
+    # ATen's inference BatchNorm: scale = gamma / sqrt(running_var + eps), shift = beta - running_mean * scale
+    scale = 1.0 / torch.sqrt(bn.running_var + bn.eps)
+    if bn.affine:
+        scale = scale * bn.weight
+    shift = -bn.running_mean * scale
+    if bn.affine:
+        shift = shift + bn.bias
+    y = _empty_like(z)
+    N.check(lib, lib.pcd_channel_affine(N.ptr(z), N.ptr(_f32c(scale)), N.ptr(_f32c(shift)), N.ptr(y), B, cout, ho * wo, st),
+            "pcd_channel_affine")
+    return y
+
+
 def unit_apply(x, dw, pw, bn, what="unit"):
     """ReLU -> `dw` (depthwise nn.Conv2d) -> `pw` (1x1 nn.Conv2d) -> `bn` on the native kernels."""
+    is_eval = _eval_guard([x, dw.weight, pw.weight, bn.weight, bn.bias], bn, what)
     _check(x, bn, what)
     ks, stride, pad, dil = dw.kernel_size[0], dw.stride[0], dw.padding[0], dw.dilation[0]
     if dw.groups != dw.in_channels or dw.kernel_size[0] != dw.kernel_size[1] or ks not in (3, 5, 7) or stride not in (1, 2) or \
             dw.bias is not None or pw.bias is not None or pw.kernel_size != (1, 1) or pw.in_channels % 4 or pw.out_channels % 4 or \
             max(pw.in_channels, pw.out_channels) > 128 or max(x.shape[2], x.shape[3]) > 64:
         raise RuntimeError(f"{what}: shape not supported by the compiled kernels (PCD_ERR_UNSUPPORTED)")
+    if is_eval:
+        return _unit_eval(x, dw, pw, bn)
     run_ptr, nbt_ptr = _bn_running(bn)
     return UnitFunction.apply(x, dw.weight, pw.weight, bn.weight if bn.affine else None, bn.bias if bn.affine else None,
                               (ks, stride, pad, dil, run_ptr, nbt_ptr))

@@ -493,11 +493,13 @@ def preprocess_apply(module, x, fr):
         if (k, stride, pad) != (1, 1, 0):
             raise NotImplementedError("only the 1x1/stride 1/pad 0 ReLUConvBN of the search network is accelerated")
         bn = module.op[2]
-    if not module.training:
-        raise NotImplementedError("preprocess kernels implement training-mode BatchNorm (batch statistics) only")
+    is_eval = eval_forward(module, x)
     if not hasattr(module, "_pcd_arena"):
         module._pcd_arena = Arena(module)
     ar = module._pcd_arena.ensure()
+    if is_eval:
+        return preprocess_forward_eval(x, fr, c_in, c_out, ar.param_ptr, ar.running_ptr,
+                                       bn.weight if affine else None, bn.bias if affine else None)
     meta = (fr, c_in, c_out, (ar.param_ptr, ar.running_ptr, ar.nbt_ptr))
     convs = [module.conv_1.weight, module.conv_2.weight] if fr else [module.op[1].weight]     # first in the arena, back to back
     yhat = PreprocessFunction.apply(x, meta, *convs)
@@ -505,6 +507,79 @@ def preprocess_apply(module, x, fr):
         from pcd_opmods import affine_apply
         return affine_apply(yhat, bn)
     return yhat
+
+
+# --------------------------------------------------------------------------------------------
+# eval mode: BatchNorm from running statistics, forward only (plain calls, no autograd Functions)
+# --------------------------------------------------------------------------------------------
+def autograd_records(tensors):
+    """True when a forward over `tensors` would be recorded by autograd."""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
+
+
+def eval_forward(module, *inputs):
+    """True when `module` is in eval mode, i.e. its forward runs the eval kernels.  There is no eval-mode backward, so eval
+    mode while autograd records (grad enabled and any parameter or input requiring grad) raises NotImplementedError."""
+    if module.training:
+        return False
+    if autograd_records(inputs) or autograd_records(module.parameters()):
+        raise NotImplementedError(
+            f"{type(module).__name__} in eval mode (BatchNorm from running statistics) is forward-only: wrap the call in "
+            "torch.no_grad() or torch.inference_mode(), or call .train() to differentiate")
+    return True
+
+
+def cell_forward_eval(s0, s1, weights, weights2, handle):
+    """Cell.forward in eval mode: two preprocess launches + one launch per node."""
+    lib = N.lib_for(s1)
+    s0c, s1c, w, w2 = _f32c(s0), _f32c(s1), _f32c(weights), _f32c(weights2)
+    B, _, H, W = s1c.shape
+    sz = handle.sizes(lib, B, H, W)
+    out = _empty((B, 4 * handle.cfg[2], sz.out_height, sz.out_width), torch.float32, s1c.device)
+    sh = handle.shape(B, H, W)
+    nwork = C.c_int64()
+    N.check(lib, lib.pcd_cell_eval_work_floats(C.byref(sh), C.byref(nwork)), "pcd_cell_eval_work_floats")
+    work = _empty(nwork.value, torch.float32, s1c.device)
+    a = N.CellEvalArgs(sh, N.ptr(s0c), N.ptr(s1c), N.ptr(w), N.ptr(w2), handle.param_ptr, handle.running_ptr, N.ptr(out),
+                       N.ptr(work))
+    N.check(lib, lib.pcd_cell_forward_eval(C.byref(a), N.stream_for(s1c)), "pcd_cell_forward_eval")
+    return out
+
+
+def mixedop_forward_eval(x, weights, handle):
+    lib = N.lib_for(x)
+    xc, w = _f32c(x), _f32c(weights)
+    B, Cc, H, W = xc.shape
+    sz = handle.sizes(lib, B, H, W)
+    out = _empty((B, Cc, sz.out_height, sz.out_width), torch.float32, xc.device)
+    a = N.MixedEvalArgs(handle.shape(B, H, W), N.ptr(xc), N.ptr(w), handle.param_ptr, handle.running_ptr, N.ptr(out))
+    N.check(lib, lib.pcd_mixedop_forward_eval(C.byref(a), N.stream_for(xc)), "pcd_mixedop_forward_eval")
+    return out
+
+
+def stem_forward_eval(x, param_ptr, running_ptr, c_out):
+    lib = N.lib_for(x)
+    xc = _f32c(x)
+    B, cin, H, W = xc.shape
+    if cin != 3:
+        raise ValueError("stem expects 3 input channels")
+    out = _empty((B, c_out, H, W), torch.float32, xc.device)
+    a = N.StemEvalArgs(B, c_out, H, W, BN_EPS, N.ptr(xc), param_ptr, running_ptr, N.ptr(out))
+    N.check(lib, lib.pcd_stem_forward_eval(C.byref(a), N.stream_for(xc)), "pcd_stem_forward_eval")
+    return out
+
+
+def preprocess_forward_eval(x, fr, c_in, c_out, weight_ptr, running_ptr, gamma=None, beta=None):
+    lib = N.lib_for(x)
+    xc = _f32c(x)
+    B, _, H, W = xc.shape
+    ho, wo = (H // 2, W // 2) if fr else (H, W)
+    y = _empty((B, c_out, ho, wo), torch.float32, xc.device)
+    g = _f32c(gamma) if gamma is not None else None
+    b = _f32c(beta) if beta is not None else None
+    a = N.PreEvalArgs(B, c_in, c_out, H, W, int(fr), BN_EPS, N.ptr(xc), weight_ptr, running_ptr, N.ptr(g), N.ptr(b), N.ptr(y))
+    N.check(lib, lib.pcd_preprocess_forward_eval(C.byref(a), N.stream_for(xc)), "pcd_preprocess_forward_eval")
+    return y
 
 
 # --------------------------------------------------------------------------------------------

@@ -15,7 +15,8 @@ stock torch layers in float64 (`stock_forward`).  The structure follows the sear
     reduction cell (model_search.py:79); node = op1(h1) + op2(h2); output = concat of the `*_concat` states.
 
 Execution: every op runs on the library's stand-alone op kernels (pcd_opmods.py), stem / pooling on the kernels the search
-network uses.  Training-mode BatchNorm only.  Drop-path and the auxiliary head of the CIFAR / ImageNet evaluation recipes
+network uses.  In eval mode under torch.no_grad() every BatchNorm uses its running statistics: the stem and the preprocess
+ops run the eval kernels, each DilConv / SepConv unit depthwise -> pointwise -> running-stat affine.  Drop-path and the auxiliary head of the CIFAR / ImageNet evaluation recipes
 are not part of this path.
 """
 import torch
@@ -104,14 +105,16 @@ class NetworkDerived(nn.Module):
             for cell in self.cells:
                 s0, s1 = s1, cell(s0, s1, stock=True)
             return self.global_pooling(s1).flatten(start_dim=1)
-        if not self.training:
-            raise NotImplementedError("eval-mode BatchNorm (running statistics) is outside the native path")
+        is_eval = pcd_ops.eval_forward(self, input)
         ar = self.__dict__.get('_stem_arena')
         if ar is None:
             ar = pcd_ops.Arena(self.stem)
             self.__dict__['_stem_arena'] = ar
         ar = ar.ensure()
-        s0 = s1 = pcd_ops.StemFunction.apply(x, (ar.param_ptr, ar.running_ptr, ar.nbt_ptr), *ar.params)
+        if is_eval:
+            s0 = s1 = pcd_ops.stem_forward_eval(x, ar.param_ptr, ar.running_ptr, self.stem[0].out_channels)
+        else:
+            s0 = s1 = pcd_ops.StemFunction.apply(x, (ar.param_ptr, ar.running_ptr, ar.nbt_ptr), *ar.params)
         for cell in self.cells:
             s0, s1 = s1, cell(s0, s1)
         return pcd_ops.AdaptiveAvgPoolFunction.apply(s1, self.output_size).flatten(start_dim=1)

@@ -47,11 +47,6 @@ class _ArenaModule(nn.Module):
         pcd_ops.bump_layout_epoch()       # storages (and buffer objects) were replaced
         return out
 
-    def _require_training(self):
-        if not self.training:
-            raise NotImplementedError(
-                "eval-mode BatchNorm (running statistics) is outside the accelerated search path; "
-                "call .train() — the reference only uses eval mode in its validation loop")
 
 
 class MixedOp(_ArenaModule):
@@ -70,10 +65,12 @@ class MixedOp(_ArenaModule):
         self.__dict__['_pcd_handle'] = pcd_ops.MixedHandle(C, stride)
 
     def forward(self, x, weights):
-        self._require_training()
+        is_eval = pcd_ops.eval_forward(self, x, weights)
         ar = self._arena()
         h = self.__dict__['_pcd_handle']
         h.param_ptr, h.running_ptr, h.nbt_ptr = ar.param_ptr, ar.running_ptr, ar.nbt_ptr
+        if is_eval:
+            return pcd_ops.mixedop_forward_eval(x, weights, h)
         return pcd_ops.MixedOpFunction.apply(x, weights, h, *ar.params)
 
 
@@ -107,10 +104,12 @@ class Cell(_ArenaModule):
         return ps
 
     def forward(self, s0, s1, weights, weights2):
-        self._require_training()
+        is_eval = pcd_ops.eval_forward(self, s0, s1, weights, weights2)
         ar = self._arena()
         h = self.__dict__['_pcd_handle']
         h.param_ptr, h.running_ptr, h.nbt_ptr = ar.param_ptr, ar.running_ptr, ar.nbt_ptr
+        if is_eval:
+            return pcd_ops.cell_forward_eval(s0, s1, weights, weights2, h)
         return pcd_ops.CellFunction.apply(s0, s1, weights, weights2, h, *ar.params)
 
 
@@ -216,7 +215,7 @@ class Network(_ArenaModule):
         return plans[key]
 
     def forward(self, input):
-        self._require_training()
+        is_eval = pcd_ops.eval_forward(self, input, *self._arch_parameters)
         n, _, h, w = input.shape
         x = input.expand(n, 3, h, w)           # 1-channel inputs are broadcast (model_search.py:150)
         ar = self._arena()
@@ -224,6 +223,8 @@ class Network(_ArenaModule):
         cells, total = self._plan(lib, n, h, w)
         if total != ar.param_floats:
             raise RuntimeError("parameter arena does not match the kernel layout")
+        if is_eval:
+            return self._forward_eval(x, ar, cells)
         params = ar.params
         wg = pcd_ops.weight_grads_enabled()
         if wg:
@@ -249,6 +250,20 @@ class Network(_ArenaModule):
             s0, s1 = s1, pcd_ops.CellFunction.apply(s0, s1, weights, weights2, handle, *cell_params)
             pos += n_par
         out = pcd_ops.AdaptiveAvgPoolFunction.apply(s1, self.output_size)
+        return out.flatten(start_dim=1)
+
+    def _forward_eval(self, x, ar, cells):
+        """Eval mode (running-statistics BatchNorm), forward only: stem, one launch per node, global pooling."""
+        s0 = s1 = pcd_ops.stem_forward_eval(x, ar.param_ptr, ar.running_ptr, self._stem_multiplier * self._C)
+        w_normal = (F.softmax(self.alphas_normal, dim=-1), _grouped_softmax(self.betas_normal, self._steps))
+        w_reduce = (F.softmax(self.alphas_reduce, dim=-1), _grouped_softmax(self.betas_reduce, self._steps))
+        for cell, (handle, p_off, r_off, _, _) in zip(self.cells, cells):
+            handle.param_ptr = ar.param_ptr + 4 * p_off
+            handle.running_ptr = ar.running_ptr + 4 * r_off
+            weights, weights2 = w_reduce if cell.reduction else w_normal
+            s0, s1 = s1, pcd_ops.cell_forward_eval(s0, s1, weights, weights2, handle)
+        with torch.no_grad():
+            out = pcd_ops.AdaptiveAvgPoolFunction.apply(s1, self.output_size)
         return out.flatten(start_dim=1)
 
     def _loss(self, images, questions, labels):
