@@ -462,6 +462,21 @@ int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const 
                       const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
                       const float* w_out, const float* b_out, long long* tokens, float* work, void* stream);
 
+/* Sampled question decode (QstEncoder.generate with deterministic=False: every word drawn from softmax(logits / temperature),
+ * darts_vqa/vqa_model.py:87-92) in the same kernel, by the Gumbel-max trick: word t of row b is
+ *     argmax_v ( logit_v / temperature + G(seed, t, row_offset + b, v) )
+ * with G a standard Gumbel variable from Philox4x32-10:  key = {seed & 0xffffffff, seed >> 32}, counter = {v >> 2, t, row, 0},
+ * x = word (v & 3) of the block, u = ((float)(x >> 9) + 0.5f) * 2^-23, G = -logf(-logf(u)).  The noise depends only on
+ * (seed, t, row, v): a batch decoded in slices (row_offset = first row of the slice) draws what one call would.  `seed` is a
+ * DEVICE pointer to one 8-byte-aligned uint64, read by the kernel (the call is CUDA-graph capturable; a graph replays the
+ * seed the buffer holds at replay time).  Envelope, token layout and workspace as pcd_decode_greedy.  PCD_ERR_ARG for a null
+ * seed, a negative row_offset or a temperature that is not finite and > 0.  The distribution equals torch.multinomial's;
+ * the random stream does not. */
+int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                      const float* b_out, long long* tokens, float* work, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Optimizer-side elementwise operations over a short table of flat runs.  The search step updates all 732 parameter
  * tensors several times per step outside the network — w' = w - eta * dL/dw (darts_vqa/pcdarts/architect_vqa.py:35-38),

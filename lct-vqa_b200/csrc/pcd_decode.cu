@@ -13,10 +13,13 @@
 //   -- grid barrier --
 //   the next phase A starts by reducing the candidates (lowest index wins ties, like torch.argmax) to the new words;
 //   the input projection is split four ways along the embedding row (all ~19 float4 loads of a thread independent).
-// The logits are never written anywhere.  Sampling (deterministic=False, torch.multinomial) is not covered: the Python side
-// keeps that on stock torch ops.
+// The logits are never written anywhere.  Sampled decoding (deterministic=False: torch.multinomial over softmax(logits / T))
+// is the same kernel with kSample = true: the phase-B epilogue ranks score = logit / T + G(seed, t, row, v) instead of the
+// logit (Gumbel-max; G from pcd_philox.cuh, the seed read from device memory, so the kernel stays graph-capturable), and
+// everything else — candidates, pick_words, barriers, phase A — is shared.
 #include "../../include/pcdarts_sm100.h"
 #include "pcd_launch.cuh"
+#include "pcd_philox.cuh"
 
 #include <limits.h>
 
@@ -28,6 +31,9 @@ PCD_HOSTDEV int u_floats(int H) { return kMaxB * (H + 4) > kStages * kStageFloat
 static inline int tiles_of(int V) { return (V + kTileN - 1) / kTileN; }
 static inline bool shape_ok(int T, int B, int H, int E, int V) {
     return T > 0 && B > 0 && B <= kMaxB && H >= 32 && H <= 512 && H % 32 == 0 && E > 0 && E % 4 == 0 && V > 0;
+}
+static inline bool sample_args_ok(float temperature, const unsigned long long* seed, int row_offset) {
+    return seed && row_offset >= 0 && isfinite(temperature) && temperature > 0.f;
 }
 }  // namespace decode
 }  // namespace pcd
@@ -49,7 +55,10 @@ struct Args {
     long long* tokens;    // [B][T]
     float* hbuf;          // [2][B][H]  h_t, double-buffered by step parity
     float* tbuf;          // [B][H]     tanh(h_t): the input of the vocabulary projection
-    float2* cand;         // [B][ntiles]  (logit, index bits): one 8-byte word per row and vocabulary tile
+    float2* cand;         // [B][ntiles]  (logit or sampled score, index bits): one 8-byte word per row and vocabulary tile
+    const unsigned long long* seed;   // sampled decode only: Philox key (device memory)
+    float temperature;
+    int row_offset;                   // global batch row of row 0 (batches above 64 are decoded in slices)
 };
 
 __device__ __forceinline__ float sigm(float x) { return 1.f / (1.f + expf(-x)); }
@@ -109,6 +118,7 @@ __device__ __forceinline__ void pick_words(const Args& a, int* TOK) {
     }
 }
 
+template <bool kSample>
 __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
     cg::grid_group grid = cg::this_grid();
     extern __shared__ __align__(16) float sm[];
@@ -264,12 +274,35 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
                 for (int i = 0; i < 4; ++i) {
                     float best = -INFINITY;
                     int bi = INT_MAX;
+                    if constexpr (kSample) {
+                        // columns col0 + tx + 16j of a lane quad (tx >> 2) share one Philox block per j: lane q = tx & 3
+                        // computes the blocks of j = q and j = q + 4, and the quad hands word q of every block to lane q
+                        const int q = tx & 3, quad = (threadIdx.x & 31) & ~3;
+                        const unsigned long long seed = __ldg(a.seed);
+                        const uint32_t v4 = (uint32_t)(col0 >> 2) + (uint32_t)(tx >> 2) + 4u * q;
+                        const uint32_t grow = (uint32_t)(a.row_offset + 4 * ty + i);
+                        const Philox4 blk[2] = {philox4x32_10(v4, (uint32_t)t, grow, 0u, (uint32_t)seed, (uint32_t)(seed >> 32)),
+                                                philox4x32_10(v4 + 16u, (uint32_t)t, grow, 0u, (uint32_t)seed, (uint32_t)(seed >> 32))};
 #pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const int col = col0 + tx + 16 * j;
-                        if (col < a.V) {
-                            const float v = acc[i][j] + __ldg(a.b_out + col);
-                            if (v > best) { best = v; bi = col; }
+                        for (int j = 0; j < 8; ++j) {
+                            uint32_t w[4];
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) w[k] = __shfl_sync(0xffffffffu, blk[j >> 2].w[k], quad | (j & 3));
+                            const uint32_t x = q == 0 ? w[0] : q == 1 ? w[1] : q == 2 ? w[2] : w[3];
+                            const int col = col0 + tx + 16 * j;
+                            if (col < a.V) {
+                                const float v = (acc[i][j] + __ldg(a.b_out + col)) / a.temperature + gumbel_of_bits(x);
+                                if (v > best) { best = v; bi = col; }
+                            }
+                        }
+                    } else {
+#pragma unroll
+                        for (int j = 0; j < 8; ++j) {
+                            const int col = col0 + tx + 16 * j;
+                            if (col < a.V) {
+                                const float v = acc[i][j] + __ldg(a.b_out + col);
+                                if (v > best) { best = v; bi = col; }
+                            }
                         }
                     }
 #pragma unroll
@@ -297,39 +330,45 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
 }  // namespace decode
 }  // namespace pcd
 
-extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                 const float* w_out, const float* b_out, long long* tokens, float* work, void* stream) {
-    using namespace pcd;
+namespace pcd {
+namespace decode {
+
+template <bool kSample>
+static int run(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+               const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
+               const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
+               float* work, void* stream) {
     if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
-    if (!decode::shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
+    if (!shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
     if ((((uintptr_t)emb) | ((uintptr_t)w_ih) | ((uintptr_t)w_hh) | ((uintptr_t)h0) | ((uintptr_t)w_out) | ((uintptr_t)work)) & 15) return PCD_ERR_ALIGN;
+    if (((uintptr_t)seed) & 7) return PCD_ERR_ALIGN;
     LaunchState& L = launch_state();
-    const size_t smem = ((size_t)16 * (H + 4) + (size_t)16 * (E + 4) + (size_t)decode::u_floats(H) + decode::kMaxB + 64 * decode::kMaxB) * sizeof(float);
+    const size_t smem = ((size_t)16 * (H + 4) + (size_t)16 * (E + 4) + (size_t)u_floats(H) + kMaxB + 64 * kMaxB) * sizeof(float);
     if (smem > 227 * 1024) return PCD_ERR_UNSUPPORTED;
-    static int sms = 0;
+    static int sms = 0;                                     // per instantiation: each one sets its own smem attribute
     if (!sms) {
         int dev = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-            cudaFuncSetAttribute(decode::decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            cudaFuncSetAttribute(decode_kernel<kSample>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
             sms = 0;
             snprintf(L.last_err, sizeof L.last_err, "decode setup: %s", cudaGetErrorString(cudaGetLastError()));
             return PCD_ERR_CUDA;
         }
     }
-    const int ntiles = decode::tiles_of(V);
+    const int ntiles = tiles_of(V);
     int grid = ntiles < sms ? ntiles : sms;                 // one block per SM: all of them co-resident (cooperative launch)
-    if (grid < H / decode::kUnits) grid = H / decode::kUnits;
+    if (grid < H / kUnits) grid = H / kUnits;
     if (grid > sms) return PCD_ERR_UNSUPPORTED;
-    decode::Args a;
+    Args a;
     a.T = T; a.B = B; a.H = H; a.E = E; a.V = V; a.start = start_token; a.ntiles = ntiles;
     a.emb = emb; a.w_ih = w_ih; a.w_hh = w_hh; a.b_ih = b_ih; a.b_hh = b_hh; a.h0 = h0; a.c0 = c0; a.w_out = w_out; a.b_out = b_out;
     a.tokens = tokens;
     a.hbuf = work;
     a.tbuf = work + (size_t)2 * B * H;
     a.cand = reinterpret_cast<float2*>(work + (size_t)3 * B * H);
+    a.seed = seed; a.temperature = temperature; a.row_offset = row_offset;
     void* args[] = {&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)decode::decode_kernel, dim3(grid), dim3(decode::kT), args, smem, (cudaStream_t)stream);
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)decode_kernel<kSample>, dim3(grid), dim3(kT), args, smem, (cudaStream_t)stream);
     count_launch(L);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) {
@@ -339,6 +378,25 @@ extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_to
     return PCD_OK;
 }
 
+}  // namespace decode
+}  // namespace pcd
+
+extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                                 const float* w_out, const float* b_out, long long* tokens, float* work, void* stream) {
+    return pcd::decode::run<false>(T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out,
+                                   tokens, work, stream);
+}
+
+extern "C" int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                                 const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                                 const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                                 const float* b_out, long long* tokens, float* work, void* stream) {
+    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset)) return PCD_ERR_ARG;
+    return pcd::decode::run<true>(T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0,
+                                  w_out, b_out, tokens, work, stream);
+}
+
 #else   // ---- CPU emulation build (tests only) ----------------------------------------------------------------------
 
 #include <math.h>
@@ -346,11 +404,15 @@ extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_to
 
 static inline float sigm_(float x) { return 1.f / (1.f + expf(-x)); }
 
-extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                 const float* w_out, const float* b_out, long long* tokens, float* work, void*) {
+// the kernel's arithmetic per row and step: fp64 gate and vocabulary sums rounded to fp32, argmax of the fp32 logit (greedy)
+// or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go to the lowest index
+static int decode_emu(bool sample, int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
+                      const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
+                      float* work) {
     if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
     if (!pcd::decode::shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
+    const unsigned long long key = sample ? *seed : 0ull;
     std::vector<float> h(h0, h0 + (size_t)B * H), c(c0, c0 + (size_t)B * H), hn((size_t)H), x((size_t)E), s((size_t)H);
     for (int b = 0; b < B; ++b) {
         int word = start_token;
@@ -376,13 +438,30 @@ extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_to
             for (int v = 0; v < V; ++v) {
                 double acc = b_out[v];
                 for (int k = 0; k < H; ++k) acc += (double)s[k] * w_out[(long long)v * H + k];
-                if ((float)acc > best) { best = (float)acc; bi = v; }
+                const float score = sample ? (float)acc / temperature + pcd::decode_gumbel(key, t, row_offset + b, v) : (float)acc;
+                if (score > best) { best = score; bi = v; }
             }
             word = bi;
             tokens[(long long)b * T + t] = bi;
         }
     }
     return PCD_OK;
+}
+
+extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                                 const float* w_out, const float* b_out, long long* tokens, float* work, void*) {
+    return decode_emu(false, T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens,
+                      work);
+}
+
+extern "C" int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                                 const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                                 const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                                 const float* b_out, long long* tokens, float* work, void*) {
+    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset)) return PCD_ERR_ARG;
+    return decode_emu(true, T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out,
+                      b_out, tokens, work);
 }
 
 #endif

@@ -7,7 +7,7 @@ import torch.nn as nn
 
 import config
 import pcd_ops
-from pcd_ops import decode_greedy, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
+from pcd_ops import decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
 from pcdarts.model_search import Network
 
 
@@ -80,8 +80,12 @@ class QstEncoder(nn.Module):
         h0 = image_embedding.reshape(batch, self.hidden_size)
         if self.deterministic and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
             return decode_greedy(h0, self.lstm, self.word2vec, self.fc2, self.max_length)      # one persistent kernel
+        if self.deterministic is False and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
+            # the same kernel, words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
+            return decode_sample(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.temperature)
         if self.deterministic:       # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
             pcd_ops._stock(f"greedy decode with hidden size {self.hidden_size}")
+        # sampled decoding outside the kernel's envelope: the reference's module loop (torch.multinomial)
         self.lstm.flatten_parameters()
         h = image_embedding.view(1, -1, self.hidden_size)
         state = (h, h)
@@ -152,4 +156,7 @@ class VqaModel(nn.Module):
                         self.hidden_size)
         twin.img_encoder.darts = self.img_encoder.darts.new()
         _copy_dropout(self, twin)
+        # the unrolled twin generates ArchitectLct's pseudo questions: it decodes the way this model was configured to
+        for name in ("deterministic", "temperature", "max_length"):
+            setattr(twin.qst_encoder, name, getattr(self.qst_encoder, name))
         return twin.to(config.DEVICE)

@@ -13,7 +13,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 SOURCES = [os.path.join(CSRC, f) for f in ("pcd_api.cu", "pcd_k_fwd.cu", "pcd_k_fwd4.cu", "pcd_k_bwd4.cu", "pcd_k_bwdA.cu", "pcd_k_bwdB.cu", "pcd_k_bwd2.cu", "pcd_k_pre.cu", "pcd_pre_tc.cu", "pcd_gemm_sm100.cu", "pcd_ce.cu", "pcd_lstm.cu", "pcd_decode.cu", "pcd_flat.cu", "pcd_gemm_small.cu", "pcd_k_ops.cu", "pcd_k_eval.cu")]
 HEADERS = [os.path.join(CSRC, f) for f in ("pcd_common.cuh", "pcd_edge.cuh", "pcd_fwd.cuh", "pcd_bwd.cuh",
-                                           "pcd_launch.cuh", "pcd_kernels.h", "pcd_pre.cuh", "pcd_edge_bwd2.cuh", "pcd_edge_v4.cuh", "pcd_edge_bwd4.cuh", "pcd_tc.cuh", "pcd_opk.cuh", "pcd_eval.cuh")] + \
+                                           "pcd_launch.cuh", "pcd_kernels.h", "pcd_pre.cuh", "pcd_edge_bwd2.cuh", "pcd_edge_v4.cuh", "pcd_edge_bwd4.cuh", "pcd_tc.cuh", "pcd_opk.cuh", "pcd_eval.cuh", "pcd_philox.cuh")] + \
           [os.path.join(ROOT, "include", "pcdarts_sm100.h")]
 BUILD_DIR = os.path.join(HERE, "build")
 CUDA_LIB = os.path.join(HERE, "libpcdarts_sm100.so")

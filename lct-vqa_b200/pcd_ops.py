@@ -6,6 +6,7 @@ scratch) is allocated here with torch and handed to the library as raw pointers;
 enqueues on torch's current stream.
 """
 import ctypes as C
+import math
 
 import torch
 
@@ -919,22 +920,20 @@ def lstm_forward(lstm, x, h0, c0):
 
 
 # --------------------------------------------------------------------------------------------
-# Greedy question decode (QstEncoder.generate): one persistent cooperative kernel
+# Question decode (QstEncoder.generate): one persistent cooperative kernel, greedy or sampled
 # --------------------------------------------------------------------------------------------
 def decode_supported(h0, lstm, word2vec, proj):
-    """Shapes pcd_decode_greedy takes (single-layer LSTM, hidden a multiple of 32 up to 512, E % 4 == 0; any batch: tiled by 64)."""
+    """Shapes pcd_decode_greedy / pcd_decode_sample take (single-layer LSTM, hidden a multiple of 32 up to 512, E % 4 == 0;
+    any batch: tiled by 64)."""
     H = lstm.hidden_size
     return (h0.is_cuda or N._emu_lib is not None) and lstm.num_layers == 1 and not lstm.bidirectional and lstm.bias and \
         32 <= H <= 512 and H % 32 == 0 and word2vec.embedding_dim % 4 == 0 and \
         proj.in_features == H and proj.bias is not None and h0.dtype == torch.float32
 
 
-def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2):
-    """tokens (B, max_length) int64 of the greedy decode that starts from `start_token` with h0 = c0 = `h0` (B, H).
-    Not differentiable (neither is the reference's argmax): parameters are read detached."""
-    if h0.shape[0] > _LSTM_BATCH:          # independent rows: ceil(B / 64) launches of the persistent kernel
-        return torch.cat([decode_greedy(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length, start_token)
-                          for b0 in range(0, h0.shape[0], _LSTM_BATCH)], 0)
+def _decode_operands(h0, lstm, word2vec, proj, max_length):
+    """(lib, leading int arguments, pointer arguments, tensors behind the pointers, tokens) of one decode launch over at most
+    64 rows.  The caller holds the tensors until the launch is enqueued."""
     lib = N.lib_for(h0)
     B, H = h0.shape
     V, E = word2vec.weight.shape
@@ -943,6 +942,43 @@ def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2):
     wout, bout = _f32c(proj.weight), _f32c(proj.bias)
     tokens = torch.empty((B, max_length), dtype=torch.long, device=h0.device)
     work = torch.empty(int(lib.pcd_decode_work_floats(B, H, V)), dtype=torch.float32, device=h0.device)
-    N.check(lib, lib.pcd_decode_greedy(max_length, B, H, E, V, start_token, *[N.ptr(t) for t in ops], N.ptr(h0c), N.ptr(h0c),
-                                       N.ptr(wout), N.ptr(bout), N.ptr(tokens), N.ptr(work), N.stream_for(h0)), "pcd_decode_greedy")
+    ptrs = [N.ptr(t) for t in ops] + [N.ptr(h0c), N.ptr(h0c), N.ptr(wout), N.ptr(bout), N.ptr(tokens), N.ptr(work),
+                                      N.stream_for(h0)]
+    return lib, (max_length, B, H, E, V), ptrs, ops + [h0c, wout, bout, work], tokens
+
+
+def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2):
+    """tokens (B, max_length) int64 of the greedy decode that starts from `start_token` with h0 = c0 = `h0` (B, H).
+    Not differentiable (neither is the reference's argmax): parameters are read detached."""
+    if h0.shape[0] > _LSTM_BATCH:          # independent rows: ceil(B / 64) launches of the persistent kernel
+        return torch.cat([decode_greedy(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length, start_token)
+                          for b0 in range(0, h0.shape[0], _LSTM_BATCH)], 0)
+    lib, dims, ptrs, _keep, tokens = _decode_operands(h0, lstm, word2vec, proj, max_length)
+    N.check(lib, lib.pcd_decode_greedy(*dims, start_token, *ptrs), "pcd_decode_greedy")
     return tokens
+
+
+def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None):
+    """tokens (B, max_length) int64 of the sampled decode (QstEncoder.sample with deterministic=False): every word is drawn from
+    softmax(logits / temperature), by the Gumbel-max trick on counter-based Philox noise (pcd_decode_sample).
+
+    seed: None draws one 64-bit seed per call on h0's device from torch's generator (so torch.manual_seed reproduces a run, and
+    a call captured in a CUDA graph draws a fresh seed on every replay); a Python int, or a 1-element int64 tensor on h0's
+    device read when the kernel runs, fixes the words.  Batches above 64 are decoded in slices of 64 with one seed: the noise
+    of a row depends on its index in the whole batch, so the words do not depend on the slicing.  Not differentiable."""
+    t32 = C.c_float(float(temperature)).value           # what the kernel divides by
+    if not math.isfinite(t32) or t32 <= 0.0:
+        raise ValueError(f"decode_sample: temperature must be finite and > 0, got {temperature}")
+    if seed is None:
+        seed = torch.empty(1, dtype=torch.int64, device=h0.device).random_(-2 ** 63, None)
+    elif not torch.is_tensor(seed):
+        s = int(seed) & (2 ** 64 - 1)                   # the uint64 the kernel reads, stored as int64
+        seed = torch.tensor([s - 2 ** 64 if s >= 2 ** 63 else s], dtype=torch.int64, device=h0.device)
+    elif seed.dtype != torch.int64 or seed.numel() != 1 or seed.device != h0.device:
+        raise ValueError("decode_sample: seed must be an int or a 1-element int64 tensor on the device of h0")
+    out = []
+    for b0 in range(0, h0.shape[0], _LSTM_BATCH):
+        lib, dims, ptrs, _keep, tokens = _decode_operands(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length)
+        N.check(lib, lib.pcd_decode_sample(*dims, start_token, b0, t32, N.ptr(seed), *ptrs), "pcd_decode_sample")
+        out.append(tokens)
+    return out[0] if len(out) == 1 else torch.cat(out, 0)

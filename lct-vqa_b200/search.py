@@ -151,7 +151,8 @@ def make_capturable(optimizer):
 class GraphedLctStep:
     """ArchitectLct.step (basic_vqa/pcdarts/architect_lct.py:32-92: 6 forward / 5 backward search-net passes, 3 greedy decodes,
     the W-model passes and the two finite-difference HVPs) captured once in a CUDA graph and replayed.  The learning rates are
-    baked in at capture; question sampling must be deterministic (argmax) — multinomial sampling draws on the host."""
+    baked in at capture.  Both question decoders are captured: greedy (argmax) and sampled (ef_model.qst_encoder.deterministic =
+    False, inside the decode kernel's envelope), which draws its seed on the device, so every replay samples fresh words."""
 
     def __init__(self, architect, train_batch, valid_batch, ef_lr, w_lr, warmup=2):
         self.architect = architect

@@ -16,7 +16,7 @@ import torch.nn as nn
 
 import config
 import pcd_ops
-from pcd_ops import decode_greedy, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
+from pcd_ops import decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
 from pcdarts.model_search import Network
 
 
@@ -92,14 +92,18 @@ class QstEncoder(nn.Module):
         return torch.multinomial(soft[:, 0, :], 1)
 
     def generate(self, image_embedding):
-        """Greedy 30-step decode from the <start> token (index 2)  (vqa_model.py:103-136)."""
+        """Greedy / sampled 30-step decode from the <start> token (index 2)  (vqa_model.py:103-136)."""
         batch = len(image_embedding)
         h0 = image_embedding.reshape(batch, self.hidden_size)
         if self.deterministic and decode_supported(h0, self.lstm, self.word2vec, self.fc1):
             return decode_greedy(h0, self.lstm, self.word2vec, self.fc1, self.max_length)      # one persistent kernel
+        if self.deterministic is False and decode_supported(h0, self.lstm, self.word2vec, self.fc1):
+            # the same kernel, words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
+            return decode_sample(h0, self.lstm, self.word2vec, self.fc1, self.max_length, self.temperature)
         if self.deterministic:       # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
             pcd_ops._stock(f"greedy decode with hidden size {self.hidden_size}")
-        # sampled decoding (deterministic=False) IS the reference's module loop: multinomial draws have no kernel counterpart
+        # sampled decoding outside the kernel's envelope is the reference's module loop (torch.multinomial), as is any other
+        # falsy `deterministic` with an overridden sample()
         self.lstm.flatten_parameters()
         h = image_embedding.view(1, -1, self.hidden_size)
         state = (h, h)
