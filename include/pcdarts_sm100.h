@@ -478,6 +478,40 @@ int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int ro
                       const float* b_out, long long* tokens, float* work, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Drop-path node sum of the derived network's cells (pcdarts/model.py; DARTS's drop_path on every non-Identity op output):
+ *     forward : out[b]     = d1(b) * h1[b] + d2(b) * h2[b]
+ *     backward: grad_h1[b] = d1(b) * grad_out[b],  grad_h2[b] = d2(b) * grad_out[b]     (either output may be NULL)
+ * h1, h2, out, grad_* are (batch, sample_numel) fp32, contiguous.  d_i(b) x = x when drop_i is 0, else (x / keep) * m_i(b) with
+ * IEEE division (DARTS's x.div_(keep_prob).mul_(mask), bit for bit for the same mask); the sum is one fp32 add, so with both
+ * flags off, or keep = 1, out is bit-equal to h1 + h2.  m_i(b) in {0, 1} is a pure function (pcd_philox.cuh):
+ *     x = Philox4x32-10(counter = {sample_offset + b, cell, 2 * node + i, 0x44504154}, key = {seed & 0xffffffff, seed >> 32}).word[0]
+ *     m = ((x >> 8) * 2^-24 < keep)
+ * so a sample's mask depends on its global index only: data-parallel shards (sample_offset = rank * local batch) draw what one
+ * process would draw on the whole batch.  `seed` (one uint64) and `keep` (one float) are DEVICE pointers read when the kernel
+ * runs (CUDA-graph capturable: a replay uses the values they hold then).  The backward recomputes the masks.
+ * PCD_ERR_ARG for a null seed or keep while a drop flag is set, a negative sample_offset (or sample_offset + batch >= 2^31),
+ * or a null tensor pointer; PCD_OK without a launch for an empty tensor.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct pcd_droppath_args {
+    int batch;
+    long long sample_numel;   /* C*H*W */
+    int drop1, drop2;         /* input i is subject to drop-path */
+    int cell, node;           /* position of the node in the network: counter words of the mask */
+    int sample_offset;        /* global index of sample 0 */
+    const unsigned long long* seed;
+    const float* keep;        /* 1 - drop_path_prob */
+    const float* h1;          /* forward */
+    const float* h2;
+    float* out;
+    const float* grad_out;    /* backward */
+    float* grad_h1;
+    float* grad_h2;
+} pcd_droppath_args;
+
+int pcd_droppath_sum_forward(const pcd_droppath_args* a, void* stream);
+int pcd_droppath_sum_backward(const pcd_droppath_args* a, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Optimizer-side elementwise operations over a short table of flat runs.  The search step updates all 732 parameter
  * tensors several times per step outside the network — w' = w - eta * dL/dw (darts_vqa/pcdarts/architect_vqa.py:35-38),
  * w +- R v of the finite-difference Hessian-vector product (:106-118), clip_grad_norm_ and Adam

@@ -9,6 +9,13 @@
 //     u       = ((float)(x >> 9) + 0.5f) * 2^-23                             exact in fp32, u in [2^-24, 1 - 2^-24]
 //     G       = -logf(-logf(u))                                              finite, in [-2.82, 16.7]
 // u is built from 23 bits so that it never rounds to 1 (24 bits + 0.5 would: G = +inf).
+//
+// The drop-path masks of the derived network's node sum (pcd_droppath_sum_*, csrc/pcd_droppath.cu) come from the same
+// generator, one Bernoulli(keep) draw per (sample, cell, node input):
+//     counter = { global_sample, cell, 2 * node + input, 0x44504154 }        'DPAT': disjoint from the decode noise (c3 = 0)
+//     x       = Philox4x32-10(counter, key = seed).word[0]
+//     u       = (x >> 8) * 2^-24                                             exact in fp32, u in [0, 1 - 2^-24]
+//     m       = 1 iff u < keep                                               keep = 1 never drops
 #pragma once
 #include "pcd_common.cuh"
 
@@ -43,6 +50,15 @@ PCD_HOSTDEV float gumbel_of_bits(uint32_t x) {
 PCD_HOSTDEV float decode_gumbel(unsigned long long seed, int t, int row, int v) {
     const Philox4 r = philox4x32_10((uint32_t)v >> 2, (uint32_t)t, (uint32_t)row, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
     return gumbel_of_bits(r.w[v & 3]);
+}
+
+constexpr uint32_t kDropPathStream = 0x44504154u;     // 'DPAT'
+
+// the drop-path mask m(seed, global sample, cell, slot = 2 * node + input) for keep probability `keep`: 1.f or 0.f
+PCD_HOSTDEV float droppath_mask(unsigned long long seed, int sample, int cell, int slot, float keep) {
+    const Philox4 r = philox4x32_10((uint32_t)sample, (uint32_t)cell, (uint32_t)slot, kDropPathStream, (uint32_t)seed,
+                                    (uint32_t)(seed >> 32));
+    return (float)(r.w[0] >> 8) * 0x1p-24f < keep ? 1.f : 0.f;
 }
 
 }  // namespace pcd

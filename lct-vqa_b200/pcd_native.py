@@ -94,6 +94,11 @@ class StemEvalArgs(C.Structure):
         [(n, vp) for n in ("x", "params", "running", "out")]
 
 
+class DropPathArgs(C.Structure):
+    _fields_ = [("batch", i32), ("sample_numel", i64)] + [(n, i32) for n in ("drop1", "drop2", "cell", "node", "sample_offset")] + \
+        [(n, vp) for n in ("seed", "keep", "h1", "h2", "out", "grad_out", "grad_h1", "grad_h2")]
+
+
 class DwConvArgs(C.Structure):
     _fields_ = [(n, i32) for n in ("batch", "channels", "height", "width", "kernel", "stride", "padding", "dilation",
                                    "relu_input")] + [(n, vp) for n in ("x", "weight", "out", "grad_out", "grad_x", "grad_weight")]
@@ -126,7 +131,7 @@ EXPORTS = ("pcd_launch_count", "pcd_profile_enable", "pcd_profile_num_kernels", 
            "pcd_dwconv_forward", "pcd_dwconv_backward", "pcd_pwconv_forward", "pcd_pwconv_backward", "pcd_bn_apply",
            "pcd_bn_backward_stats", "pcd_pool3x3_forward", "pcd_pool3x3_backward", "pcd_channel_affine",
            "pcd_cell_eval_work_floats", "pcd_cell_forward_eval", "pcd_mixedop_forward_eval", "pcd_preprocess_forward_eval",
-           "pcd_stem_forward_eval")
+           "pcd_stem_forward_eval", "pcd_droppath_sum_forward", "pcd_droppath_sum_backward")
 
 
 def _declare(lib):
@@ -184,6 +189,8 @@ def _declare(lib):
     for fn, st in (("pcd_cell_forward_eval", CellEvalArgs), ("pcd_mixedop_forward_eval", MixedEvalArgs),
                    ("pcd_preprocess_forward_eval", PreEvalArgs), ("pcd_stem_forward_eval", StemEvalArgs)):
         getattr(lib, fn).argtypes = [C.POINTER(st), vp]
+    for fn in ("pcd_droppath_sum_forward", "pcd_droppath_sum_backward"):
+        getattr(lib, fn).argtypes = [C.POINTER(DropPathArgs), vp]
     return lib
 
 

@@ -417,6 +417,61 @@ class AdaptiveAvgPoolFunction(torch.autograd.Function):
         return gx, None
 
 
+def _droppath_args(x, meta, **tensors):
+    drop1, drop2, keep, seed, cell, node, offset = meta
+    B = x.shape[0]
+    a = N.DropPathArgs(B, x.numel() // B if B else 0, int(drop1), int(drop2), cell, node, offset, N.ptr(seed), N.ptr(keep))
+    for k, t in tensors.items():
+        setattr(a, k, N.ptr(t))
+    return a
+
+
+class DropPathSumFunction(torch.autograd.Function):
+    """One node of a derived cell, d1 * h1 + d2 * h2 with DARTS's drop-path on the flagged inputs (pcd_droppath_sum_*)."""
+
+    @staticmethod
+    def forward(ctx, h1, h2, meta):
+        lib = N.lib_for(h1)
+        a1, a2 = _f32c(h1), _f32c(h2)
+        if a1.shape != a2.shape:
+            raise ValueError(f"droppath_sum: inputs of one node differ in shape: {tuple(a1.shape)} vs {tuple(a2.shape)}")
+        out = _empty(a1.shape, torch.float32, a1.device)
+        N.check(lib, lib.pcd_droppath_sum_forward(C.byref(_droppath_args(a1, meta, h1=a1, h2=a2, out=out)),
+                                                  N.stream_for(a1)), "pcd_droppath_sum_forward")
+        ctx.meta = meta
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        drop1, drop2 = ctx.meta[:2]
+        if not (drop1 or drop2):
+            return g, g, None
+        lib = N.lib_for(g)
+        g = _f32c(g)
+        g1 = _empty(g.shape, torch.float32, g.device) if drop1 and ctx.needs_input_grad[0] else None
+        g2 = _empty(g.shape, torch.float32, g.device) if drop2 and ctx.needs_input_grad[1] else None
+        N.check(lib, lib.pcd_droppath_sum_backward(C.byref(_droppath_args(g, ctx.meta, grad_out=g, grad_h1=g1, grad_h2=g2)),
+                                                   N.stream_for(g)), "pcd_droppath_sum_backward")
+        return (g1 if drop1 else g), (g2 if drop2 else g), None
+
+
+def droppath_sum(h1, h2, drop1, drop2, keep, seed, cell, node, sample_offset=0):
+    """node = d1 * h1 + d2 * h2 of a derived cell (pcdarts/model.py), in one kernel pass.  d_i x = (x / keep) * m_i(b) for a
+    flagged input (DARTS's drop_path: x.div_(keep_prob).mul_(mask), one Bernoulli(keep) mask per sample), else x; with no flag
+    set, or keep = 1, the result is bit-equal to h1 + h2.  The mask of sample b is a pure function of (seed, sample_offset + b,
+    cell, 2 * node + input) (include/pcdarts_sm100.h), recomputed in the backward.
+
+    keep: 1-element float32 tensor on the inputs' device, seed: 1-element int64 tensor there; both are read when the kernel
+    runs (a CUDA graph follows what they hold at replay time) and may be None when neither flag is set."""
+    if drop1 or drop2:
+        for t, dt, what in ((keep, torch.float32, "keep"), (seed, torch.int64, "seed")):
+            if not torch.is_tensor(t) or t.dtype != dt or t.numel() != 1 or t.device != h1.device:
+                raise ValueError(f"droppath_sum: {what} must be a 1-element {dt} tensor on {h1.device}")
+    if sample_offset < 0:
+        raise ValueError(f"droppath_sum: sample_offset must be >= 0, got {sample_offset}")
+    return DropPathSumFunction.apply(h1, h2, (bool(drop1), bool(drop2), keep, seed, int(cell), int(node), int(sample_offset)))
+
+
 class ChannelShuffleFunction(torch.autograd.Function):
     """channel_shuffle (model_search.py:14-28); backward is the inverse permutation."""
 

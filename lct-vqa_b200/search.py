@@ -138,6 +138,42 @@ class GraphedSearchStep:
         return self.loss
 
 
+class GraphedTrainStep:
+    """SearchStep.w_step alone (the train step of experiment.py:187-200 without an architect: the derived network after the
+    search, or the weights with the architecture frozen) captured once in a CUDA graph and replayed.  The eager step is
+    several hundred small launches with host work between them.  Inputs are copied into static device buffers.
+
+    Requirements as GraphedSearchStep: fixed shapes, an optimizer whose state lives on the device (pcd_flat.FlatAdam or a
+    torch optimizer created with capturable=True); the learning rate is baked in at capture.  Under data parallelism the
+    step's GradReducer all-reduces are captured with the rest.  The warm-up steps are UNDONE (weights, BN buffers and
+    optimizer state restored in place), so the first replay is training step 1 as in the eager path.  What the graph reads
+    from device memory follows its current value on every replay: a drawn drop-path seed is drawn anew, and a changed
+    `drop_path_prob` of a derived network takes effect without a new capture."""
+
+    def __init__(self, step, batch, warmup=3):
+        self.step_obj = step
+        self.batch = [t.clone() for t in batch]
+        side = torch.cuda.Stream(priority=-1)
+        side.wait_stream(torch.cuda.current_stream())
+        snap = _TrainingState([step.model], [], [step.optimizer])
+        with torch.cuda.stream(side):
+            for _ in range(warmup):
+                step.w_step(*self.batch)
+            snap.restore()
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph, stream=side):
+            self.loss = step.w_step(*self.batch)
+
+    def __call__(self, batch=None):
+        if batch is not None:
+            for dst, src in zip(self.batch, batch):
+                dst.copy_(src, non_blocking=True)
+        self.graph.replay()
+        return self.loss
+
+
 def make_capturable(optimizer):
     """Adam keeps `step` on the host unless capturable; flip an existing optimizer (state included) to the device form."""
     for group in optimizer.param_groups:

@@ -33,9 +33,21 @@ class DartsEncoder(nn.Module):
         return feat.div(feat.norm(p=2, dim=1, keepdim=True).detach())
 
 
+class DerivedEncoder(DartsEncoder):
+    """The network DERIVED from a searched genotype (pcdarts/model.py NetworkDerived) -> Linear -> x / ||x||_2.detach(): the
+    image encoder of the VQA model trained after the search.  The network sits under the same attribute name, `darts`."""
+
+    def __init__(self, embed_size, network):
+        nn.Module.__init__(self)
+        self.darts = network
+        self.fc = nn.Linear(network.output_ch * network.output_size ** 2, embed_size)
+
+
 def get_img_encoder(img_encoder_type, embed_size):
     if img_encoder_type == 'darts':
         return DartsEncoder(embed_size)
+    if img_encoder_type == 'derived':
+        raise ValueError("a derived image encoder is built from a search model: vqa_model.derive_vqa(search_model)")
     if img_encoder_type == 'vgg':
         raise NotImplementedError("the VGG19 encoder (vqa_model.py:8-45) is outside the PC-DARTS search path")
     raise Exception(f'Unrecognized encoder type: {img_encoder_type}')
@@ -201,3 +213,17 @@ class VqaModel(VqaModelBase):
         if qst_only:
             return qst_loss, img_feature
         return self.criterion(self._answer(img_feature, qst_feature), labels) + qst_loss, img_feature
+
+
+def derive_vqa(search_model, layers=None):
+    """A freshly initialised VqaModel with the dimensions of `search_model` whose image encoder is the network its genotype
+    describes (pcdarts.model.derive; `layers` overrides the depth).  As in DARTS, the derived network is trained from
+    scratch: nothing but the genotype is taken over.  genotype() returns it, arch_parameters() is empty.  new() (the unrolled
+    twin of an architecture search) does not apply."""
+    from pcdarts.model import derive
+    m = VqaModel(search_model.embed_size, search_model.qst_vocab_size, search_model.ans_vocab_size,
+                 search_model.word_embed_size, search_model.num_layers, search_model.hidden_size, img_encoder_type='darts')
+    m.img_encoder = DerivedEncoder(search_model.embed_size, derive(search_model.img_encoder.darts, layers))
+    m.img_encoder_type = 'derived'
+    device = next(search_model.parameters()).device
+    return m.to(device)
