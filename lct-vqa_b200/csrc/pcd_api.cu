@@ -106,40 +106,39 @@ struct EdgeGeom {
 
 static bool aligned16(const void* p) { return (((uintptr_t)p) & 15) == 0; }
 
-// preconditions of the compile-time-tile ("FAST") specialisations: the tile picked for this geometry is one of
-// the fixed ones, tiles are full and span the whole image width, every row of every tensor touched starts 16-byte aligned
-static bool fast_ok(const EdgeGeom& q, const Tile& t, bool stageB) {
-    return edge_tile_is_fixed(q.c, q.S, t.TH, t.TW, stageB) && q.Ho % t.TH == 0 && q.Wo == t.TW && q.Ws == q.S * q.Wo &&
-           q.Hs == q.S * q.Ho && q.Ws % 4 == 0;
+// The five production edge shapes run the v4 forward (pcd_edge_v4.cuh), the stage-B data and weight-gradient kernels of
+// pcd_edge_bwd2.cuh and the v4 stage-A backward (pcd_edge_bwd4.cuh); every other geometry runs the generic kernels of
+// pcd_edge.cuh.  fwd4_supported implies Ho % 16 == 0, so bwd2_tile holds as well.  A production geometry with a pointer
+// that is not 16-byte aligned is an error (PCD_ERR_ALIGN), not a fall-back: the arenas handed to the cell / MixedOp
+// entry points are 16-byte aligned by contract.
+static bool edge_is_production(const EdgeGeom& q) {
+    return q.Hs == q.S * q.Ho && q.Ws == q.S * q.Wo && q.Ws % 4 == 0 && fwd4_supported(q.c, q.S, q.Ho, q.Wo);
 }
 
 static int run_passAB(const EdgeGeom& q, const EdgeF* edges, int n, float eps, int save_t, void* stream) {
     if (n == 0) return PCD_OK;
     if (n > kMaxEdgesPerLaunch) return PCD_ERR_ARG;
-    PassArgs a;
-    memset(&a, 0, sizeof a);
-    a.B = q.B; a.Hs = q.Hs; a.Ws = q.Ws; a.Ho = q.Ho; a.Wo = q.Wo; a.S = q.S; a.eps = eps; a.nedges = n;
-    bool al = true;
-    for (int i = 0; i < n; ++i) {
-        a.e[i] = edges[i];
-        al = al && aligned16(edges[i].x) && aligned16(edges[i].saved) && edges[i].x_ns % 4 == 0;
-    }
-    // production geometries: the v4 kernels (one block runs every stage-A job from one staged tile)
-    bool al4 = al;
-    for (int i = 0; i < n; ++i) al4 = al4 && aligned16(edges[i].par);
-    if (al4 && q.Hs == q.S * q.Ho && q.Ws == q.S * q.Wo && fwd4_supported(q.c, q.S, q.Ho, q.Wo) && !getenv("PCD_NO_V4")) {
+    if (edge_is_production(q)) {      // one block runs every stage-A job from one staged tile
         FwdV4Args v;
         memset(&v, 0, sizeof v);
         v.B = q.B; v.Hs = q.Hs; v.Ws = q.Ws; v.Ho = q.Ho; v.Wo = q.Wo; v.eps = eps; v.nedges = n; v.save_t = save_t; v.jobs = 1;
-        for (int i = 0; i < n; ++i) v.e[i] = edges[i];
+        for (int i = 0; i < n; ++i) {
+            if (!aligned16(edges[i].x) || !aligned16(edges[i].saved) || !aligned16(edges[i].par) || edges[i].x_ns % 4)
+                return PCD_ERR_ALIGN;
+            v.e[i] = edges[i];
+        }
         return launch_fwd4(v, q.c, q.S, stream);
     }
+    PassArgs a;
+    memset(&a, 0, sizeof a);
+    a.B = q.B; a.Hs = q.Hs; a.Ws = q.Ws; a.Ho = q.Ho; a.Wo = q.Wo; a.S = q.S; a.eps = eps; a.nedges = n;
+    for (int i = 0; i < n; ++i) a.e[i] = edges[i];
     Tile t = pick_tile(q.Ho, q.Wo, q.c, q.S == 1 ? 4096 : 2048);
     a.TH = t.TH; a.TW = t.TW; a.tiles_x = t.tiles_x;
-    PCD_TRY(launch_fwdA(a, q.c, al && fast_ok(q, t, false), t.tiles_x * t.tiles_y, q.B, n * kFwdAJobs, stream));
+    PCD_TRY(launch_fwdA(a, q.c, t.tiles_x * t.tiles_y, q.B, n * kFwdAJobs, stream));
     Tile tb = pick_tile(q.Ho, q.Wo, q.c, 4096);
     a.TH = tb.TH; a.TW = tb.TW; a.tiles_x = tb.tiles_x;
-    PCD_TRY(launch_fwdB(a, q.c, al && fast_ok(q, tb, true), tb.tiles_x * tb.tiles_y, q.B, n * 2, stream));
+    PCD_TRY(launch_fwdB(a, q.c, tb.tiles_x * tb.tiles_y, q.B, n * 2, stream));
     return PCD_OK;
 }
 
@@ -180,20 +179,7 @@ static void fill_edge_bwd_args(EdgeBwdArgs& a, const EdgeGeom& q, const EdgeG* e
     }
 }
 
-// does this edge geometry run the v3 backward kernels (merged partial-grad slots)?  Pointer alignment is checked again
-// at launch; the arenas handed to the cell / MixedOp entry points are 16-byte aligned by contract.
-static bool edge_bwd_is_v3(const EdgeGeom& q) {
-    int thA = 0, thB = 0;
-    return q.Ws % 4 == 0 && q.Hs == q.S * q.Ho && q.Ws == q.S * q.Wo && bwd2_tile(q.c, q.S, q.Ho, q.Wo, &thA) &&
-           bwd2_tile(q.c, 1, q.Ho, q.Wo, &thB);
-}
-
-// v4 stage-A data kernels (plain stores into the partial-grad slots: no memset, no reductions)
-static bool edge_bwd_is_v4(const EdgeGeom& q) {
-    return edge_bwd_is_v3(q) && fwd4_supported(q.c, q.S, q.Ho, q.Wo) && !getenv("PCD_NO_V4");
-}
-
-// v3 weight-gradient jobs for edges whose data jobs already ran (any number of edges, one stride)
+// weight-gradient jobs of production-geometry edges whose data jobs already ran (any number of edges, one stride)
 static int run_edge_wgrad2(const EdgeGeom& q, const EdgeG* edges, int n, float eps, void* stream) {
     int thA = 0;
     if (!bwd2_tile(q.c, q.S, q.Ho, q.Wo, &thA)) return PCD_ERR_UNSUPPORTED;
@@ -208,34 +194,26 @@ static int run_edge_wgrad2(const EdgeGeom& q, const EdgeG* edges, int n, float e
     return PCD_OK;
 }
 
-// Backward of a group of edges with one geometry.  Production geometries run the v3 data kernels; their weight
-// gradients are either launched here (defer == nullptr) or left to the caller (*defer set to 1), which batches
-// them over the whole cell.  Other geometries run the generic v2 kernels (weight grads inline).
+// Backward of a group of edges with one geometry.  Production geometries run bwdB2 + bwdA4, which leave two slots in
+// every edge's pd, the first already ReLU-masked (SrcEdge::merged); their weight gradients are either launched here
+// (defer == nullptr) or left to the caller (*defer set to 1), which batches them over the whole cell.  Other geometries
+// run the generic kernels (one pd slot per job, weight grads inline).
 static int run_edge_bwd(const EdgeGeom& q, const EdgeG* edges, int n, float eps, int need_wgrad, void* stream,
-                        int* defer = nullptr, int* merged = nullptr) {
+                        int* defer = nullptr) {
     if (defer) *defer = 0;
-    if (merged) *merged = 0;
     if (n == 0) return PCD_OK;
     if (n > kMaxEdgesPerLaunch) return PCD_ERR_ARG;
     EdgeBwdArgs a;
     bool al;
     fill_edge_bwd_args(a, q, edges, n, eps, need_wgrad, &al);
-    int thA = 0, thB = 0;
-    if (edge_bwd_is_v3(q)) {
+    if (edge_is_production(q)) {
         if (!al) return PCD_ERR_ALIGN;
-        bwd2_tile(q.c, q.S, q.Ho, q.Wo, &thA);
+        int thB = 0;
         bwd2_tile(q.c, 1, q.Ho, q.Wo, &thB);
         a.need_wgrad = 0;
         a.TH = thB; a.TW = q.Wo; a.tiles_x = 1;
         PCD_TRY(launch_bwdB2(a, q.c, n * 2, stream));
-        a.TH = thA;
-        if (edge_bwd_is_v4(q)) {
-            if (merged) *merged = 2;     // edges[i].pd: two slots written with plain stores, ReLU mask already applied to slot 0
-            PCD_TRY(launch_bwdA4(a, q.c, n, stream));
-        } else {
-            if (merged) *merged = 1;     // edges[i].pd: two zeroed slots accumulated with reductions (caller's job)
-            PCD_TRY(launch_bwdA2(a, q.c, n * bwdA_njobs(q.S), stream));
-        }
+        PCD_TRY(launch_bwdA4(a, q.c, n, stream));
         if (need_wgrad) {
             if (defer) *defer = 1;
             else PCD_TRY(run_edge_wgrad2(q, edges, n, eps, stream));
@@ -244,10 +222,10 @@ static int run_edge_bwd(const EdgeGeom& q, const EdgeG* edges, int n, float eps,
     }
     Tile tb = pick_tile(q.Ho, q.Wo, q.c, 4096);
     a.TH = tb.TH; a.TW = tb.TW; a.tiles_x = tb.tiles_x;
-    PCD_TRY(launch_bwdB(a, q.c, al && fast_ok(q, tb, true), tb.tiles_x * tb.tiles_y, q.B, n * 2, stream));
+    PCD_TRY(launch_bwdB(a, q.c, tb.tiles_x * tb.tiles_y, q.B, n * 2, stream));
     Tile t = pick_tile(q.Ho, q.Wo, q.c, q.S == 1 ? 4096 : 2048);
     a.TH = t.TH; a.TW = t.TW; a.tiles_x = t.tiles_x;
-    PCD_TRY(launch_bwdA(a, q.c, al && fast_ok(q, t, false), t.tiles_x * t.tiles_y, q.B, n * bwdA_njobs(q.S), stream));
+    PCD_TRY(launch_bwdA(a, q.c, t.tiles_x * t.tiles_y, q.B, n * bwdA_njobs(q.S), stream));
     return PCD_OK;
 }
 
@@ -313,7 +291,6 @@ struct CellLayout {
     int node_of[PCD_MAX_EDGES], src_of[PCD_MAX_EDGES], stride[PCD_MAX_EDGES], first_edge[PCD_MAX_STEPS];
     long long par[PCD_MAX_EDGES], run[PCD_MAX_EDGES], nbt[PCD_MAX_EDGES], stats[PCD_MAX_EDGES], bstats[PCD_MAX_EDGES];
     long long saved[PCD_MAX_EDGES], ga[PCD_MAX_EDGES], dxs[PCD_MAX_EDGES];
-    long long pd2[PCD_MAX_EDGES], pd2_begin, pd2_floats;     // v3: two merged partial-grad slots per edge, contiguous over the cell
     long long pre_par[2], pre_run[2], pre_nbt[2], pre_stats[2], pre_bstats[2], pre_out[2], pre_dout[2];
     long long dn[PCD_MAX_STEPS];
     pcd_cell_sizes tot;
@@ -364,12 +341,6 @@ static int cell_layout(const pcd_cell_shape& s, CellLayout& L) {
     }
     const long long node = (long long)L.B * L.C * L.Ho * L.Wo;
     for (int i = 0; i < 3; ++i) { L.dn[i] = wk; wk += node; }
-    L.pd2_begin = wk;
-    for (int k = 0; k < PCD_MAX_EDGES; ++k) {
-        const long long in_px = (long long)L.B * c * (L.stride[k] == 2 ? L.Hs * L.Ws : L.Ho * L.Wo);
-        L.pd2[k] = wk; wk += 2 * in_px;
-    }
-    L.pd2_floats = wk - L.pd2_begin;
     L.tot.param_floats = par; L.tot.running_floats = run; L.tot.nbt_int64 = nbt;
     L.tot.out_floats = 4 * node; L.tot.saved_floats = sv; L.tot.stats_doubles = st;
     L.tot.bwd_work_floats = wk; L.tot.bwd_stats_doubles = bst;
@@ -547,22 +518,11 @@ int pcd_cell_backward(const pcd_cell_bwd_args* a, void* stream) {
     const long long node = (long long)L.B * L.C * L.Ho * L.Wo;
     PCD_TRY(zero_async(a->bstats, L.tot.bwd_stats_doubles * sizeof(double), stream));
     if (a->need_param_grads) PCD_TRY(zero_async(a->grad_params, L.tot.param_floats * sizeof(float), stream));
-    {   // merged partial-grad slots: the v3 data kernels accumulate into them (zero first); the v4 kernels store
-        bool all_v4 = true;
-        for (int e = 0; e < PCD_MAX_EDGES; ++e) {
-            StateRef s = state_ref(L, a->saved, a->out, L.src_of[e]);
-            EdgeGeom q;
-            q.B = L.B; q.c = L.c; q.S = L.stride[e]; q.Hs = s.H; q.Ws = s.W; q.Ho = L.Ho; q.Wo = L.Wo;
-            all_v4 = all_v4 && edge_bwd_is_v4(q);
-        }
-        if (!all_v4) PCD_TRY(zero_async(a->work + L.pd2_begin, L.pd2_floats * sizeof(float), stream));
-    }
     auto dn_ptr = [&](int i, long long& ns) -> const float* {
         if (i == 3) { ns = 4 * (node / L.B); return a->grad_out + 3 * (node / L.B); }
         ns = node / L.B;
         return a->work + L.dn[i];
     };
-    int edge_merged[PCD_MAX_EDGES] = {0};
     EdgeG wq[2][PCD_MAX_EDGES];          // edges whose weight-grad jobs are deferred, by stride
     EdgeGeom wgeo[2];
     int nwq[2] = {0, 0};
@@ -601,15 +561,12 @@ int pcd_cell_backward(const pcd_cell_bwd_args* a, void* stream) {
             eg[n].beta = a->weights2 + e;
             eg[n].ga = a->work + L.ga[e];
             q.S = L.stride[e]; q.Hs = s.H; q.Ws = s.W;
-            eg[n].pd = a->work + (edge_bwd_is_v3(q) ? L.pd2[e] : L.dxs[e]);
+            eg[n].pd = a->work + L.dxs[e];
             ++n;
         }
-        int deferred = 0, merged = 0;
-        PCD_TRY(run_edge_bwd(q, eg, n, eps, a->need_param_grads, stream, &deferred, &merged));
-        for (int e = 0; e < PCD_MAX_EDGES; ++e) {
-            const int j = L.src_of[e];
-            if (!((i == 0) ? (j >= 2) : (j != i + 1))) edge_merged[e] = merged;
-        }
+        int deferred = 0;
+        PCD_TRY(run_edge_bwd(q, eg, n, eps, a->need_param_grads, stream, &deferred));
+        const int merged = edge_is_production(q);      // layout of the pd slots of this wave's edges, read in step 3
         if (deferred && n > 0) {
             const int g = q.S - 1;
             wgeo[g] = q;
@@ -635,8 +592,8 @@ int pcd_cell_backward(const pcd_cell_bwd_args* a, void* stream) {
                 if (m >= kMaxSrcEdges) return PCD_ERR_ARG;
                 long long cns;
                 const float* cdn = dn_ptr(L.node_of[e], cns);
-                sg.e[m].pd = a->work + (edge_merged[e] ? L.pd2[e] : L.dxs[e]); sg.e[m].dn = cdn; sg.e[m].dn_ns = cns;
-                sg.e[m].beta = a->weights2 + e; sg.e[m].stride = L.stride[e]; sg.e[m].merged = edge_merged[e];
+                sg.e[m].pd = a->work + L.dxs[e]; sg.e[m].dn = cdn; sg.e[m].dn_ns = cns;
+                sg.e[m].beta = a->weights2 + e; sg.e[m].stride = L.stride[e]; sg.e[m].merged = merged;
                 ++m;
             }
             sg.nedges = m;
@@ -746,15 +703,13 @@ int pcd_mixedop_backward(const pcd_mixedop_bwd_args* a, void* stream) {
     eg.x = a->x; eg.x_ns = es.x_ns; eg.dn = a->grad_out; eg.dn_ns = C * q.Ho * q.Wo; eg.saved = a->saved; eg.stats = a->stats;
     eg.bstats = a->bstats; eg.par = a->params; eg.gpar = a->need_param_grads ? a->grad_params : nullptr;
     eg.alpha = a->weights; eg.beta = nullptr; eg.ga = a->work; eg.pd = a->work + 2 * q.nslot();
-    int merged = 0;
-    if (edge_bwd_is_v3(q) && !edge_bwd_is_v4(q)) PCD_TRY(zero_async(eg.pd, (size_t)2 * q.B * q.c * q.Hs * q.Ws * sizeof(float), stream));
-    PCD_TRY(run_edge_bwd(q, &eg, 1, a->shape.bn_eps, a->need_param_grads, stream, nullptr, &merged));
+    PCD_TRY(run_edge_bwd(q, &eg, 1, a->shape.bn_eps, a->need_param_grads, stream));
     SourceGradArgs sg;
     memset(&sg, 0, sizeof sg);
     sg.B = q.B; sg.C = (int)C; sg.Hs = q.Hs; sg.Ws = q.Ws; sg.x = a->x; sg.x_ns = es.x_ns; sg.g0 = nullptr;
     sg.out = a->grad_x; sg.out_ns = es.x_ns; sg.nedges = 1;
     sg.e[0].pd = eg.pd; sg.e[0].dn = a->grad_out; sg.e[0].dn_ns = eg.dn_ns; sg.e[0].beta = nullptr; sg.e[0].stride = q.S;
-    sg.e[0].merged = merged;
+    sg.e[0].merged = edge_is_production(q);
     PCD_TRY(run_source_grad(sg, stream));
     ArchGradArgs ag;
     memset(&ag, 0, sizeof ag);

@@ -154,8 +154,8 @@ struct SrcEdge {
     long long dn_ns;
     const float* beta;     // null => 1
     int stride;
-    int merged;            // 1: slot 0 = sum of the pre-mask partials (A3 A5 D3 D5 FR), slot 1 = max-pool + avg-pool(+identity)
-                           // 2: the same two slots, the ReLU mask already applied to slot 0 by its producer (v4 backward)
+    int merged;            // set: the two slots of the production backward (bwdA4): slot 0 = the ReLU-masked sum of the conv / FR
+                           // partials, slot 1 = max-pool + avg-pool(+identity).  Clear: the generic kernels' per-job slots
 };
 
 constexpr int kMaxSrcEdges = 4;
@@ -211,7 +211,7 @@ PCD_HD void source_grad_body(const SourceGradArgs& a, int bx, int ch, int nz) {
     }
     float bs = 0.f, bq = 0.f;          // BatchNorm-backward partial sums (bn_sums): per thread; the emulation loops once per block
     if (ch < c && vec && all_merged) {
-        // production path: every load of a task (2 per edge + mask + initial grad) is issued before the first use
+        // production path: every load of a task (2 per edge + x + initial grad) is issued before the first use
         PCD_FOR(tt, nimg * tpp) {
             const int n = n0 + tt / tpp, i4 = tt % tpp;
             if (n >= a.B) continue;
@@ -230,11 +230,10 @@ PCD_HD void source_grad_body(const SourceGradArgs& a, int bx, int ch, int nz) {
 #pragma unroll
             for (int k = 0; k < kMaxSrcEdges; ++k)
                 if (k < a.nedges) {
-                    const bool pre = a.e[k].merged == 2;        // mask already applied
-                    v.x += ((pre || xv.x > 0.f) ? m[k].x : 0.f) + q4[k].x;
-                    v.y += ((pre || xv.y > 0.f) ? m[k].y : 0.f) + q4[k].y;
-                    v.z += ((pre || xv.z > 0.f) ? m[k].z : 0.f) + q4[k].z;
-                    v.w += ((pre || xv.w > 0.f) ? m[k].w : 0.f) + q4[k].w;
+                    v.x += m[k].x + q4[k].x;
+                    v.y += m[k].y + q4[k].y;
+                    v.z += m[k].z + q4[k].z;
+                    v.w += m[k].w + q4[k].w;
                 }
             *reinterpret_cast<F4*>(a.out + (long long)n * a.out_ns + (long long)ch * HW + p) = v;
             bs += (v.x + v.y) + (v.z + v.w);
@@ -258,11 +257,10 @@ PCD_HD void source_grad_body(const SourceGradArgs& a, int bx, int ch, int nz) {
                 const float* pd = e.pd + ((long long)n * c + ch) * HW + p;
                 if (e.merged) {
                     const F4 m = *reinterpret_cast<const F4*>(pd), q4 = *reinterpret_cast<const F4*>(pd + pslot);
-                    const bool pre = e.merged == 2;
-                    v.x += ((pre || xv.x > 0.f) ? m.x : 0.f) + q4.x;
-                    v.y += ((pre || xv.y > 0.f) ? m.y : 0.f) + q4.y;
-                    v.z += ((pre || xv.z > 0.f) ? m.z : 0.f) + q4.z;
-                    v.w += ((pre || xv.w > 0.f) ? m.w : 0.f) + q4.w;
+                    v.x += m.x + q4.x;
+                    v.y += m.y + q4.y;
+                    v.z += m.z + q4.z;
+                    v.w += m.w + q4.w;
                     continue;
                 }
                 F4 m = {0.f, 0.f, 0.f, 0.f};
@@ -380,7 +378,7 @@ PCD_HD void source_grad_body(const SourceGradArgs& a, int bx, int ch, int nz) {
             if (ch < c) {
                 const float* pd = e.pd + ((long long)n * c + ch) * HW + p;
                 if (e.merged) {
-                    v += ((e.merged == 2 || xb[p] > 0.f) ? pd[0] : 0.f) + pd[pslot];
+                    v += pd[0] + pd[pslot];
                     continue;
                 }
                 float m = pd[0] + pd[pslot] + pd[2 * pslot] + pd[3 * pslot];

@@ -9,9 +9,10 @@
 // Splitting by job instead of looping over the candidate ops inside a block multiplies the number of
 // resident blocks (B=64 gives only 64..256 tiles per edge) and keeps shared memory per block small.
 //
-// Template <C, S, FTH, FTW>: FTH/FTW != 0 fixes the tile at compile time (production shapes: every
-// index expression folds to shifts/constants, tiles are full, rows are float4-aligned).  FTH == 0 is the
-// generic path (run-time tile, masked edges) used for any other shape.
+// These are the generic kernels (run-time tile, masked edges): they run every edge geometry except the five
+// production edge shapes, which take the v4 forward (pcd_edge_v4.cuh), the stage-B backward and weight-gradient
+// kernels of pcd_edge_bwd2.cuh and the v4 stage-A backward (pcd_edge_bwd4.cuh).  This file also holds the argument
+// structs and the small building blocks those kernels share.
 #pragma once
 #include "pcd_common.cuh"
 
@@ -41,15 +42,9 @@ PCD_HD long long out_index(const Geo& g, int C, int ch, int oy, int ox) {
     return (((long long)g.n * C + ch) * g.Ho + oy) * g.Wo + ox;
 }
 
-// store 4 consecutive pixels of row oy starting at ox; FAST: tiles are full and rows 16-byte aligned
-template <bool FAST>
+// store 4 consecutive pixels of row oy starting at ox (the part inside the image)
 PCD_HD void store4(float* base, const Geo& g, int C, int ch, int oy, int ox, const float (&v)[4]) {
     float* p = base + out_index(g, C, ch, oy, ox);
-    if (FAST) {
-        F4 t = {v[0], v[1], v[2], v[3]};
-        *reinterpret_cast<F4*>(p) = t;
-        return;
-    }
     if (oy >= g.Ho) return;
     if (ox + 3 < g.Wo && (((uintptr_t)p) & 15) == 0) {
         F4 t = {v[0], v[1], v[2], v[3]};
@@ -61,10 +56,9 @@ PCD_HD void store4(float* base, const Geo& g, int C, int ch, int oy, int ox, con
     }
 }
 
-// 4 consecutive pixels of an image row; zero outside [0,W).  FAST => caller guarantees 0 <= x, x+3 < W, aligned.
-template <bool FAST>
+// 4 consecutive pixels of an image row; zero outside [0,W)
 PCD_HD void load4(const float* row, int x, int W, float (&v)[4]) {
-    if (FAST || (x >= 0 && x + 3 < W && (((uintptr_t)(row + x)) & 15) == 0)) {
+    if (x >= 0 && x + 3 < W && (((uintptr_t)(row + x)) & 15) == 0) {
         const F4 t = *reinterpret_cast<const F4*>(row + x);
         v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
     } else {
@@ -74,7 +68,7 @@ PCD_HD void load4(const float* row, int x, int W, float (&v)[4]) {
 }
 
 // dst[C][rows][pitch] <- f(ch, src[ch*cs + gy*W + gx]) inside the image, 0 outside.  gx0 is a multiple of 4.
-template <bool FAST, class F>
+template <class F>
 PCD_HD void load_tile(float* dst, const float* src, long long cs, int C, int rows, int pitch, int gy0, int gx0, int H,
                       int W, F f) {
     const int p4 = pitch >> 2;
@@ -83,12 +77,10 @@ PCD_HD void load_tile(float* dst, const float* src, long long cs, int C, int row
         const int gy = gy0 + r, gx = gx0 + 4 * c4;
         float v[4] = {0.f, 0.f, 0.f, 0.f};
         if (gy >= 0 && gy < H && gx + 3 >= 0 && gx < W) {
-            const float* row = src + ch * cs + (long long)gy * W;
-            if (FAST) load4<true>(row, gx, W, v);       // W % 4 == 0: a group is entirely inside or outside
-            else load4<false>(row, gx, W, v);
+            load4(src + ch * cs + (long long)gy * W, gx, W, v);
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                if (FAST || (gx + j >= 0 && gx + j < W)) v[j] = f(ch, v[j]);
+                if (gx + j >= 0 && gx + j < W) v[j] = f(ch, v[j]);
         }
         F4 t = {v[0], v[1], v[2], v[3]};
         *reinterpret_cast<F4*>(dst + (size_t)i * 4) = t;
@@ -125,14 +117,6 @@ PCD_HD void st4(float* p, float a, float b, float c, float d) {
     F4 t = {a, b, c, d};
     *reinterpret_cast<F4*>(p) = t;
 }
-// p[0..3] += (a, b, c, d), no return value: one 16-byte reduction at the L2 (sm_90+)
-PCD_HD void red4(float* p, float a, float b, float c, float d) {
-#if PCD_CUDA
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-#else
-    p[0] += a; p[1] += b; p[2] += c; p[3] += d;
-#endif
-}
 
 // 16-byte global -> shared copy that does not occupy a register (cp.async; zero fill when !valid); cp16_wait() makes this
 // thread's copies visible to it (a barrier then publishes them to the block)
@@ -152,62 +136,11 @@ PCD_HD void cp16_wait() {
 #endif
 }
 
-// Tile rows that span the full image width W (the compile-time-tile kernels): dst[C][ROWS][W + 8] <- f(ch, src row),
-// image rows gy0 .. gy0 + ROWS - 1 (zero outside the image); the two 4-float column halos are zero padding.
-template <int C, int ROWS, int W, class F>
-PCD_HD void load_rows_full(float* dst, const float* PCD_RESTRICT src, long long cs, int gy0, int H, F f) {
-    constexpr int W4 = W / 4, P = W + 8;
-    static_assert((W4 & (W4 - 1)) == 0, "row width must be a power-of-two number of float4");
-    for_tasks<C * ROWS * W4>([&](int i) {
-        const int x4 = i % W4, row = i / W4, ch = row / ROWS, r = row - ch * ROWS;
-        const int gy = gy0 + r;
-        F4 v = {0.f, 0.f, 0.f, 0.f};
-        if (gy >= 0 && gy < H) {
-            v = ld4(src + ch * cs + (long long)gy * W + 4 * x4);
-            v.x = f(ch, v.x); v.y = f(ch, v.y); v.z = f(ch, v.z); v.w = f(ch, v.w);
-        }
-        *reinterpret_cast<F4*>(dst + row * P + 4 + 4 * x4) = v;
-    });
-    for_tasks<C * ROWS * 2>([&](int i) {
-        const int row = i >> 1;
-        st4(dst + row * P + ((i & 1) ? 4 + W : 0), 0.f, 0.f, 0.f, 0.f);
-    });
-}
-
-// the same in two steps: raw rows with cp.async (no registers, no dependence on f's constants), then f in place
-template <int C, int ROWS, int W>
-PCD_HD void stage_rows_full(float* dst, const float* PCD_RESTRICT src, long long cs, int gy0, int H) {
-    constexpr int W4 = W / 4, P = W + 8;
-    static_assert((W4 & (W4 - 1)) == 0, "row width must be a power-of-two number of float4");
-    for_tasks<C * ROWS * W4>([&](int i) {
-        const int x4 = i % W4, row = i / W4, ch = row / ROWS, r = row - ch * ROWS;
-        const int gy = gy0 + r;
-        const bool ok = gy >= 0 && gy < H;
-        cp16(dst + row * P + 4 + 4 * x4, ok ? src + ch * cs + (long long)gy * W + 4 * x4 : src, ok);
-    });
-    for_tasks<C * ROWS * 2>([&](int i) {
-        const int row = i >> 1;
-        st4(dst + row * P + ((i & 1) ? 4 + W : 0), 0.f, 0.f, 0.f, 0.f);
-    });
-}
-template <int C, int ROWS, int W, class F>
-PCD_HD void apply_rows_full(float* dst, int gy0, int H, F f) {
-    constexpr int W4 = W / 4, P = W + 8;
-    for_tasks<C * ROWS * W4>([&](int i) {
-        const int x4 = i % W4, row = i / W4, ch = row / ROWS, r = row - ch * ROWS;
-        const int gy = gy0 + r;
-        if (gy >= 0 && gy < H) {
-            F4 v = ld4(dst + row * P + 4 + 4 * x4);
-            st4(dst + row * P + 4 + 4 * x4, f(ch, v.x), f(ch, v.y), f(ch, v.z), f(ch, v.w));
-        }
-    });
-}
-
 // ======================================================================================================
 // forward
 // ======================================================================================================
 // One depthwise->pointwise unit on a shared-memory input tile [C][rows][pitch] (col halo 4, row halo halo_y).
-template <int C, int KS, int DIL, int S, bool RELU, bool FAST>
+template <int C, int KS, int DIL, int S, bool RELU>
 PCD_HD void unit_forward(const float* tile, int rows, int pitch, int halo_y, const float* w_dw, const float* w_pw,
                          float* T, float* P, float* P2, float* WS, float* t_out, float* z_out, double* st, const Geo& g) {
     constexpr int PAD = DIL * (KS - 1) / 2;
@@ -228,7 +161,7 @@ PCD_HD void unit_forward(const float* tile, int rows, int pitch, int halo_y, con
         for (int i = 0; i < 4; ++i) {
             F4 v = {acc[i][0], acc[i][1], acc[i][2], acc[i][3]};
             *reinterpret_cast<F4*>(T + ch * NPIX + (py + i) * TW + px) = v;
-            store4<FAST>(t_out, g, C, ch, g.oy0 + py + i, g.ox0 + px, acc[i]);
+            store4(t_out, g, C, ch, g.oy0 + py + i, g.ox0 + px, acc[i]);
         }
     }
     PCD_SYNC();
@@ -262,11 +195,11 @@ PCD_HD void unit_forward(const float* tile, int rows, int pitch, int halo_y, con
         const int oy = g.oy0 + oyl, ox = g.ox0 + oxl;
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            store4<FAST>(z_out, g, C, cg * 4 + i, oy, ox, z[i]);
+            store4(z_out, g, C, cg * 4 + i, oy, ox, z[i]);
             float s = 0.f, q = 0.f;
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                if (FAST || (oy < g.Ho && ox + j < g.Wo)) {
+                if (oy < g.Ho && ox + j < g.Wo) {
                     s += z[i][j];
                     q = fmaf(z[i][j], z[i][j], q);
                 }
@@ -290,10 +223,9 @@ PCD_HOSTDEV size_t fwdA_smem_floats(int C, int S, int TH, int TW) {
     return (size_t)C * IH * IW + (size_t)C * TH * TW * 2 + 4 * C * fwd_np(C) + C * C + 64;
 }
 
-template <int C, int S, int FTH, int FTW>
+template <int C, int S>
 PCD_HD void fwdA_body(const PassArgs& a, int bx, int n, int z, float* smem) {
-    constexpr bool FAST = FTH != 0;
-    const int TH = FTH ? FTH : a.TH, TW = FTW ? FTW : a.TW;
+    const int TH = a.TH, TW = a.TW;
     const int ez = z / kFwdAJobs, job = z - ez * kFwdAJobs;
     const EdgeF& e = a.e[ez];
     Geo g;
@@ -308,21 +240,14 @@ PCD_HD void fwdA_body(const PassArgs& a, int bx, int n, int z, float* smem) {
     float* P2 = P + C * NPIX;
     float* WS = P2 + 4 * C * fwd_np(C);
     const long long nslot = (long long)a.B * C * a.Ho * a.Wo;
-    if (FAST) {      // full-width tile; the conv jobs get relu(x) (applied once here), the pool job the raw tile
-        constexpr int FIH = S * (FTH ? FTH : 4) + 8, FW = S * (FTW ? FTW : 4);
-        const float* src = e.x + (long long)n * e.x_ns;
-        if (job < 4) load_rows_full<C, FIH, FW>(XIN, src, (long long)a.Hs * a.Ws, S * g.oy0 - 4, a.Hs, [](int, float v) { return relu(v); });
-        else load_rows_full<C, FIH, FW>(XIN, src, (long long)a.Hs * a.Ws, S * g.oy0 - 4, a.Hs, [](int, float v) { return v; });
-    } else {
-        load_tile<FAST>(XIN, e.x + (long long)n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, IW, S * g.oy0 - 4, S * g.ox0 - 4,
-                        a.Hs, a.Ws, [](int, float v) { return v; });
-    }
+    load_tile(XIN, e.x + (long long)n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, IW, S * g.oy0 - 4, S * g.ox0 - 4, a.Hs, a.Ws,
+              [](int, float v) { return v; });
     PCD_SYNC();
 
 #define PCD_UNIT_A(U, KS, DIL)                                                                                     \
-    unit_forward<C, KS, DIL, S, !FAST, FAST>(XIN, IH, IW, 4, e.par + edge_dw_off(C, S, U), e.par + edge_pw_off(C, S, U), \
-                                            T, P, P2, WS, e.saved + slot_t(U) * nslot, e.saved + slot_z(U) * nslot, \
-                                            e.stats + bn_unit(S, U) * 2 * C, g)
+    unit_forward<C, KS, DIL, S, true>(XIN, IH, IW, 4, e.par + edge_dw_off(C, S, U), e.par + edge_pw_off(C, S, U),  \
+                                      T, P, P2, WS, e.saved + slot_t(U) * nslot, e.saved + slot_z(U) * nslot,       \
+                                      e.stats + bn_unit(S, U) * 2 * C, g)
     if (job == 0) { PCD_UNIT_A(0, 3, 1); return; }
     if (job == 1) { PCD_UNIT_A(2, 5, 1); return; }
     if (job == 2) { PCD_UNIT_A(4, 3, 2); return; }
@@ -330,55 +255,6 @@ PCD_HD void fwdA_body(const PassArgs& a, int bx, int n, int z, float* smem) {
 #undef PCD_UNIT_A
 
     // ---- job 4: 3x3 max / avg pool (operations.py:6-7), stride S, pad 1, count_include_pad=False ---------
-    if (FAST) {
-        // full-width tile: the only out-of-image taps are whole rows, the left-most tap of the first pixel of a row
-        // and (stride 1) the right-most tap of the last one; the column halo holds zeros (right for the sums)
-        PCD_FOR(task, C * NSTRIP) {
-            const int ch = task / NSTRIP, strip = task - ch * NSTRIP;
-            const int oyl = strip / PW4, oxl = (strip - oyl * PW4) * 4;
-            const float* pl = XIN + ch * IH * IW;
-            const int oy = g.oy0 + oyl;
-            const bool left = oxl == 0, right = (S == 1) && (oxl + 4 == TW);
-            float mx[4], sm[4];
-            int nrow = 0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { mx[j] = -INFINITY; sm[j] = 0.f; }
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy) {
-                const int gy = S * oy + dy - 1;
-                if (gy < 0 || gy >= a.Hs) continue;
-                ++nrow;
-                const F4* rp = reinterpret_cast<const F4*>(pl + (S * oyl + dy + 3) * IW + S * oxl);
-                float v[12];
-#pragma unroll
-                for (int q = 0; q < 3; ++q) { const F4 t = rp[q]; v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w; }
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-#pragma unroll
-                    for (int dx = 0; dx < 3; ++dx) {
-                        const int idx = S * j + dx + 3;
-                        const float val = v[idx];
-                        sm[j] += val;
-                        float vm = val;
-                        if (idx == 3) vm = left ? -INFINITY : val;
-                        if (S == 1 && idx == 8 && j == 3) vm = right ? -INFINITY : val;
-                        mx[j] = vm > mx[j] ? vm : mx[j];
-                    }
-            }
-            float av[4], s1 = 0.f, q1 = 0.f, s2 = 0.f, q2 = 0.f;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int ncol = 3 - ((j == 0 && left) ? 1 : 0) - ((j == 3 && right) ? 1 : 0);
-                av[j] = sm[j] / (float)(nrow * ncol);
-                s1 += mx[j]; q1 = fmaf(mx[j], mx[j], q1);
-                s2 += av[j]; q2 = fmaf(av[j], av[j], q2);
-            }
-            store4<true>(e.saved + slot_p1() * nslot, g, C, ch, oy, oxl, mx);
-            store4<true>(e.saved + slot_p2() * nslot, g, C, ch, oy, oxl, av);
-            const int NT = C * NSTRIP;
-            P[0 * NT + task] = s1; P[1 * NT + task] = q1; P[2 * NT + task] = s2; P[3 * NT + task] = q2;
-        }
-    } else
     PCD_FOR(task, C * NSTRIP) {
         const int ch = task / NSTRIP, strip = task - ch * NSTRIP;
         const int oyl = strip / PW4, oxl = (strip - oyl * PW4) * 4;
@@ -422,13 +298,13 @@ PCD_HD void fwdA_body(const PassArgs& a, int bx, int n, int z, float* smem) {
             const int cnt = nrow * ncol;
             mx[j] = cnt ? mx[j] : 0.f;
             av[j] = cnt ? sm[j] / (float)cnt : 0.f;
-            if (FAST || (oy < a.Ho && ox < a.Wo)) {
+            if (oy < a.Ho && ox < a.Wo) {
                 s1 += mx[j]; q1 = fmaf(mx[j], mx[j], q1);
                 s2 += av[j]; q2 = fmaf(av[j], av[j], q2);
             }
         }
-        store4<FAST>(e.saved + slot_p1() * nslot, g, C, ch, oy, g.ox0 + oxl, mx);
-        store4<FAST>(e.saved + slot_p2() * nslot, g, C, ch, oy, g.ox0 + oxl, av);
+        store4(e.saved + slot_p1() * nslot, g, C, ch, oy, g.ox0 + oxl, mx);
+        store4(e.saved + slot_p2() * nslot, g, C, ch, oy, g.ox0 + oxl, av);
         const int NT = C * NSTRIP;
         P[0 * NT + task] = s1; P[1 * NT + task] = q1; P[2 * NT + task] = s2; P[3 * NT + task] = q2;
     }
@@ -453,11 +329,11 @@ PCD_HD void fwdA_body(const PassArgs& a, int bx, int n, int z, float* smem) {
                 for (int j = 0; j < 4; ++j) f[j] = fmaf(wv, relu(pl[2 * j]), f[j]);
             }
             const int oy = g.oy0 + oyl, ox = g.ox0 + oxl;
-            store4<FAST>(e.saved + slot_f() * nslot, g, C, co, oy, ox, f);
+            store4(e.saved + slot_f() * nslot, g, C, co, oy, ox, f);
             float s = 0.f, q = 0.f;
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                if (FAST || (oy < a.Ho && ox + j < a.Wo)) { s += f[j]; q = fmaf(f[j], f[j], q); }
+                if (oy < a.Ho && ox + j < a.Wo) { s += f[j]; q = fmaf(f[j], f[j], q); }
             const int NT = C * NSTRIP;
             P[task] = s; P[NT + task] = q;
         }
@@ -472,10 +348,9 @@ PCD_HOSTDEV size_t fwdB_smem_floats(int C, int TH, int TW) {
 }
 
 // second half of SepConv: BN -> ReLU -> dw (stride 1) -> pw   (operations.py:58-62); job = half (k=3 | k=5)
-template <int C, int FTH, int FTW>
+template <int C>
 PCD_HD void fwdB_body(const PassArgs& a, int bx, int n, int z, float* smem) {
-    constexpr bool FAST = FTH != 0;
-    const int TH = FTH ? FTH : a.TH, TW = FTW ? FTW : a.TW;
+    const int TH = a.TH, TW = a.TW;
     const int ez = z >> 1, half = z & 1;
     const EdgeF& e = a.e[ez];
     Geo g;
@@ -494,36 +369,23 @@ PCD_HD void fwdB_body(const PassArgs& a, int bx, int n, int z, float* smem) {
     const double cnt = (double)a.B * a.Ho * a.Wo;
     const int S = a.S, uA = half ? 2 : 0, uB = uA + 1;
     const float* src = e.saved + slot_z(uA) * nslot + (long long)n * C * a.Ho * a.Wo;
-    constexpr int FTH_ = FTH ? FTH : 4, FW = FTW ? FTW : 4;
-    if (FAST) {      // the raw zA rows start their way into shared memory before the BN constants are derived
-        if (half == 0) stage_rows_full<C, FTH_ + 2, FW>(Q, src, (long long)a.Ho * a.Wo, g.oy0 - 1, a.Ho);
-        else stage_rows_full<C, FTH_ + 4, FW>(Q, src, (long long)a.Ho * a.Wo, g.oy0 - 2, a.Ho);
-    }
     PCD_FOR(j, C) {
         BnC b = bn_consts(e.stats, C, bn_unit(S, uA), j, cnt, a.eps);
         BNC[2 * j] = b.mean;
         BNC[2 * j + 1] = b.rstd;
     }
-    if (FAST) cp16_wait();
     PCD_SYNC();
-    {
-        auto bnrelu = [&](int ch, float v) { return relu((v - BNC[2 * ch]) * BNC[2 * ch + 1]); };
-        if (FAST) {
-            if (half == 0) apply_rows_full<C, FTH_ + 2, FW>(Q, g.oy0 - 1, a.Ho, bnrelu);
-            else apply_rows_full<C, FTH_ + 4, FW>(Q, g.oy0 - 2, a.Ho, bnrelu);
-        } else {
-            load_tile<FAST>(Q, src, (long long)a.Ho * a.Wo, C, IH, IW, g.oy0 - HY, g.ox0 - 4, a.Ho, a.Wo, bnrelu);
-        }
-    }
+    load_tile(Q, src, (long long)a.Ho * a.Wo, C, IH, IW, g.oy0 - HY, g.ox0 - 4, a.Ho, a.Wo,
+              [&](int ch, float v) { return relu((v - BNC[2 * ch]) * BNC[2 * ch + 1]); });
     PCD_SYNC();
     if (half == 0)
-        unit_forward<C, 3, 1, 1, false, FAST>(Q, IH, IW, 1, e.par + edge_dw_off(C, S, uB), e.par + edge_pw_off(C, S, uB), T,
-                                              P, P2, WS, e.saved + slot_t(uB) * nslot, e.saved + slot_z(uB) * nslot,
-                                              e.stats + bn_unit(S, uB) * 2 * C, g);
+        unit_forward<C, 3, 1, 1, false>(Q, IH, IW, 1, e.par + edge_dw_off(C, S, uB), e.par + edge_pw_off(C, S, uB), T,
+                                        P, P2, WS, e.saved + slot_t(uB) * nslot, e.saved + slot_z(uB) * nslot,
+                                        e.stats + bn_unit(S, uB) * 2 * C, g);
     else
-        unit_forward<C, 5, 1, 1, false, FAST>(Q, IH, IW, 2, e.par + edge_dw_off(C, S, uB), e.par + edge_pw_off(C, S, uB), T,
-                                              P, P2, WS, e.saved + slot_t(uB) * nslot, e.saved + slot_z(uB) * nslot,
-                                              e.stats + bn_unit(S, uB) * 2 * C, g);
+        unit_forward<C, 5, 1, 1, false>(Q, IH, IW, 2, e.par + edge_dw_off(C, S, uB), e.par + edge_pw_off(C, S, uB), T,
+                                        P, P2, WS, e.saved + slot_t(uB) * nslot, e.saved + slot_z(uB) * nslot,
+                                        e.stats + bn_unit(S, uB) * 2 * C, g);
 }
 
 // ======================================================================================================
@@ -571,7 +433,7 @@ struct EdgeBwdArgs {
 
 // dz on the haloed output tile -> dt = Wpw^T dz into DT[C][RH][IW] (row halo halo_y, col halo 4);
 // centre dz into DZ[C][NPIX] when DZ != null.  WT holds Wpw transposed: WT[ci][co].
-template <int C, bool FAST>
+template <int C>
 PCD_HD void dz_dt_tile(float* DT, float* DZ, int RH, int IW, int halo_y, const float* dy_img, long long dy_cs, int dy_chm,
                        const float* z_img, const float* WT, const float* COEF, const Geo& g) {
     const int NPIX = g.TH * g.TW, p4 = IW >> 2;
@@ -586,12 +448,12 @@ PCD_HD void dz_dt_tile(float* DT, float* DZ, int RH, int IW, int halo_y, const f
         for (int j = 0; j < C; ++j) {
             float dy[4] = {0.f, 0.f, 0.f, 0.f}, zz[4] = {0.f, 0.f, 0.f, 0.f};
             if (in) {
-                load4<FAST>(dy_img + (long long)(j * dy_chm) * dy_cs + (long long)oy * g.Wo, ox, g.Wo, dy);
-                load4<FAST>(z_img + (long long)j * HW + (long long)oy * g.Wo, ox, g.Wo, zz);
+                load4(dy_img + (long long)(j * dy_chm) * dy_cs + (long long)oy * g.Wo, ox, g.Wo, dy);
+                load4(z_img + (long long)j * HW + (long long)oy * g.Wo, ox, g.Wo, zz);
             }
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                const bool ok = in && (FAST || (ox + t >= 0 && ox + t < g.Wo));
+                const bool ok = in && ox + t >= 0 && ox + t < g.Wo;
                 dz[j][t] = ok ? COEF[4 * j] * (dy[t] - COEF[4 * j + 1] - (zz[t] - COEF[4 * j + 2]) * COEF[4 * j + 3]) : 0.f;
             }
         }
@@ -629,7 +491,7 @@ struct WgradPw {
     static constexpr int PFLOATS = 16 * NT;
 };
 
-template <int C, bool FAST>
+template <int C>
 PCD_HD void wgrad_pw(const float* DZ, const float* t_slot, float* gw, float* P, float* P2, const Geo& g) {
     constexpr int NOG = WgradPw<C>::NOG, NSL = WgradPw<C>::NSL, NT = WgradPw<C>::NT;
     const int NPIX = g.TH * g.TW, SPS = (NPIX / 4 + NSL - 1) / NSL, PW4 = g.TW / 4;   // strips per slice
@@ -644,11 +506,11 @@ PCD_HD void wgrad_pw(const float* DZ, const float* t_slot, float* gw, float* P, 
         for (int st = sl * SPS; st < (sl + 1) * SPS && st < NPIX / 4; ++st) {
             const int oyl = st / PW4, oxl = (st - oyl * PW4) * 4;
             const int oy = g.oy0 + oyl, ox = g.ox0 + oxl;
-            if (!FAST && oy >= g.Ho) continue;
+            if (oy >= g.Ho) continue;
             float tv[4][4], dz[4][4];
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                load4<FAST>(t_slot + out_index(g, C, ci0 + k, oy, 0), ox, g.Wo, tv[k]);
+                load4(t_slot + out_index(g, C, ci0 + k, oy, 0), ox, g.Wo, tv[k]);
                 const F4 d = *reinterpret_cast<const F4*>(DZ + (co0 + k) * NPIX + st * 4);
                 dz[k][0] = d.x; dz[k][1] = d.y; dz[k][2] = d.z; dz[k][3] = d.w;
             }
@@ -714,7 +576,7 @@ PCD_HOSTDEV size_t bwdB_smem_floats(int C, int TH, int TW, int need_wgrad) {
     return 2 * tile + scratch + 6 * C + C * C + 64;
 }
 
-template <int C, int KS, bool FAST>
+template <int C, int KS>
 PCD_HD void bwdB_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int half, float* smem) {
     constexpr int PAD = (KS - 1) / 2;
     const int S = a.S, TH = g.TH, TW = g.TW, NPIX = TH * TW, RH = TH + 2 * PAD, IW = TW + 8;
@@ -749,9 +611,9 @@ PCD_HD void bwdB_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int hal
     PCD_SYNC();
     const float* zA = e.saved + slot_z(uA) * nslot + (long long)g.n * C * HW;
     const float* zB = e.saved + slot_z(uB) * nslot + (long long)g.n * C * HW;
-    dz_dt_tile<C, FAST>(DT, DZ, RH, IW, PAD, e.dn + (long long)g.n * e.dn_ns, HW, 4, zB, WT, COEF, g);
-    load_tile<FAST>(Q, zA, HW, C, RH, IW, g.oy0 - PAD, g.ox0 - 4, a.Ho, a.Wo,
-                    [&](int ch, float v) { return relu((v - BNA[2 * ch]) * BNA[2 * ch + 1]); });
+    dz_dt_tile<C>(DT, DZ, RH, IW, PAD, e.dn + (long long)g.n * e.dn_ns, HW, 4, zB, WT, COEF, g);
+    load_tile(Q, zA, HW, C, RH, IW, g.oy0 - PAD, g.ox0 - 4, a.Ho, a.Wo,
+              [&](int ch, float v) { return relu((v - BNA[2 * ch]) * BNA[2 * ch + 1]); });
     PCD_SYNC();
     // grad wrt relu(bn(zA)) = flipped depthwise correlation of dt; mask by the ReLU; sums for BN-A backward
     float* ga = e.ga + half * nslot;
@@ -772,16 +634,16 @@ PCD_HD void bwdB_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int hal
             const F4 q4 = *reinterpret_cast<const F4*>(Q + (ch * RH + py + i + PAD) * IW + px + 4);
             const float q[4] = {q4.x, q4.y, q4.z, q4.w};
             float o[4], za[4] = {0.f, 0.f, 0.f, 0.f};
-            if (FAST || oy < a.Ho) load4<FAST>(zA + (long long)ch * HW + (long long)oy * a.Wo, g.ox0 + px, a.Wo, za);
+            if (oy < a.Ho) load4(zA + (long long)ch * HW + (long long)oy * a.Wo, g.ox0 + px, a.Wo, za);
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 o[j] = q[j] > 0.f ? acc[i][j] : 0.f;
-                if (FAST || (oy < a.Ho && g.ox0 + px + j < a.Wo)) {
+                if (oy < a.Ho && g.ox0 + px + j < a.Wo) {
                     s += o[j];
                     sz = fmaf(o[j], za[j], sz);
                 }
             }
-            store4<FAST>(ga, g, C, ch, oy, g.ox0 + px, o);
+            store4(ga, g, C, ch, oy, g.ox0 + px, o);
         }
         Pga[task] = s;
         Pga[C * NPATCH + task] = sz;
@@ -790,21 +652,19 @@ PCD_HD void bwdB_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int hal
         pcd_atomic_add(e.bstats + (bs_ga(half) + k) * C + ch, (double)v);
     });
     if (a.need_wgrad) {
-        wgrad_pw<C, FAST>(DZ, e.saved + slot_t(uB) * nslot, e.gpar + edge_pw_off(C, S, uB), Ppw, P2, g);
+        wgrad_pw<C>(DZ, e.saved + slot_t(uB) * nslot, e.gpar + edge_pw_off(C, S, uB), Ppw, P2, g);
         wgrad_dw<C, KS, 1, 1, false>(DT, RH, IW, PAD, Q, RH, IW, PAD, e.gpar + edge_dw_off(C, S, uB), Pdw, P2, g);
     }
 }
 
-template <int C, int FTH, int FTW>
+template <int C>
 PCD_HD void bwdB_body(const EdgeBwdArgs& a, int bx, int n, int z, float* smem) {
-    constexpr bool FAST = FTH != 0;
-    const int TH = FTH ? FTH : a.TH, TW = FTW ? FTW : a.TW;
     Geo g;
-    g.n = n; g.TH = TH; g.TW = TW; g.Ho = a.Ho; g.Wo = a.Wo;
-    g.oy0 = (bx / a.tiles_x) * TH;
-    g.ox0 = (bx % a.tiles_x) * TW;
-    if ((z & 1) == 0) bwdB_job<C, 3, FAST>(a, a.e[z >> 1], g, 0, smem);
-    else bwdB_job<C, 5, FAST>(a, a.e[z >> 1], g, 1, smem);
+    g.n = n; g.TH = a.TH; g.TW = a.TW; g.Ho = a.Ho; g.Wo = a.Wo;
+    g.oy0 = (bx / a.tiles_x) * a.TH;
+    g.ox0 = (bx % a.tiles_x) * a.TW;
+    if ((z & 1) == 0) bwdB_job<C, 3>(a, a.e[z >> 1], g, 0, smem);
+    else bwdB_job<C, 5>(a, a.e[z >> 1], g, 1, smem);
 }
 
 // ---- stage A ------------------------------------------------------------------------------------------------
@@ -846,14 +706,8 @@ PCD_HD void dw_bwd_data_s2(const float* dtp /* plane [RH][IW], row halo HY, col 
         }
 }
 
-template <bool FAST>
 PCD_HD void store_in4(float* pd_img, int ch, int gy, int gx, int Hs, int Ws, const float (&v)[4]) {
     float* p = pd_img + ((long long)ch * Hs + gy) * Ws + gx;
-    if (FAST) {
-        F4 t = {v[0], v[1], v[2], v[3]};
-        *reinterpret_cast<F4*>(p) = t;
-        return;
-    }
     if (gy >= Hs) return;
 #pragma unroll
     for (int j = 0; j < 4; ++j)
@@ -861,7 +715,7 @@ PCD_HD void store_in4(float* pd_img, int ch, int gy, int gx, int Hs, int Ws, con
 }
 
 // conv job: unit u (A3/A5: dy = GA, D3/D5: dy = dN[:, 0::4]) -> partial d relu(xs) (pre mask), weight grads
-template <int C, int S, int KS, int DIL, bool FAST>
+template <int C, int S, int KS, int DIL>
 PCD_HD void bwdA_conv_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int u, int slot, float* smem) {
     constexpr int PAD = DIL * (KS - 1) / 2;
     constexpr int HY = (S == 1) ? PAD : (PAD + 1) / 2;
@@ -894,12 +748,12 @@ PCD_HD void bwdA_conv_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
     }
     PCD_FOR(i, C * C) WT[(i % C) * C + i / C] = w_pw[i];
     if (a.need_wgrad)
-        load_tile<FAST>(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, S * g.oy0 - 4, S * g.ox0 - 4,
-                        a.Hs, a.Ws, [](int, float v) { return v; });
+        load_tile(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, S * g.oy0 - 4, S * g.ox0 - 4,
+                  a.Hs, a.Ws, [](int, float v) { return v; });
     PCD_SYNC();
     const float* dy_img = isA ? e.ga + which * nslot + (long long)g.n * C * HW : e.dn + (long long)g.n * e.dn_ns;
-    dz_dt_tile<C, FAST>(DT, DZ, RH, IW, HY, dy_img, HW, isA ? 1 : 4, e.saved + slot_z(u) * nslot + (long long)g.n * C * HW,
-                        WT, COEF, g);
+    dz_dt_tile<C>(DT, DZ, RH, IW, HY, dy_img, HW, isA ? 1 : 4, e.saved + slot_z(u) * nslot + (long long)g.n * C * HW,
+                  WT, COEF, g);
     PCD_SYNC();
     float* pd_img = e.pd + (long long)slot * a.B * C * a.Hs * a.Ws + (long long)g.n * C * a.Hs * a.Ws;
     const int AH = S * TH, AW = S * TW, APW4 = AW / 4, ANP = (AH / 4) * APW4;
@@ -916,16 +770,16 @@ PCD_HD void bwdA_conv_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
         else
             dw_bwd_data_s2<KS, DIL>(DT + ch * RH * IW, IW, HY, qy, qx, w_dw + ch * KS * KS, acc);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) store_in4<FAST>(pd_img, ch, S * g.oy0 + qy + i, S * g.ox0 + qx, a.Hs, a.Ws, acc[i]);
+        for (int i = 0; i < 4; ++i) store_in4(pd_img, ch, S * g.oy0 + qy + i, S * g.ox0 + qx, a.Hs, a.Ws, acc[i]);
     }
     if (a.need_wgrad) {
-        wgrad_pw<C, FAST>(DZ, e.saved + slot_t(u) * nslot, e.gpar + edge_pw_off(C, S, u), Ppw, P2, g);
+        wgrad_pw<C>(DZ, e.saved + slot_t(u) * nslot, e.gpar + edge_pw_off(C, S, u), Ppw, P2, g);
         wgrad_dw<C, KS, DIL, S, true>(DT, RH, IW, HY, XIN, IH, XW, 4, e.gpar + edge_dw_off(C, S, u), Pdw, P2, g);
     }
 }
 
 // pool jobs: which = 0 max-pool (argmax recomputed from the raw tile), 1 avg-pool (+ identity skip at stride 1)
-template <int C, int S, bool FAST>
+template <int C, int S>
 PCD_HD void bwdA_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int which, float* smem) {
     const int TH = g.TH, TW = g.TW, RH = TH + 2, IW = TW + 8, IH = S * TH + 8, XW = S * TW + 8, p4 = IW >> 2;
     float* COEF = smem;
@@ -942,8 +796,8 @@ PCD_HD void bwdA_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
         COEF[4 * j] = d.c0; COEF[4 * j + 1] = d.a; COEF[4 * j + 2] = d.m; COEF[4 * j + 3] = d.c1;
     }
     if (!which)
-        load_tile<FAST>(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, S * g.oy0 - 4, S * g.ox0 - 4,
-                        a.Hs, a.Ws, [](int, float v) { return v; });
+        load_tile(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, S * g.oy0 - 4, S * g.ox0 - 4,
+                  a.Hs, a.Ws, [](int, float v) { return v; });
     PCD_SYNC();
     const float* dn_img = e.dn + (long long)g.n * e.dn_ns;
     const float* Z = e.saved + (which ? slot_p2() : slot_p1()) * nslot + (long long)g.n * C * HW;
@@ -955,8 +809,8 @@ PCD_HD void bwdA_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
         float dz[4] = {0.f, 0.f, 0.f, 0.f}, code[4] = {-1.f, -1.f, -1.f, -1.f};
         if (oy >= 0 && oy < a.Ho && ox + 3 >= 0 && ox < a.Wo) {
             float h[4], zz[4];
-            load4<FAST>(dn_img + (long long)(4 * ch) * HW + (long long)oy * a.Wo, ox, a.Wo, h);
-            load4<FAST>(Z + (long long)ch * HW + (long long)oy * a.Wo, ox, a.Wo, zz);
+            load4(dn_img + (long long)(4 * ch) * HW + (long long)oy * a.Wo, ox, a.Wo, h);
+            load4(Z + (long long)ch * HW + (long long)oy * a.Wo, ox, a.Wo, zz);
             int nrow = 0;
 #pragma unroll
             for (int dy = 0; dy < 3; ++dy) {
@@ -965,7 +819,7 @@ PCD_HD void bwdA_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
             }
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                if (!FAST && (ox + t < 0 || ox + t >= a.Wo)) continue;
+                if (ox + t < 0 || ox + t >= a.Wo) continue;
                 float v = COEF[4 * ch] * (h[t] - COEF[4 * ch + 1] - (zz[t] - COEF[4 * ch + 2]) * COEF[4 * ch + 3]);
                 if (which) {
                     int ncol = 0;
@@ -1026,18 +880,18 @@ PCD_HD void bwdA_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, in
                 }
         }
         const int gy = S * g.oy0 + qy, gx = S * g.ox0 + qx0;
-        if (which && S == 1 && (FAST || gy < a.Ho)) {       // identity skip: d xs += beta * w3 * dN[:, 0::4]
+        if (which && S == 1 && gy < a.Ho) {       // identity skip: d xs += beta * w3 * dN[:, 0::4]
             float h[4];
-            load4<FAST>(dn_img + (long long)(4 * ch) * HW + (long long)gy * a.Wo, gx, a.Wo, h);
+            load4(dn_img + (long long)(4 * ch) * HW + (long long)gy * a.Wo, gx, a.Wo, h);
 #pragma unroll
             for (int t = 0; t < 4; ++t) s[t] = fmaf(idc, h[t], s[t]);
         }
-        store_in4<FAST>(pd_img, ch, gy, gx, a.Hs, a.Ws, s);
+        store_in4(pd_img, ch, gy, gx, a.Hs, a.Ws, s);
     }
 }
 
 // FactorizedReduce backward (stride-2 skip): partial d relu(xs) (pre mask) + the two 1x1 weight grads
-template <int C, bool FAST>
+template <int C>
 PCD_HD void bwdA_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, float* smem) {
     const int TH = g.TH, TW = g.TW, NPIX = TH * TW, IH = 2 * TH + 8, XW = 2 * TW + 8, PW4 = TW / 4;
     float* COEF = smem;
@@ -1054,8 +908,8 @@ PCD_HD void bwdA_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, floa
         COEF[4 * j] = d.c0; COEF[4 * j + 1] = d.a; COEF[4 * j + 2] = d.m; COEF[4 * j + 3] = d.c1;
     }
     if (a.need_wgrad)
-        load_tile<FAST>(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, 2 * g.oy0 - 4, 2 * g.ox0 - 4,
-                        a.Hs, a.Ws, [](int, float v) { return v; });
+        load_tile(XIN, e.x + (long long)g.n * e.x_ns, (long long)a.Hs * a.Ws, C, IH, XW, 2 * g.oy0 - 4, 2 * g.ox0 - 4,
+                  a.Hs, a.Ws, [](int, float v) { return v; });
     PCD_SYNC();
     const float* dn_img = e.dn + (long long)g.n * e.dn_ns;
     const float* F = e.saved + slot_f() * nslot + (long long)g.n * C * HW;
@@ -1067,14 +921,14 @@ PCD_HD void bwdA_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, floa
 #pragma unroll
         for (int j = 0; j < C; ++j) {
             float h[4] = {0.f, 0.f, 0.f, 0.f}, f[4] = {0.f, 0.f, 0.f, 0.f};
-            const bool in = FAST || oy < a.Ho;
+            const bool in = oy < a.Ho;
             if (in) {
-                load4<FAST>(dn_img + (long long)(4 * j) * HW + (long long)oy * a.Wo, ox, a.Wo, h);
-                load4<FAST>(F + (long long)j * HW + (long long)oy * a.Wo, ox, a.Wo, f);
+                load4(dn_img + (long long)(4 * j) * HW + (long long)oy * a.Wo, ox, a.Wo, h);
+                load4(F + (long long)j * HW + (long long)oy * a.Wo, ox, a.Wo, f);
             }
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                const bool ok = in && (FAST || ox + t < a.Wo);
+                const bool ok = in && ox + t < a.Wo;
                 dz[j][t] = ok ? COEF[4 * j] * (h[t] - COEF[4 * j + 1] - (f[t] - COEF[4 * j + 2]) * COEF[4 * j + 3]) : 0.f;
             }
             if (a.need_wgrad) {
@@ -1098,10 +952,10 @@ PCD_HD void bwdA_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, floa
             }
             const float a0[4] = {r0[0], r0[1], r0[2], r0[3]}, a1[4] = {r0[4], r0[5], r0[6], r0[7]};
             const float b0[4] = {r1[0], r1[1], r1[2], r1[3]}, b1[4] = {r1[4], r1[5], r1[6], r1[7]};
-            store_in4<FAST>(pd_img, ci, 2 * oy, 2 * ox, a.Hs, a.Ws, a0);
-            store_in4<FAST>(pd_img, ci, 2 * oy, 2 * ox + 4, a.Hs, a.Ws, a1);
-            store_in4<FAST>(pd_img, ci, 2 * oy + 1, 2 * ox, a.Hs, a.Ws, b0);
-            store_in4<FAST>(pd_img, ci, 2 * oy + 1, 2 * ox + 4, a.Hs, a.Ws, b1);
+            store_in4(pd_img, ci, 2 * oy, 2 * ox, a.Hs, a.Ws, a0);
+            store_in4(pd_img, ci, 2 * oy, 2 * ox + 4, a.Hs, a.Ws, a1);
+            store_in4(pd_img, ci, 2 * oy + 1, 2 * ox, a.Hs, a.Ws, b0);
+            store_in4(pd_img, ci, 2 * oy + 1, 2 * ox + 4, a.Hs, a.Ws, b1);
         }
     }
     if (a.need_wgrad) {
@@ -1145,24 +999,22 @@ PCD_HD void bwdA_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, floa
     }
 }
 
-template <int C, int S, int FTH, int FTW>
+template <int C, int S>
 PCD_HD void bwdA_body(const EdgeBwdArgs& a, int bx, int n, int z, float* smem) {
-    constexpr bool FAST = FTH != 0;
-    const int TH = FTH ? FTH : a.TH, TW = FTW ? FTW : a.TW;
     const int NJ = 6 + (S == 2);
     const int ez = z / NJ, job = z - ez * NJ;
     const EdgeG& e = a.e[ez];
     Geo g;
-    g.n = n; g.TH = TH; g.TW = TW; g.Ho = a.Ho; g.Wo = a.Wo;
-    g.oy0 = (bx / a.tiles_x) * TH;
-    g.ox0 = (bx % a.tiles_x) * TW;
-    if (job == 0) bwdA_conv_job<C, S, 3, 1, FAST>(a, e, g, 0, 0, smem);
-    else if (job == 1) bwdA_conv_job<C, S, 5, 1, FAST>(a, e, g, 2, 1, smem);
-    else if (job == 2) bwdA_conv_job<C, S, 3, 2, FAST>(a, e, g, 4, 2, smem);
-    else if (job == 3) bwdA_conv_job<C, S, 5, 2, FAST>(a, e, g, 5, 3, smem);
-    else if (job == 4) bwdA_pool_job<C, S, FAST>(a, e, g, 0, smem);
-    else if (job == 5) bwdA_pool_job<C, S, FAST>(a, e, g, 1, smem);
-    else if (S == 2) bwdA_fr_job<C, FAST>(a, e, g, smem);
+    g.n = n; g.TH = a.TH; g.TW = a.TW; g.Ho = a.Ho; g.Wo = a.Wo;
+    g.oy0 = (bx / a.tiles_x) * a.TH;
+    g.ox0 = (bx % a.tiles_x) * a.TW;
+    if (job == 0) bwdA_conv_job<C, S, 3, 1>(a, e, g, 0, 0, smem);
+    else if (job == 1) bwdA_conv_job<C, S, 5, 1>(a, e, g, 2, 1, smem);
+    else if (job == 2) bwdA_conv_job<C, S, 3, 2>(a, e, g, 4, 2, smem);
+    else if (job == 3) bwdA_conv_job<C, S, 5, 2>(a, e, g, 5, 3, smem);
+    else if (job == 4) bwdA_pool_job<C, S>(a, e, g, 0, smem);
+    else if (job == 5) bwdA_pool_job<C, S>(a, e, g, 1, smem);
+    else if (S == 2) bwdA_fr_job<C>(a, e, g, smem);
 }
 
 }  // namespace pcd

@@ -1,14 +1,14 @@
-// pcd_edge_bwd2.cuh — backward kernels of the MixedOp edges (model_search.py:44-58), v3, for the production
-// geometries: compile-time tile <TH, TW> with TW == the full output width (so the column halo of every tile is
-// zero padding) and full tiles.  Other shapes keep the generic v2 kernels of pcd_edge.cuh.
+// pcd_edge_bwd2.cuh — backward kernels of the MixedOp edges (model_search.py:44-58) for the production geometries:
+// the stage-B data kernel and the weight-gradient kernel (the stage-A data kernel is pcd_edge_bwd4.cuh).  Compile-time
+// tile <TH, TW> with TW == the full output width (so the column halo of every tile is zero padding) and full tiles.
+// Other shapes run the generic kernels of pcd_edge.cuh.
 //
-// v3 splits every depthwise->pointwise unit's backward into two independent jobs:
+// Every depthwise->pointwise unit's backward is split into two independent jobs:
 //   data  job : dz on the row-haloed tile -> dt = Wpw^T dz -> flipped depthwise correlation -> grad of the unit input
-//               (small shared-memory footprint: 3 blocks per SM, three barriers)
 //   wgrad job : dz, dt on the tile centre only + the unit's input tile and its saved depthwise output
 //               -> dW(pointwise), dW(depthwise)       (deferred: one launch per cell covers every edge)
-// Jobs per block (blockIdx.z):  stage B data: B3 | B5          stage A data: A3 | A5 | D3 | D5 | max | avg(+id) | [FR]
-//                               wgrad: A3 | B3 | A5 | B5 | D3 | D5 | [FR]
+// Jobs per block (blockIdx.z):  stage B data: B3 | B5          wgrad: A3 | B3 | A5 | B5 | D3 | D5 | [FR]
+// The building blocks below (dz_rows, dz_stage / dz_finish, dt_rows, zero_col_halo, edge_coef) serve pcd_edge_bwd4.cuh too.
 #pragma once
 #include "pcd_edge.cuh"
 
@@ -203,271 +203,6 @@ PCD_HD void bwdB2_body(const EdgeBwdArgs& a, int bx, int n, int z, float* smem) 
     g.oy0 = bx * TH; g.ox0 = 0;
     if ((z & 1) == 0) bwdB2_data_job<C, 3, TH, TW>(a, a.e[z >> 1], g, 0, smem);
     else bwdB2_data_job<C, 5, TH, TW>(a, a.e[z >> 1], g, 1, smem);
-}
-
-// ======================================================================================================
-// stage A, data jobs
-// ======================================================================================================
-template <int C, int S, int TH, int TW>
-PCD_HOSTDEV size_t bwdA2_smem_floats() {
-    constexpr size_t conv = (size_t)C * (TH + 8) * TW + (size_t)C * (TH + 8) * (TW + 8);
-    constexpr size_t pool = (size_t)C * (S * TH + 8) * (S * TW + 8) + (size_t)C * (TH + 2) * (TW + 8) * 5 / 4 + 16;
-    return (conv > pool ? conv : pool) + 4 * C + C * C + 64;
-}
-
-// conv job: unit u (A3/A5: dy = GA, D3/D5: dy = dN[:, 0::4]) -> partial d relu(xs) (pre mask)
-template <int C, int S, int KS, int DIL, int TH, int TW>
-PCD_HD void bwdA2_conv_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int u, int slot, float* smem) {
-    constexpr int PAD = DIL * (KS - 1) / 2;
-    constexpr int HY = (S == 1) ? PAD : (PAD + 1) / 2;
-    constexpr int RH = TH + 2 * HY, IW = TW + 8;
-    static_assert(RH <= TH + 8, "row halo");
-    float* COEF = smem;
-    float* WT = COEF + 4 * C;
-    float* DZ = WT + C * C;                         // [C][RH][TW]
-    float* DT = DZ + C * (TH + 8) * TW;             // [C][RH][IW]
-    const long long nslot = (long long)a.B * C * a.Ho * a.Wo, HW = (long long)a.Ho * a.Wo;
-    const double cnt = (double)a.B * a.Ho * a.Wo;
-    const float beta = e.beta ? e.beta[0] : 1.f;
-    const float* w_dw = e.par + edge_dw_off(C, S, u);
-    const float* w_pw = e.par + edge_pw_off(C, S, u);
-    const bool isA = (u == 0 || u == 2);
-    const int which = (u == 2) ? 1 : 0;
-    // the raw dy / z rows start their way into shared memory (DZ / the DT area) before the BN constants are derived
-    const float* dy_img = isA ? e.ga + which * nslot + (long long)g.n * C * HW : e.dn + (long long)g.n * e.dn_ns;
-    dz_stage<C, RH, TW>(DZ, DT, dy_img, HW, isA ? 1 : 4, e.saved + slot_z(u) * nslot + (long long)g.n * C * HW, HW, g.oy0 - HY, a.Ho);
-    PCD_FOR(j, C) {
-        const int bn = bn_unit(S, u);
-        if (isA)
-            edge_coef(COEF, j, dz_consts(e.stats, C, bn, j, cnt, a.eps, e.bstats[bs_ga(which) * C + j],
-                                         e.bstats[(bs_ga(which) + 1) * C + j], 1.f));
-        else
-            edge_coef(COEF, j, dz_consts(e.stats, C, bn, j, cnt, a.eps, e.bstats[bs_s0() * C + j], e.bstats[bs_sz(bn) * C + j],
-                                         beta * e.alpha[u == 4 ? 6 : 7]));
-    }
-    PCD_FOR(i, C * C) WT[(i % C) * C + i / C] = w_pw[i];
-    cp16_wait();
-    PCD_SYNC();
-    dz_finish<C, RH, TW>(DZ, DT, COEF, g.oy0 - HY, a.Ho);
-    PCD_SYNC();                                     // raw z consumed: DT can be rewritten
-    zero_col_halo<C * RH, TW, IW>(DT);
-    dt_rows<C, RH, TW, IW, 4>(DT, DZ, WT, g.oy0 - HY, a.Ho);
-    PCD_SYNC();
-    // v3 layout of the partial input grads: slot 0 accumulates every pre-mask partial (A3 A5 D3 D5 FR), slot 1 the two
-    // pool partials; both are zeroed by the launcher and summed with 16-byte reductions (SrcEdge::merged)
-    (void)slot;
-    float* pd_img = e.pd + (long long)g.n * C * a.Hs * a.Ws;
-    constexpr int AH = S * TH, AW = S * TW, APW4 = AW / 4, ANP = (AH / 4) * APW4;
-    for_tasks_rolled<C * ANP>([&](int task) {
-        const int ch = task / ANP, patch = task - ch * ANP;
-        const int qy = (patch / APW4) * 4, qx = (patch % APW4) * 4;
-        float acc[4][4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-        if (S == 1)
-            dw_patch<KS, DIL, 1, true, false>(DT + ch * RH * IW, IW, qy, qx, w_dw + ch * KS * KS, acc);
-        else
-            dw_bwd_data_s2<KS, DIL>(DT + ch * RH * IW, IW, HY, qy, qx, w_dw + ch * KS * KS, acc);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-            red4(pd_img + ((long long)ch * a.Hs + S * g.oy0 + qy + i) * a.Ws + qx, acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
-    });
-}
-
-// pool jobs: which = 0 max-pool (argmax recomputed from the raw tile), 1 avg-pool (+ identity skip at stride 1)
-template <int C, int S, int TH, int TW>
-PCD_HD void bwdA2_pool_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, int which, float* smem) {
-    constexpr int RH = TH + 2, IW = TW + 8, IH = S * TH + 8, XW = S * TW + 8, p4 = IW / 4;
-    float* COEF = smem;
-    float* XIN = COEF + 4 * C + C * C;
-    float* DT = XIN + (size_t)C * IH * XW;
-    unsigned char* AM = reinterpret_cast<unsigned char*>(DT + (size_t)C * RH * IW);     // argmax code per (haloed) output
-    const long long nslot = (long long)a.B * C * a.Ho * a.Wo, HW = (long long)a.Ho * a.Wo;
-    const double cnt = (double)a.B * a.Ho * a.Wo;
-    const float beta = e.beta ? e.beta[0] : 1.f;
-    const int bn = which ? bn_p2() : bn_p1();
-    if (!which) {      // raw input tile (argmax recomputation): cp.async, in flight while the BN constants are derived
-        const float* xi = e.x + (long long)g.n * e.x_ns;
-        const long long xcs = (long long)a.Hs * a.Ws;
-        for_tasks<C * IH * (XW / 4)>([&](int i) {
-            const int c4 = i % (XW / 4), r = (i / (XW / 4)) % IH, ch = i / ((XW / 4) * IH);
-            const int gy = S * g.oy0 - 4 + r, gx = 4 * c4 - 4;
-            const bool ok = gy >= 0 && gy < a.Hs && gx >= 0 && gx < a.Ws;
-            cp16(XIN + (size_t)i * 4, ok ? xi + ch * xcs + (long long)gy * a.Ws + gx : xi, ok);
-        });
-    }
-    PCD_FOR(j, C) {
-        edge_coef(COEF, j, dz_consts(e.stats, C, bn, j, cnt, a.eps, e.bstats[bs_s0() * C + j], e.bstats[bs_sz(bn) * C + j],
-                                     beta * e.alpha[which ? 2 : 1]));
-    }
-    if (!which) cp16_wait();
-    PCD_SYNC();
-    const float* dn_img = e.dn + (long long)g.n * e.dn_ns;
-    const float* Z = e.saved + (which ? slot_p2() : slot_p1()) * nslot + (long long)g.n * C * HW;
-    // dz (and, for max-pool, the argmax code) of every output pixel within one pixel of the tile
-    for_tasks_rolled<C * RH * p4>([&](int i) {
-        const int c4 = i % p4, rr = i / p4, r = rr % RH, ch = rr / RH;
-        const int oyl = r - 1, oxl = 4 * c4 - 4;
-        const int oy = g.oy0 + oyl, ox = oxl;
-        float dz[4] = {0.f, 0.f, 0.f, 0.f};
-        int code[4] = {15, 15, 15, 15};
-        if (oy >= 0 && oy < a.Ho && ox >= 0 && ox < TW) {
-            const F4 h4 = ld4(dn_img + (long long)(4 * ch) * HW + (long long)oy * TW + ox);
-            const F4 z4 = ld4(Z + (long long)ch * HW + (long long)oy * TW + ox);
-            const float h[4] = {h4.x, h4.y, h4.z, h4.w}, zz[4] = {z4.x, z4.y, z4.z, z4.w};
-            int nrow = 0;
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy) {
-                const int gy = S * oy + dy - 1;
-                nrow += (gy >= 0 && gy < a.Hs) ? 1 : 0;
-            }
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                float v = COEF[4 * ch] * (h[t] - COEF[4 * ch + 1] - (zz[t] - COEF[4 * ch + 2]) * COEF[4 * ch + 3]);
-                if (which) {
-                    int ncol = 0;
-#pragma unroll
-                    for (int dx = 0; dx < 3; ++dx) {
-                        const int gx = S * (ox + t) + dx - 1;
-                        ncol += (gx >= 0 && gx < a.Ws) ? 1 : 0;
-                    }
-                    v = v / (float)(nrow * ncol);
-                } else {
-                    float m = -INFINITY;
-                    int best = -1;
-#pragma unroll
-                    for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-                        for (int dx = 0; dx < 3; ++dx) {
-                            const int gy = S * oy + dy - 1, gx = S * (ox + t) + dx - 1;
-                            if (gy >= 0 && gy < a.Hs && gx >= 0 && gx < a.Ws) {
-                                const float xv = XIN[(ch * IH + S * oyl + dy + 3) * XW + S * (oxl + t) + dx + 3];
-                                if (xv > m || best < 0) { m = xv; best = dy * 3 + dx; }
-                            }
-                        }
-                    code[t] = best;
-                }
-                dz[t] = v;
-            }
-        }
-        st4(DT + (ch * RH + r) * IW + 4 * c4, dz[0], dz[1], dz[2], dz[3]);
-        if (!which) {
-            unsigned char* q = AM + (ch * RH + r) * IW + 4 * c4;
-            q[0] = (unsigned char)code[0]; q[1] = (unsigned char)code[1]; q[2] = (unsigned char)code[2]; q[3] = (unsigned char)code[3];
-        }
-    });
-    PCD_SYNC();
-    // gather over the windows that contain each input pixel
-    constexpr int AH = S * TH, AW = S * TW, AW4 = AW / 4;
-    float* pd_img = e.pd + (long long)a.B * C * a.Hs * a.Ws + (long long)g.n * C * a.Hs * a.Ws;      // slot 1 (both pools)
-    const float idc = beta * e.alpha[3];
-    for_tasks_rolled<C * AH * AW4>([&](int task) {
-        const int q4 = task % AW4, rr = task / AW4, qy = rr % AH, ch = rr / AH;
-        const int qx0 = q4 * 4;
-        float s[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-        for (int dy = 0; dy < 3; ++dy) {
-            const int ty = qy + 1 - dy;
-            if (ty % S != 0) continue;
-            const int pr = ty / S + 1;             // ty >= -1 (only when S == 1)
-#pragma unroll
-            for (int t = 0; t < 4; ++t)
-#pragma unroll
-                for (int dx = 0; dx < 3; ++dx) {
-                    const int tx = qx0 + t + 1 - dx;
-                    if (tx % S != 0) continue;
-                    const int idx = (ch * RH + pr) * IW + tx / S + 4;
-                    if (which) s[t] += DT[idx];
-                    else if (AM[idx] == (unsigned char)(dy * 3 + dx)) s[t] += DT[idx];
-                }
-        }
-        const int gy = S * g.oy0 + qy, gx = qx0;
-        if (which && S == 1) {       // identity skip: d xs += beta * w3 * dN[:, 0::4]
-            const F4 h = ld4(dn_img + (long long)(4 * ch) * HW + (long long)gy * TW + gx);
-            s[0] = fmaf(idc, h.x, s[0]); s[1] = fmaf(idc, h.y, s[1]); s[2] = fmaf(idc, h.z, s[2]); s[3] = fmaf(idc, h.w, s[3]);
-        }
-        red4(pd_img + ((long long)ch * a.Hs + gy) * a.Ws + gx, s[0], s[1], s[2], s[3]);
-    });
-}
-
-// FactorizedReduce backward, data part (stride-2 skip): partial d relu(xs) (pre mask)
-template <int C, int TH, int TW>
-PCD_HD void bwdA2_fr_job(const EdgeBwdArgs& a, const EdgeG& e, const Geo& g, float* smem) {
-    constexpr int PW4 = TW / 4, NPIX = TH * TW;
-    float* COEF = smem;
-    float* WF = COEF + 4 * C;                      // [C][C] conv_1 rows then conv_2 rows
-    const long long nslot = (long long)a.B * C * a.Ho * a.Wo, HW = (long long)a.Ho * a.Wo;
-    const double cnt = (double)a.B * a.Ho * a.Wo;
-    const float beta = e.beta ? e.beta[0] : 1.f;
-    PCD_FOR(j, C) {
-        edge_coef(COEF, j, dz_consts(e.stats, C, bn_f(), j, cnt, a.eps, e.bstats[bs_s0() * C + j], e.bstats[bs_sz(bn_f()) * C + j],
-                                     beta * e.alpha[3]));
-    }
-    PCD_FOR(i, C * C) WF[i] = e.par[i];
-    PCD_SYNC();
-    const float* dn_img = e.dn + (long long)g.n * e.dn_ns;
-    const float* F = e.saved + slot_f() * nslot + (long long)g.n * C * HW;
-    float* pd_img = e.pd + (long long)g.n * C * a.Hs * a.Ws;      // slot 0 (pre-mask partials)
-    // task = (strip of 4 output pixels, group of 4 input channels)
-    for_tasks_rolled<(NPIX / 4) * (C / 4)>([&](int task) {
-        const int st = task % (NPIX / 4), cig = task / (NPIX / 4);
-        const int oyl = st / PW4, oxl = (st - oyl * PW4) * 4;
-        const int oy = g.oy0 + oyl, ox = oxl;
-        float r0[4][4], r1[4][4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-#pragma unroll
-            for (int t = 0; t < 4; ++t) { r0[q][t] = 0.f; r1[q][t] = 0.f; }
-#pragma unroll 4
-        for (int co = 0; co < C / 2; ++co) {
-            const F4 h0 = ld4(dn_img + (long long)(4 * co) * HW + (long long)oy * TW + ox);
-            const F4 f0 = ld4(F + (long long)co * HW + (long long)oy * TW + ox);
-            const F4 h1 = ld4(dn_img + (long long)(4 * (co + C / 2)) * HW + (long long)oy * TW + ox);
-            const F4 f1 = ld4(F + (long long)(co + C / 2) * HW + (long long)oy * TW + ox);
-            const float* k0 = COEF + 4 * co;
-            const float* k1 = COEF + 4 * (co + C / 2);
-            const float d0[4] = {k0[0] * (h0.x - k0[1] - (f0.x - k0[2]) * k0[3]), k0[0] * (h0.y - k0[1] - (f0.y - k0[2]) * k0[3]),
-                                 k0[0] * (h0.z - k0[1] - (f0.z - k0[2]) * k0[3]), k0[0] * (h0.w - k0[1] - (f0.w - k0[2]) * k0[3])};
-            const float d1[4] = {k1[0] * (h1.x - k1[1] - (f1.x - k1[2]) * k1[3]), k1[0] * (h1.y - k1[1] - (f1.y - k1[2]) * k1[3]),
-                                 k1[0] * (h1.z - k1[1] - (f1.z - k1[2]) * k1[3]), k1[0] * (h1.w - k1[1] - (f1.w - k1[2]) * k1[3])};
-            const F4 w0 = ld4(WF + co * C + cig * 4), w1 = ld4(WF + (co + C / 2) * C + cig * 4);
-            const float wa[4] = {w0.x, w0.y, w0.z, w0.w}, wb[4] = {w1.x, w1.y, w1.z, w1.w};
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-#pragma unroll
-                for (int t = 0; t < 4; ++t) {
-                    r0[q][t] = fmaf(wa[q], d0[t], r0[q][t]);
-                    r1[q][t] = fmaf(wb[q], d1[t], r1[q][t]);
-                }
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            float* p0 = pd_img + ((long long)(cig * 4 + q) * a.Hs + 2 * oy) * a.Ws + 2 * ox;
-            red4(p0, r0[q][0], 0.f, r0[q][1], 0.f);
-            red4(p0 + 4, r0[q][2], 0.f, r0[q][3], 0.f);
-            red4(p0 + a.Ws, 0.f, r1[q][0], 0.f, r1[q][1]);
-            red4(p0 + a.Ws + 4, 0.f, r1[q][2], 0.f, r1[q][3]);
-        }
-    });
-}
-
-template <int C, int S, int TH, int TW>
-PCD_HD void bwdA2_body(const EdgeBwdArgs& a, int bx, int n, int z, float* smem) {
-    constexpr int NJ = 6 + (S == 2);
-    const int ez = z / NJ, job = z - ez * NJ;
-    const EdgeG& e = a.e[ez];
-    Geo g;
-    g.n = n; g.TH = TH; g.TW = TW; g.Ho = a.Ho; g.Wo = a.Wo;
-    g.oy0 = bx * TH; g.ox0 = 0;
-    if (job == 0) bwdA2_conv_job<C, S, 3, 1, TH, TW>(a, e, g, 0, 0, smem);
-    else if (job == 1) bwdA2_conv_job<C, S, 5, 1, TH, TW>(a, e, g, 2, 1, smem);
-    else if (job == 2) bwdA2_conv_job<C, S, 3, 2, TH, TW>(a, e, g, 4, 2, smem);
-    else if (job == 3) bwdA2_conv_job<C, S, 5, 2, TH, TW>(a, e, g, 5, 3, smem);
-    else if (job == 4) bwdA2_pool_job<C, S, TH, TW>(a, e, g, 0, smem);
-    else if (job == 5) bwdA2_pool_job<C, S, TH, TW>(a, e, g, 1, smem);
-    else if (S == 2) bwdA2_fr_job<C, TH, TW>(a, e, g, smem);
 }
 
 // ======================================================================================================

@@ -1,8 +1,7 @@
 // pcd_edge_bwd4.cuh — stage-A backward DATA kernels of the MixedOp edges for the production geometries, v4.
 //
-// v3 (pcd_edge_bwd2.cuh) ran six or seven blocks per (edge, image, tile) — one per candidate op — each adding its partial
-// d xs into two zero-initialised slots with 16-byte reductions; source_grad then applied the ReLU mask and summed the
-// slots.  v4 runs TWO blocks per (edge, image, tile):
+// Where the generic kernel (pcd_edge.cuh) runs six or seven blocks per (edge, image, tile), one per candidate op, each
+// storing its own partial d xs plane that source_grad masks and sums, v4 runs TWO blocks per (edge, image, tile):
 //   conv block : A5, D5, A3, D3 (+ FactorizedReduce at stride 2) one after the other, the partial input gradients summed in
 //                REGISTERS across the units, the ReLU mask applied at the end (x re-read from L2), ONE plain store;
 //   pool block : max-pool (argmax recomputed from the raw tile) + avg-pool (+ identity skip at stride 1), ONE plain store.
@@ -10,7 +9,8 @@
 // narrow segment loads of pcd_edge_v4.cuh.  At stride 2 the transposed depthwise convs are evaluated per input parity
 // plane (input pixel (2i+a, 2j+b) only sees the taps of parity (a, b)): unit-stride everywhere, a thread produces the
 // interleaved even/odd columns of its rows and stores whole float4s.
-// The slots keep their v3 place (two per edge): slot 0 = masked conv/FR partial, slot 1 = pool partial (SrcEdge::merged = 2).
+// The two slots are the first two planes of the edge's partial-gradient region (EdgeG::pd): slot 0 = masked conv/FR
+// partial, slot 1 = pool partial (SrcEdge::merged set).
 #pragma once
 #include "pcd_edge_bwd2.cuh"
 #include "pcd_edge_v4.cuh"

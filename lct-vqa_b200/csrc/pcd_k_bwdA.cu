@@ -4,23 +4,21 @@
 
 namespace pcd {
 
-template <int C, int S, int TH, int TW> struct KBwdA {
+template <int C, int S> struct KBwdA {
     static constexpr int kMinBlocks = 2; static const char* name() {
         return S == 1 ? (C == 4 ? "bwdA_c4_s1" : C == 8 ? "bwdA_c8_s1" : "bwdA_c16_s1")
                       : (C == 4 ? "bwdA_c4_s2" : C == 8 ? "bwdA_c8_s2" : "bwdA_c16_s2");
     }
-    static PCD_D void run(const EdgeBwdArgs& a, int x, int y, int z, float* sm) { bwdA_body<C, S, TH, TW>(a, x, y, z, sm); }
+    static PCD_D void run(const EdgeBwdArgs& a, int x, int y, int z, float* sm) { bwdA_body<C, S>(a, x, y, z, sm); }
 };
 
-#define GO_A(C_, S_, H_, W_) \
-    return launch<KBwdA<C_, S_, H_, W_>, EdgeBwdArgs>(a, gx, gy, gz, bwdA_smem_floats(C_, S_, a.TH, a.TW, a.need_wgrad), stream)
-int launch_bwdA(const EdgeBwdArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream) {
+#define GO_A(C_, S_) \
+    return launch<KBwdA<C_, S_>, EdgeBwdArgs>(a, gx, gy, gz, bwdA_smem_floats(C_, S_, a.TH, a.TW, a.need_wgrad), stream)
+int launch_bwdA(const EdgeBwdArgs& a, int c, int gx, int gy, int gz, void* stream) {
     if (a.S == 1) {
-        if (fast) { if (c == 4) GO_A(4, 1, 16, 64); if (c == 8) GO_A(8, 1, 16, 32); if (c == 16) GO_A(16, 1, 16, 16); }
-        if (c == 4) GO_A(4, 1, 0, 0); if (c == 8) GO_A(8, 1, 0, 0); if (c == 16) GO_A(16, 1, 0, 0);
+        if (c == 4) GO_A(4, 1); if (c == 8) GO_A(8, 1); if (c == 16) GO_A(16, 1);
     } else {
-        if (fast) { if (c == 8) GO_A(8, 2, 8, 32); if (c == 16) GO_A(16, 2, 8, 16); }
-        if (c == 4) GO_A(4, 2, 0, 0); if (c == 8) GO_A(8, 2, 0, 0); if (c == 16) GO_A(16, 2, 0, 0);
+        if (c == 4) GO_A(4, 2); if (c == 8) GO_A(8, 2); if (c == 16) GO_A(16, 2);
     }
     return PCD_ERR_UNSUPPORTED;
 }

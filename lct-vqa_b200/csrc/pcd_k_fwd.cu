@@ -4,39 +4,31 @@
 
 namespace pcd {
 
-template <int C, int S, int TH, int TW> struct KFwdA {
+template <int C, int S> struct KFwdA {
     static constexpr int kMinBlocks = 3; static const char* name() {
         return S == 1 ? (C == 4 ? "fwdA_c4_s1" : C == 8 ? "fwdA_c8_s1" : "fwdA_c16_s1")
                       : (C == 4 ? "fwdA_c4_s2" : C == 8 ? "fwdA_c8_s2" : "fwdA_c16_s2");
     }
-    static PCD_D void run(const PassArgs& a, int x, int y, int z, float* sm) { fwdA_body<C, S, TH, TW>(a, x, y, z, sm); }
+    static PCD_D void run(const PassArgs& a, int x, int y, int z, float* sm) { fwdA_body<C, S>(a, x, y, z, sm); }
 };
-template <int C, int TH, int TW> struct KFwdB {
+template <int C> struct KFwdB {
     static constexpr int kMinBlocks = 3; static const char* name() { return C == 4 ? "fwdB_c4" : C == 8 ? "fwdB_c8" : "fwdB_c16"; }
-    static PCD_D void run(const PassArgs& a, int x, int y, int z, float* sm) { fwdB_body<C, TH, TW>(a, x, y, z, sm); }
+    static PCD_D void run(const PassArgs& a, int x, int y, int z, float* sm) { fwdB_body<C>(a, x, y, z, sm); }
 };
 
-bool edge_tile_is_fixed(int c, int S, int TH, int TW, bool stageB) {
-    if (stageB || S == 1) return (c == 4 && TH == 16 && TW == 64) || (c == 8 && TH == 16 && TW == 32) || (c == 16 && TH == 16 && TW == 16);
-    return (c == 8 && TH == 8 && TW == 32) || (c == 16 && TH == 8 && TW == 16);
-}
-
-#define GO_A(C_, S_, H_, W_) return launch<KFwdA<C_, S_, H_, W_>, PassArgs>(a, gx, gy, gz, fwdA_smem_floats(C_, S_, a.TH, a.TW), stream)
-int launch_fwdA(const PassArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream) {
+#define GO_A(C_, S_) return launch<KFwdA<C_, S_>, PassArgs>(a, gx, gy, gz, fwdA_smem_floats(C_, S_, a.TH, a.TW), stream)
+int launch_fwdA(const PassArgs& a, int c, int gx, int gy, int gz, void* stream) {
     if (a.S == 1) {
-        if (fast) { if (c == 4) GO_A(4, 1, 16, 64); if (c == 8) GO_A(8, 1, 16, 32); if (c == 16) GO_A(16, 1, 16, 16); }
-        if (c == 4) GO_A(4, 1, 0, 0); if (c == 8) GO_A(8, 1, 0, 0); if (c == 16) GO_A(16, 1, 0, 0);
+        if (c == 4) GO_A(4, 1); if (c == 8) GO_A(8, 1); if (c == 16) GO_A(16, 1);
     } else {
-        if (fast) { if (c == 8) GO_A(8, 2, 8, 32); if (c == 16) GO_A(16, 2, 8, 16); }
-        if (c == 4) GO_A(4, 2, 0, 0); if (c == 8) GO_A(8, 2, 0, 0); if (c == 16) GO_A(16, 2, 0, 0);
+        if (c == 4) GO_A(4, 2); if (c == 8) GO_A(8, 2); if (c == 16) GO_A(16, 2);
     }
     return PCD_ERR_UNSUPPORTED;
 }
 
-#define GO_B(C_, H_, W_) return launch<KFwdB<C_, H_, W_>, PassArgs>(a, gx, gy, gz, fwdB_smem_floats(C_, a.TH, a.TW), stream)
-int launch_fwdB(const PassArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream) {
-    if (fast) { if (c == 4) GO_B(4, 16, 64); if (c == 8) GO_B(8, 16, 32); if (c == 16) GO_B(16, 16, 16); }
-    if (c == 4) GO_B(4, 0, 0); if (c == 8) GO_B(8, 0, 0); if (c == 16) GO_B(16, 0, 0);
+#define GO_B(C_) return launch<KFwdB<C_>, PassArgs>(a, gx, gy, gz, fwdB_smem_floats(C_, a.TH, a.TW), stream)
+int launch_fwdB(const PassArgs& a, int c, int gx, int gy, int gz, void* stream) {
+    if (c == 4) GO_B(4); if (c == 8) GO_B(8); if (c == 16) GO_B(16);
     return PCD_ERR_UNSUPPORTED;
 }
 

@@ -4,16 +4,14 @@
 #include "pcd_edge.cuh"
 
 namespace pcd {
-// `fast` selects the compile-time-tile specialisation for (c, S, a.TH, a.TW); caller guarantees its preconditions.
-bool edge_tile_is_fixed(int c, int S, int TH, int TW, bool stageB);
-int launch_fwdA(const PassArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream);
-int launch_fwdB(const PassArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream);
-int launch_bwdA(const EdgeBwdArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream);
-int launch_bwdB(const EdgeBwdArgs& a, int c, bool fast, int gx, int gy, int gz, void* stream);
-// v3 backward (pcd_edge_bwd2.cuh): production geometries only; a.TH / a.TW hold the tile (TW == Wo)
+// generic edge kernels (pcd_edge.cuh): any geometry, run-time tile a.TH x a.TW
+int launch_fwdA(const PassArgs& a, int c, int gx, int gy, int gz, void* stream);
+int launch_fwdB(const PassArgs& a, int c, int gx, int gy, int gz, void* stream);
+int launch_bwdA(const EdgeBwdArgs& a, int c, int gx, int gy, int gz, void* stream);
+int launch_bwdB(const EdgeBwdArgs& a, int c, int gx, int gy, int gz, void* stream);
+// stage-B data and weight-gradient backward (pcd_edge_bwd2.cuh): production geometries only; a.TH / a.TW hold the tile (TW == Wo)
 bool bwd2_tile(int c, int S, int Ho, int Wo, int* TH);
 int launch_bwdB2(const EdgeBwdArgs& a, int c, int gz, void* stream);
-int launch_bwdA2(const EdgeBwdArgs& a, int c, int gz, void* stream);
 int launch_wgrad2(const EdgeBwdArgs& a, int c, int gz, void* stream);
 // v4 forward (pcd_edge_v4.cuh): stage A + stage B of a group of production-geometry edges
 struct FwdV4Args;

@@ -202,8 +202,8 @@ def shuffle_case(device):
     assert torch.equal(x.grad.cpu(), ref.grad)
 
 
-def mixed_vs_oracle(C, stride, B, H, device, seed=7, check_grads=True, quantized=False):
-    """Larger shapes than the goldens: product on `device` vs the oracle on CPU, same seeded inputs.
+def mixed_vs_oracle(C, stride, B, H, device, seed=7, check_grads=True, quantized=False, W=None):
+    """Larger shapes than the goldens: product on `device` vs the oracle on CPU, same seeded inputs (H x W, square by default).
     quantized: the input only takes multiples of 0.5, so 3x3 / 2x2 max-pool windows are full of exact ties (ATen routes the
     gradient to the FIRST maximum in scan order) and many ReLU inputs are exactly 0 (gradient 0)."""
     import config
@@ -216,11 +216,12 @@ def mixed_vs_oracle(C, stride, B, H, device, seed=7, check_grads=True, quantized
     for v in par.values():
         v.requires_grad_(True)
     gen = torch.Generator().manual_seed(seed)
-    x = torch.randn(B, C, H, H, generator=gen)
+    W = H if W is None else W
+    x = torch.randn(B, C, H, W, generator=gen)
     if quantized:
         x = torch.round(2 * x) / 2
     w = torch.softmax(torch.randn(8, generator=gen), 0)
-    G = torch.randn(B, C, H // stride, H // stride, generator=gen)
+    G = torch.randn(B, C, H // stride, W // stride, generator=gen)
     xr, wr = x.clone().requires_grad_(True), w.clone().requires_grad_(True)
     yr = O.mixed_op(par, O.BNState(buf), "_ops.", xr, wr, stride)
     (yr * G).sum().backward()

@@ -27,13 +27,17 @@ def test_cell_emulated(name, cpp, cp, C, red, rp):
     P.cell_case(name, cpp, cp, C, red, rp, "cpu")
 
 
-# production tile geometries (compile-time-tile "FAST" specialisations), one image each
-@pytest.mark.parametrize("C,stride,B,H", [(16, 1, 1, 64), (32, 2, 1, 64), (32, 1, 2, 32), (64, 2, 1, 32), (64, 1, 2, 16)])
+# the five production edge geometries (v4 forward, production backward kernels), one image each; then two non-square
+# inputs at a production width whose output height is not a multiple of 16: they run the generic kernels
+@pytest.mark.parametrize("C,stride,B,H", [(16, 1, 1, 64), (32, 2, 1, 64), (32, 1, 2, 32), (64, 2, 1, 32), (64, 1, 2, 16),
+                                          pytest.param(32, 2, 1, (48, 64), id="32-2-1-48x64"),
+                                          pytest.param(64, 2, 1, (16, 32), id="64-2-1-16x32")])
 @pytest.mark.parametrize("jobs", ["1", "2"])
 def test_mixed_op_fixed_tiles_emulated(C, stride, B, H, jobs, monkeypatch):
     # v4 forward kernels: one block runs every stage-A job (large waves) | jobs split over two blocks (small waves)
     monkeypatch.setenv("PCD_V4_JOBS", jobs)
-    P.mixed_vs_oracle(C, stride, B, H, "cpu")
+    H, W = H if isinstance(H, tuple) else (H, H)
+    P.mixed_vs_oracle(C, stride, B, H, "cpu", W=W)
 
 
 @pytest.mark.parametrize("C,stride,B,H", [(16, 1, 1, 64), (32, 2, 1, 64), (64, 2, 1, 32), (64, 1, 2, 16)])
@@ -50,7 +54,7 @@ def test_preprocess_emulated(c_in, c_out, fr, B, H):
     P.pre_vs_oracle(c_in, c_out, fr, B, H, "cpu")
 
 
-# a production-geometry cell (v3 backward kernels + deferred weight-grad launch), one image
+# a production-geometry cell (production backward kernels + deferred weight-grad launch), one image
 @pytest.mark.parametrize("cpp,cp,C,red,rp,H", [(128, 256, 64, False, True, 16), (64, 128, 64, True, True, 32)])
 def test_cell_production_geometry_emulated(cpp, cp, C, red, rp, H):
     P.cell_vs_oracle(cpp, cp, C, red, rp, 1, H, "cpu")

@@ -35,14 +35,18 @@ def test_shuffle_bit_exact():
     P.shuffle_case(DEV)
 
 
-# the five production edge shapes of SURVEY.md §8(a) at a batch the oracle finishes in seconds
-@pytest.mark.parametrize("C,stride,B,H", [(16, 1, 4, 64), (32, 2, 4, 64), (32, 1, 4, 32), (64, 2, 4, 32), (64, 1, 8, 16)])
+# the five production edge shapes of SURVEY.md §8(a) at a batch the oracle finishes in seconds; then two non-square inputs
+# at a production width whose output height is not a multiple of 16: they run the generic kernels
+@pytest.mark.parametrize("C,stride,B,H", [(16, 1, 4, 64), (32, 2, 4, 64), (32, 1, 4, 32), (64, 2, 4, 32), (64, 1, 8, 16),
+                                          pytest.param(32, 2, 4, (48, 64), id="32-2-4-48x64"),
+                                          pytest.param(64, 2, 4, (16, 32), id="64-2-4-16x32")])
 @pytest.mark.parametrize("jobs", ["auto", "1", "2"])
 def test_mixed_op_production_shapes_vs_oracle(C, stride, B, H, jobs, monkeypatch):
     # jobs: the v4 forward kernels' two block layouts (all stage-A jobs in one block | split over two), forced either way
     if jobs != "auto":
         monkeypatch.setenv("PCD_V4_JOBS", jobs)
-    P.mixed_vs_oracle(C, stride, B, H, DEV)
+    H, W = H if isinstance(H, tuple) else (H, H)
+    P.mixed_vs_oracle(C, stride, B, H, DEV, W=W)
 
 
 @pytest.mark.parametrize("C,stride,B,H", [(16, 1, 4, 64), (32, 2, 4, 64), (32, 1, 4, 32), (64, 2, 4, 32), (64, 1, 8, 16)])
@@ -101,7 +105,7 @@ def test_preprocess_tensor_core_path_full_batch(c_in, c_out, H, monkeypatch):
         assert v["tc_vs_fp64"] <= 2e-5, (name, rep)
 
 
-# the four production cells (C=16@64, reduce C=32 64->32, reduce C=64 32->16, C=64@16) at batch 2: v3 backward kernels
+# the four production cells (C=16@64, reduce C=32 64->32, reduce C=64 32->16, C=64@16) at batch 2: production backward kernels
 # with the cell-wide deferred weight-gradient launch; once more with frozen weights (activation-only backward, HVP passes)
 @pytest.mark.parametrize("cpp,cp,C,red,rp,H", [(48, 48, 16, False, False, 64), (48, 64, 32, True, False, 64),
                                                (64, 128, 64, True, True, 32), (128, 256, 64, False, True, 16)])
