@@ -1,7 +1,7 @@
 // pcd_ce.cu — cross-entropy over the vocabulary logits, fused around the tcgen05 projection (pcd_gemm_sm100.cu):
 //   vqa_model.py:192-194  qst_out = fc1(tanh(lstm_out))            -> pcd_gemm_tn_3xtf32 into a padded-pitch buffer
 //   vqa_model.py:356-358  CE(qst_out[:, :-1], qst[:, 1:])          -> pcd_ce_forward / pcd_ce_backward on that buffer
-// The logits never get sliced / re-laid-out: rows whose target is negative are ignored (the last time step), the
+// The logits never get sliced / re-laid-out: rows whose target is negative (the last time step) or >= V are ignored, the
 // gradient is written straight into the padded-pitch layout the backward GEMMs read through TMA, and
 // pcd_transpose_pad produces the K-major operands (dlogits^T, W^T, h^T) of those GEMMs.
 #include "../../include/pcdarts_sm100.h"
@@ -168,7 +168,7 @@ int pcd_ce_backward(const float* logits, long long ld, int M, int V, const long 
     for (int r = 0; r < M; ++r)
         for (long long c = 0; c < ld; ++c) {
             const long long t = targets[r];
-            dl[r * ld + c] = (t >= 0 && c < V) ? *scale * (expf(logits[r * ld + c] - lse[r]) - (c == t ? 1.f : 0.f)) : 0.f;
+            dl[r * ld + c] = (t >= 0 && t < V && c < V) ?*scale * (expf(logits[r * ld + c] - lse[r]) - (c == t ? 1.f : 0.f)) : 0.f;
         }
     return PCD_OK;
 }

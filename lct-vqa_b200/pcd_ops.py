@@ -809,7 +809,7 @@ def _transpose_pad(lib, src, ld_s, rows, cols, ld_d, ref):
 
 
 class VocabCrossEntropyFunction(torch.autograd.Function):
-    """mean_r CE(x_r @ W^T + b, target_r) over the rows with target >= 0  — the question-decoder loss
+    """mean_r CE(x_r @ W^T + b, target_r) over the rows with 0 <= target < V  — the question-decoder loss
     (vqa_model.py:192-194 + 356-358) without ever slicing or re-laying-out the (B*T, V) logits: projection on the
     tensor cores into a 16-byte-pitch buffer, row statistics and the loss from it, gradient written in the same layout,
     transposed once for the K-major operand of dW."""
@@ -828,7 +828,9 @@ class VocabCrossEntropyFunction(torch.autograd.Function):
         lse = _empty(m, torch.float32, x2.device)
         rows = _empty(m, torch.float32, x2.device)
         N.check(lib, lib.pcd_ce_forward(N.ptr(logits), vp, m, v, N.ptr(tg), N.ptr(lse), N.ptr(rows), N.stream_for(x2)), "pcd_ce_forward")
-        nvalid = (tg >= 0).sum().clamp_min(1).to(torch.float32)
+        # a row is ignored when its target is negative or >= V (the kernels score both 0); checked on the device, so the
+        # step stays capturable: a host-side range check would synchronise
+        nvalid = ((tg >= 0) & (tg < v)).sum().clamp_min(1).to(torch.float32)
         ctx.save_for_backward(x2, w, logits, lse, tg, nvalid)
         ctx.meta = (x.shape, v, vp, bias is not None)
         return rows.sum() / nvalid
@@ -863,7 +865,7 @@ class VocabCrossEntropyFunction(torch.autograd.Function):
 
 
 def vocab_cross_entropy(x, weight, bias, targets):
-    """Fused projection + cross-entropy (ignore target < 0, mean over the rest); a depth that is not a multiple of 4 raises
+    """Fused projection + cross-entropy (ignore a target < 0 or >= V, mean over the rest); a depth that is not a multiple of 4 raises
     unless allow_stock_ops."""
     if not (x.is_cuda or N._emu_lib is not None):
         raise RuntimeError("pcdarts_sm100 kernels need CUDA tensors (no CPU fallback)")

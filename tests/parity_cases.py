@@ -104,7 +104,7 @@ def network_case(device):
     return net
 
 
-def network_vs_oracle(B, H, device, seed=17):
+def network_vs_oracle(B, H, device, seed=17, W=None):
     """The whole search network (stem, 4 cells at the production geometries, global pooling) at full batch.
 
     Forward: output vs the oracle network.  Backward: every cell is replayed through the oracle on the very tensors our
@@ -120,7 +120,7 @@ def network_vs_oracle(B, H, device, seed=17):
     net = Network(16, 10, 4).train()
     _fill(net, seed)
     gen = torch.Generator().manual_seed(seed)
-    x = torch.randn(B, 3, H, H, generator=gen)
+    x = torch.randn(B, 3, H, H if W is None else W, generator=gen)
     arch = [1e-1 * torch.randn(s, generator=gen) for s in ((14, 8), (14, 8), (14,), (14,))]
     G = torch.randn(B, 256 * 49, generator=gen)
     sd0 = {k: v.detach().clone() for k, v in net.state_dict().items()}
@@ -271,8 +271,9 @@ def pre_vs_oracle(c_in, c_out, fr, B, H, device, seed=11):
             assert_close(v, buf[k], 1e-5, k)
 
 
-def cell_vs_oracle(cpp, cp, C, red, rp, B, H, device, seed=13, act_only=False):
-    """A whole Cell at a production spatial size (compile-time-tile kernels, deferred weight-grad launch) vs the oracle."""
+def cell_vs_oracle(cpp, cp, C, red, rp, B, H, device, seed=13, act_only=False, W=None):
+    """A whole Cell at a production spatial size (compile-time-tile kernels, deferred weight-grad launch) vs the oracle;
+    H x W input state (square by default)."""
     import config
     config.DEVICE = device
     from pcdarts.model_search import Cell
@@ -283,13 +284,14 @@ def cell_vs_oracle(cpp, cp, C, red, rp, B, H, device, seed=13, act_only=False):
     for v in par.values():
         v.requires_grad_(not act_only)
     gen = torch.Generator().manual_seed(seed)
-    H0 = 2 * H if rp else H
-    Ho = H // 2 if red else H
-    s0 = torch.randn(B, cpp, H0, H0, generator=gen)
-    s1 = torch.randn(B, cp, H, H, generator=gen)
+    W = H if W is None else W
+    H0, W0 = (2 * H, 2 * W) if rp else (H, W)
+    Ho, Wo = (H // 2, W // 2) if red else (H, W)
+    s0 = torch.randn(B, cpp, H0, W0, generator=gen)
+    s1 = torch.randn(B, cp, H, W, generator=gen)
     w = torch.softmax(torch.randn(14, 8, generator=gen), -1)
     w2 = torch.softmax(torch.randn(14, generator=gen), 0)
-    G = torch.randn(B, 4 * C, Ho, Ho, generator=gen)
+    G = torch.randn(B, 4 * C, Ho, Wo, generator=gen)
     ref_in = [t.clone().requires_grad_(True) for t in (s0, s1, w, w2)]
     yr = O.cell_forward(par, O.BNState(buf), "", *ref_in, red, rp)
     (yr * G).sum().backward()
@@ -302,7 +304,7 @@ def cell_vs_oracle(cpp, cp, C, red, rp, B, H, device, seed=13, act_only=False):
     assert_close(y, yr, REL_TOL, "y")
     (y * G.to(device)).sum().backward()
     for t, r, k in zip(ins, ref_in, ("ds0", "ds1", "dw", "dw2")):
-        if k in ("ds0", "ds1") and B * H * H >= 2048:
+        if k in ("ds0", "ds1") and B * H * W >= 2048:
             # a ReLU input within rounding of 0 (or a max-pool near-tie) flips between two correct fp32 evaluations and moves
             # the input gradient by O(1) on one stencil neighbourhood x all channels: bound the SHARE of such elements
             d = (t.grad.detach().cpu().double() - r.grad.double()).abs()
@@ -311,11 +313,11 @@ def cell_vs_oracle(cpp, cp, C, red, rp, B, H, device, seed=13, act_only=False):
         else:
             assert_close(t.grad, r.grad, REL_TOL, k)
     if not act_only:
-        flip = 5.0 / (B * Ho * Ho) ** 0.5          # one flipped decision moves a sum over B*Ho*Wo pixels by ~1/sqrt of it
+        flip = 5.0 / (B * Ho * Wo) ** 0.5          # one flipped decision moves a sum over B*Ho*Wo pixels by ~1/sqrt of it
         errs = []
         for k, p_ in m.named_parameters():
             e = rel_err(p_.grad, par[k].grad)
-            assert e <= max(REL_TOL, flip if B * H * H >= 2048 else 0.0), f"{k}: rel err {e:.3e}"
+            assert e <= max(REL_TOL, flip if B * H * W >= 2048 else 0.0), f"{k}: rel err {e:.3e}"
             errs.append(e)
         assert sum(e <= REL_TOL for e in errs) >= 0.97 * len(errs), "more than 3% of the weight grads beyond rel 1e-4"
 

@@ -371,3 +371,26 @@ def test_arena_verify_detects_a_rebound_parameter():
     ar.ensure()                              # ends unchanged: not noticed here
     with pytest.raises(RuntimeError, match="left its flat arena"):
         ar.verify()
+
+
+def test_vocab_cross_entropy_out_of_range_targets_emulated():
+    """Targets < 0 or >= V are ignored rows: loss 0, gradient 0, not counted in the mean (the GPU kernels' rule, emulated);
+    the float64 reference drops those rows itself."""
+    import torch.nn.functional as F
+    import pcd_ops
+    g = torch.Generator().manual_seed(4)
+    V = 13
+    x = torch.randn(3, 5, 8, generator=g)
+    w, b = torch.randn(V, 8, generator=g), torch.randn(V, generator=g)
+    tg = torch.randint(0, V, (3, 5), generator=g)
+    tg[0, 1], tg[1, 3], tg[2, 0], tg[2, 4] = V, -100, V + 5, 1 << 40
+    xe, we, be = (t.clone().requires_grad_(True) for t in (x, w, b))
+    loss = pcd_ops.vocab_cross_entropy(xe, we, be, tg)
+    loss.backward()
+    keep = ((tg >= 0) & (tg < V)).flatten()
+    xr, wr, br = (t.double().requires_grad_(True) for t in (x, w, b))
+    ref = F.cross_entropy(F.linear(xr, wr, br).flatten(end_dim=1)[keep], tg.flatten()[keep])
+    ref.backward()
+    P.assert_close(loss, ref, 1e-6, "loss")
+    for got, r, name in ((xe.grad, xr.grad, "dx"), (we.grad, wr.grad, "dw"), (be.grad, br.grad, "db")):
+        P.assert_close(got, r, 1e-5, name)

@@ -126,7 +126,6 @@ def test_w_step_with_wgrad_overlap_matches_golden():
         pcd_ops.set_wgrad_overlap(False)
 
 
-# tcgen05 3xTF32 projection (nn.Linear drop-in) vs an fp64 reference: forward, dX (split-K), dW, db; ragged tiles
 @pytest.mark.parametrize("cpp,cp,C,red,rp,H,B", [(48, 48, 16, False, False, 64, 5), (64, 128, 64, True, True, 32, 7),
                                                  (128, 256, 64, False, True, 16, 9), (48, 64, 32, True, False, 64, 1)])
 def test_cell_production_geometry_ragged_batch(cpp, cp, C, red, rp, H, B):
@@ -137,9 +136,14 @@ def test_cell_production_geometry_ragged_batch(cpp, cp, C, red, rp, H, B):
 
 @pytest.mark.parametrize("M,K,N", [(1920, 512, 17858), (64, 512, 1000), (120, 36, 70), (256, 1024, 512), (64, 12544, 512),
                                    (64, 1000, 1000), (6, 16, 12)])
-def test_linear_3xtf32_vs_fp64(M, K, N):
+def test_linear_3xtf32_vs_fp64(M, K, N, monkeypatch):
+    """Linear3xTF32Function (nn.Linear drop-in) vs an fp64 reference: forward, dX (split-K), dW, db, ragged tiles.  The
+    size threshold is lifted so that the products linear_3xtf32 would send to the FMA kernel (covered by
+    test_small_linear_vs_fp64) run on the tcgen05 GEMM as well."""
     import torch.nn.functional as F
+    import pcd_ops
     from pcd_ops import linear_3xtf32
+    monkeypatch.setattr(pcd_ops, "_TC_MIN_FLOP", 0.0)
     g = torch.Generator().manual_seed(M + K + N)
     L = 4 if M % 4 == 0 else 2
     x = torch.randn(M // L, L, K, generator=g).to(DEV).requires_grad_(True)

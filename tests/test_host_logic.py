@@ -37,3 +37,24 @@ def test_auto_split_fills_whole_rounds():
         s = f(m, n, k)
         bk = 16 if n >= 256 else 32
         assert 1 <= s <= max(1, min(32, -(-k // bk) // 8))
+
+
+def test_3xtf32_acceptance_rejects_fewer_terms():
+    """The criterion the GPU sweep of pcd_gemm_tn_3xtf32 applies (helpers.accept_3xtf32) can fail: at every shape of that
+    sweep it accepts the 3-term split product hi*hi + hi*lo + lo*hi (operands truncated as kind::tf32 truncates them) and
+    rejects the 1-term product and both 2-term products (either correction dropped)."""
+    from helpers import GEMM_CASES, accept_3xtf32, gemm_errors, trunc_tf32
+    g = torch.Generator().manual_seed(0)
+    for m, n, k, _, _, _, has_bias in GEMM_CASES:
+        a, b = torch.randn(m, k, generator=g), torch.randn(n, k, generator=g)
+        bias = torch.randn(n, generator=g) if has_bias else None
+        ah, bh = trunc_tf32(a), trunc_tf32(b)
+        al, bl = trunc_tf32(a - ah).double(), trunc_tf32(b - bh).double()
+        ah, bh = ah.double(), bh.double()
+        bias64 = 0.0 if bias is None else bias.double()
+        terms = {"hi*hi": ah @ bh.T, "hi*lo": ah @ bl.T, "lo*hi": al @ bh.T}
+        for kept, want in ((("hi*hi",), False), (("hi*hi", "hi*lo"), False), (("hi*hi", "lo*hi"), False),
+                           (("hi*hi", "hi*lo", "lo*hi"), True)):
+            c = sum(terms[t] for t in kept) + bias64
+            errs = gemm_errors(c, a, b, bias)
+            assert accept_3xtf32(*errs) == want, (m, n, k, kept, errs)
