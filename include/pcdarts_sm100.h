@@ -477,6 +477,27 @@ int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int ro
                       const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
                       const float* b_out, long long* tokens, float* work, void* stream);
 
+/* Beam-search question decode (QstEncoder.generate with deterministic=True and beam_size = K > 1) in the same kernel.
+ * Items b = 0..B-1, beams k = 0..K-1, rows r = b*K + k, exactly T words (no end-of-sequence handling, no length penalty).
+ *   t = 0:     every row of item b starts from h = h0[b], c = c0[b] with input tanh(emb[start_token]); the beam scores start
+ *              at (0, -inf, ..., -inf), so only beam 0 of an item contributes candidates.
+ *   each step: per row one LSTM step gives (h_t, c_t); logits l_r = tanh(h_t) w_out^T + b_out; log-probabilities
+ *              lambda_r = l_r - logsumexp(l_r) (temperature 1).  The candidates of item b are the pairs (k, v) scored
+ *              s_{b,k} + lambda_{b,k}[v]; the K highest become the new beams j = 0..K-1 in descending order, exact ties going
+ *              to the lower k, then the lower v.  Beam j takes over the (h_t, c_t) of its parent row, and its next input is
+ *              emb[v_j] (no tanh, as the greedy decode after the start token).
+ *   output:    tokens [B][K][T] int64, the words on beam j's path (backtracked through the parent pointers); scores [B][K]
+ *              fp32, the cumulative log-probability of that path; beams best first.
+ * Envelope: H, E and V as pcd_decode_greedy, 1 <= K <= 8, K <= V, B*K <= 64 rows; PCD_ERR_UNSUPPORTED outside it, PCD_ERR_ARG
+ * for a null pointer, PCD_ERR_ALIGN as pcd_decode_greedy.  work: pcd_decode_beam_work_floats(B, K, H, V) floats, 16-byte
+ * aligned; tokens is also used as scratch until the kernel ends.  The call only uses caller-owned memory and neither
+ * synchronises nor allocates (CUDA-graph capturable).  All reductions run in a fixed order: equal inputs give bit-equal
+ * outputs. */
+size_t pcd_decode_beam_work_floats(int B, int K, int H, int V);
+int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                    const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                    const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Drop-path node sum of the derived network's cells (pcdarts/model.py; DARTS's drop_path on every non-Identity op output):
  *     forward : out[b]     = d1(b) * h1[b] + d2(b) * h2[b]

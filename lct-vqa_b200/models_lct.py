@@ -7,7 +7,7 @@ import torch.nn as nn
 
 import config
 import pcd_ops
-from pcd_ops import decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
+from pcd_ops import decode_beam, decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
 from pcdarts.model_search import Network
 
 
@@ -32,12 +32,13 @@ class ImgEncoder(nn.Module):
 
 class QstEncoder(nn.Module):
     def __init__(self, qst_vocab_size, word_embed_size, embed_size, num_layers, hidden_size, deterministic=True,
-                 temperature=0.1, max_length=30):
+                 temperature=0.1, max_length=30, beam_size=1):
         super().__init__()
         self.hidden_size = hidden_size
         self.deterministic = deterministic
         self.temperature = temperature
         self.max_length = max_length
+        self.beam_size = beam_size          # > 1: deterministic decoding by beam search; generate() returns the best beam
         self.word2vec = nn.Embedding(qst_vocab_size, word_embed_size)
         self.tanh = nn.Tanh()
         self.lstm = nn.LSTM(word_embed_size, hidden_size, num_layers)
@@ -75,9 +76,14 @@ class QstEncoder(nn.Module):
         return torch.multinomial(soft[:, 0, :], 1)
 
     def generate(self, image_embedding):
-        """Greedy / sampled 30-step decode from <start> = 2 (models_lct.py:124-157); the word choice is not differentiable."""
+        """Greedy / sampled / beam-search 30-step decode from <start> = 2 (models_lct.py:124-157); the word choice is not
+        differentiable."""
         batch = len(image_embedding)
         h0 = image_embedding.reshape(batch, self.hidden_size)
+        if self.beam_size > 1:       # beam search runs on the decode kernel only: no stock loop outside its envelope
+            if not self.deterministic:
+                raise ValueError(f"beam_size = {self.beam_size} needs deterministic=True (beam search is not sampled)")
+            return decode_beam(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.beam_size)[0][:, 0].contiguous()
         if self.deterministic and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
             return decode_greedy(h0, self.lstm, self.word2vec, self.fc2, self.max_length)      # one persistent kernel
         if self.deterministic is False and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
@@ -157,6 +163,6 @@ class VqaModel(nn.Module):
         twin.img_encoder.darts = self.img_encoder.darts.new()
         _copy_dropout(self, twin)
         # the unrolled twin generates ArchitectLct's pseudo questions: it decodes the way this model was configured to
-        for name in ("deterministic", "temperature", "max_length"):
+        for name in ("deterministic", "temperature", "max_length", "beam_size"):
             setattr(twin.qst_encoder, name, getattr(self.qst_encoder, name))
         return twin.to(config.DEVICE)

@@ -126,7 +126,7 @@ EXPORTS = ("pcd_launch_count", "pcd_profile_enable", "pcd_profile_num_kernels", 
            "pcd_preprocess_forward", "pcd_preprocess_backward", "pcd_adaptive_avgpool_forward", "pcd_adaptive_avgpool_backward",
            "pcd_gemm_tn_3xtf32", "pcd_set_overlap", "pcd_overlap_join", "pcd_ce_forward", "pcd_ce_backward",
            "pcd_transpose_pad", "pcd_lstm_pbuf_floats", "pcd_lstm_forward", "pcd_lstm_backward",
-           "pcd_decode_work_floats", "pcd_decode_greedy", "pcd_decode_sample", "pcd_flat_max_runs", "pcd_flat_axpy", "pcd_flat_scale",
+           "pcd_decode_work_floats", "pcd_decode_greedy", "pcd_decode_sample", "pcd_decode_beam_work_floats", "pcd_decode_beam", "pcd_flat_max_runs", "pcd_flat_axpy", "pcd_flat_scale",
            "pcd_flat_sumsq", "pcd_flat_sumsq_work", "pcd_flat_adam", "pcd_gemm_small_f32",
            "pcd_dwconv_forward", "pcd_dwconv_backward", "pcd_pwconv_forward", "pcd_pwconv_backward", "pcd_bn_apply",
            "pcd_bn_backward_stats", "pcd_pool3x3_forward", "pcd_pool3x3_backward", "pcd_channel_affine",
@@ -168,6 +168,9 @@ def _declare(lib):
     lib.pcd_decode_work_floats.argtypes = [C.c_int, C.c_int, C.c_int]
     lib.pcd_decode_greedy.argtypes = [C.c_int] * 6 + [vp] * 12
     lib.pcd_decode_sample.argtypes = [C.c_int] * 7 + [C.c_float] + [vp] * 13
+    lib.pcd_decode_beam_work_floats.restype = C.c_size_t
+    lib.pcd_decode_beam_work_floats.argtypes = [C.c_int] * 4
+    lib.pcd_decode_beam.argtypes = [C.c_int] * 7 + [vp] * 13
     lib.pcd_transpose_pad.argtypes = [vp, C.c_longlong, C.c_int, C.c_int, vp, C.c_longlong, vp]
     lib.pcd_gemm_tn_3xtf32.argtypes = [vp, C.c_longlong, vp, C.c_longlong, vp, C.c_longlong, C.c_int, C.c_int, C.c_int, vp,
                                        C.c_int, vp]

@@ -977,7 +977,7 @@ def lstm_forward(lstm, x, h0, c0):
 
 
 # --------------------------------------------------------------------------------------------
-# Question decode (QstEncoder.generate): one persistent cooperative kernel, greedy or sampled
+# Question decode (QstEncoder.generate): one persistent cooperative kernel, greedy, sampled or beam search
 # --------------------------------------------------------------------------------------------
 def decode_supported(h0, lstm, word2vec, proj):
     """Shapes pcd_decode_greedy / pcd_decode_sample take (single-layer LSTM, hidden a multiple of 32 up to 512, E % 4 == 0;
@@ -988,19 +988,22 @@ def decode_supported(h0, lstm, word2vec, proj):
         proj.in_features == H and proj.bias is not None and h0.dtype == torch.float32
 
 
-def _decode_operands(h0, lstm, word2vec, proj, max_length):
+def _decode_operands(h0, lstm, word2vec, proj, max_length, tokens=True):
     """(lib, leading int arguments, pointer arguments, tensors behind the pointers, tokens) of one decode launch over at most
-    64 rows.  The caller holds the tensors until the launch is enqueued."""
+    64 rows.  The caller holds the tensors until the launch is enqueued.  tokens=False: the pointer arguments stop after the
+    parameters (the beam decode has outputs and a workspace of its own)."""
     lib = N.lib_for(h0)
     B, H = h0.shape
     V, E = word2vec.weight.shape
     h0c = _f32c(h0)
     ops = [_f32c(t) for t in (word2vec.weight, lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0)]
     wout, bout = _f32c(proj.weight), _f32c(proj.bias)
+    params = [N.ptr(t) for t in ops] + [N.ptr(h0c), N.ptr(h0c), N.ptr(wout), N.ptr(bout)]
+    if not tokens:
+        return lib, (max_length, B, H, E, V), params, ops + [h0c, wout, bout], None
     tokens = torch.empty((B, max_length), dtype=torch.long, device=h0.device)
     work = torch.empty(int(lib.pcd_decode_work_floats(B, H, V)), dtype=torch.float32, device=h0.device)
-    ptrs = [N.ptr(t) for t in ops] + [N.ptr(h0c), N.ptr(h0c), N.ptr(wout), N.ptr(bout), N.ptr(tokens), N.ptr(work),
-                                      N.stream_for(h0)]
+    ptrs = params + [N.ptr(tokens), N.ptr(work), N.stream_for(h0)]
     return lib, (max_length, B, H, E, V), ptrs, ops + [h0c, wout, bout, work], tokens
 
 
@@ -1039,3 +1042,36 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
         N.check(lib, lib.pcd_decode_sample(*dims, start_token, b0, t32, N.ptr(seed), *ptrs), "pcd_decode_sample")
         out.append(tokens)
     return out[0] if len(out) == 1 else torch.cat(out, 0)
+
+
+_MAX_BEAM = 8
+
+
+def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2):
+    """Beam search over exactly `max_length` words from `start_token` with h0 = c0 = `h0` (B, H) (pcd_decode_beam): at every
+    step each item keeps the `beam_size` = K paths of highest cumulative log-probability.  Returns (tokens (B, K, max_length)
+    int64, scores (B, K) float32), beams best first; beam_size = 1 is the greedy decode scored by its log-probability.
+    Batches are decoded in slices of floor(64 / K) items (the kernel takes 64 rows); items are independent, so the result does
+    not depend on the slicing.  Not differentiable: parameters are read detached."""
+    V = proj.out_features
+    if isinstance(beam_size, bool) or int(beam_size) != beam_size or not 1 <= beam_size <= _MAX_BEAM or beam_size > V:
+        raise ValueError(f"decode_beam: beam_size must be an integer in [1, min({_MAX_BEAM}, vocabulary size {V})], "
+                         f"got {beam_size}")
+    K = int(beam_size)
+    if not decode_supported(h0, lstm, word2vec, proj):
+        raise RuntimeError(f"decode_beam: LSTM(layers={lstm.num_layers}, H={lstm.hidden_size}) with E = "
+                           f"{word2vec.embedding_dim} is outside the decode kernel's envelope (PCD_ERR_UNSUPPORTED)")
+    per = _LSTM_BATCH // K
+    tokens, scores = [], []
+    for b0 in range(0, h0.shape[0], per):
+        lib, dims, ptrs, _keep, _ = _decode_operands(h0[b0:b0 + per], lstm, word2vec, proj, max_length, tokens=False)
+        T, B, H, E, V = dims
+        tok = torch.empty((B, K, T), dtype=torch.long, device=h0.device)
+        sc = torch.empty((B, K), dtype=torch.float32, device=h0.device)
+        work = torch.empty(int(lib.pcd_decode_beam_work_floats(B, K, H, V)), dtype=torch.float32, device=h0.device)
+        N.check(lib, lib.pcd_decode_beam(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
+                                         N.stream_for(h0)), "pcd_decode_beam")
+        tokens.append(tok); scores.append(sc)
+    if len(tokens) == 1:
+        return tokens[0], scores[0]
+    return torch.cat(tokens, 0), torch.cat(scores, 0)

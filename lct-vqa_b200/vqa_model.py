@@ -16,7 +16,7 @@ import torch.nn as nn
 
 import config
 import pcd_ops
-from pcd_ops import decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
+from pcd_ops import decode_beam, decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
 from pcdarts.model_search import Network
 
 
@@ -58,12 +58,13 @@ class QstEncoder(nn.Module):
     logits (vqa_model.py:77-196; QstEncoderBase and QstEncoder merged, names unchanged)."""
 
     def __init__(self, qst_vocab_size, word_embed_size, embed_size, num_layers, hidden_size,
-                 deterministic=True, temperature=0.1, max_length=30):
+                 deterministic=True, temperature=0.1, max_length=30, beam_size=1):
         super().__init__()
         self.hidden_size = hidden_size
         self.deterministic = deterministic
         self.temperature = temperature
         self.max_length = max_length
+        self.beam_size = beam_size          # > 1: deterministic decoding by beam search; generate() returns the best beam
         self.word2vec = nn.Embedding(qst_vocab_size, word_embed_size)
         self.tanh = nn.Tanh()
         self.lstm = nn.LSTM(word_embed_size, hidden_size, num_layers)
@@ -104,9 +105,13 @@ class QstEncoder(nn.Module):
         return torch.multinomial(soft[:, 0, :], 1)
 
     def generate(self, image_embedding):
-        """Greedy / sampled 30-step decode from the <start> token (index 2)  (vqa_model.py:103-136)."""
+        """Greedy / sampled / beam-search 30-step decode from the <start> token (index 2)  (vqa_model.py:103-136)."""
         batch = len(image_embedding)
         h0 = image_embedding.reshape(batch, self.hidden_size)
+        if self.beam_size > 1:       # beam search runs on the decode kernel only: no stock loop outside its envelope
+            if not self.deterministic:
+                raise ValueError(f"beam_size = {self.beam_size} needs deterministic=True (beam search is not sampled)")
+            return decode_beam(h0, self.lstm, self.word2vec, self.fc1, self.max_length, self.beam_size)[0][:, 0].contiguous()
         if self.deterministic and decode_supported(h0, self.lstm, self.word2vec, self.fc1):
             return decode_greedy(h0, self.lstm, self.word2vec, self.fc1, self.max_length)      # one persistent kernel
         if self.deterministic is False and decode_supported(h0, self.lstm, self.word2vec, self.fc1):
