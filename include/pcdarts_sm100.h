@@ -478,7 +478,8 @@ int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int ro
                       const float* b_out, long long* tokens, float* work, void* stream);
 
 /* Beam-search question decode (QstEncoder.generate with deterministic=True and beam_size = K > 1) in the same kernel.
- * Items b = 0..B-1, beams k = 0..K-1, rows r = b*K + k, exactly T words (no end-of-sequence handling, no length penalty).
+ * Items b = 0..B-1, beams k = 0..K-1, rows r = b*K + k, exactly T words (no end-of-sequence handling, no length penalty:
+ * pcd_decode_beam_stop below adds both).
  *   t = 0:     every row of item b starts from h = h0[b], c = c0[b] with input tanh(emb[start_token]); the beam scores start
  *              at (0, -inf, ..., -inf), so only beam 0 of an item contributes candidates.
  *   each step: per row one LSTM step gives (h_t, c_t); logits l_r = tanh(h_t) w_out^T + b_out; log-probabilities
@@ -497,6 +498,41 @@ size_t pcd_decode_beam_work_floats(int B, int K, int H, int V);
 int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
                     const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
                     const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void* stream);
+
+/* End-of-sequence decoding: the three decodes above with a stop word E = end_token, a padding word P = pad_token and, for
+ * beams, a length penalty alpha = length_penalty.  Arguments, envelope, workspace and capturability as the call without
+ * _stop; `stop` is a HOST pointer read at the call.
+ *   greedy, sampled: every word is chosen exactly as without the stop; once a row has emitted E, every later position is P
+ *              (E itself stays).  A stopped decode therefore equals the unstopped one truncated after the first E and filled
+ *              with P, bit for bit (rows are independent, the sampled noise depends on (seed, t, row, v) only).
+ *   beam:      a beam is finished once its last word is E.  A live beam k contributes the candidates (k, v) for every v, raw
+ *              score s_k + lambda_k[v]; a finished beam contributes exactly one, (k, P), with its raw score s_k unchanged.
+ *              Candidates are ranked by the key s / powf((float)L, alpha) in fp32 (s itself when alpha = 0), L the
+ *              hypothesis length counting E: t + 1 for a live candidate at step t, the frozen length for a finished beam.
+ *              Ties as pcd_decode_beam (lower k, then lower v).  scores returns the raw cumulative log-probability of each
+ *              path up to and including E (P adds 0); beams come out best first by key.  With alpha = 0 and E never
+ *              emitted the result is bit-equal to pcd_decode_beam.
+ *   early exit: once every row of the launch has finished, the kernel leaves its time loop and the remaining positions are
+ *              P (beams: the backtrack starts from the last step run).
+ * PCD_ERR_ARG for a null `stop`, an E or P outside [0, V) or an alpha that is not finite, and as the call without _stop. */
+typedef struct pcd_decode_stop {
+    int end_token;
+    int pad_token;
+    float length_penalty;     /* beam only */
+} pcd_decode_stop;
+
+int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                           const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                           const float* w_out, const float* b_out, long long* tokens, float* work,
+                           const pcd_decode_stop* stop, void* stream);
+int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                           const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                           const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                           const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop, void* stream);
+int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                         const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                         const float* w_out, const float* b_out, long long* tokens, float* scores, float* work,
+                         const pcd_decode_stop* stop, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Drop-path node sum of the derived network's cells (pcdarts/model.py; DARTS's drop_path on every non-Identity op output):

@@ -23,6 +23,12 @@
 // writes (word, parent row) packed into tokens[row][t]; the next phase A reads a row's word, stages h_{t-1} and reads c_{t-1}
 // of its parent row (c_t goes to a double-buffered [2][rows][H] buffer), and after the last step block 0 backtracks the
 // parent pointers in place.  An item's top K lies in the union of its rows' per-tile top K, so the reduction is exact.
+// End-of-sequence decoding (kStop = true, one more instantiation per mode): a greedy / sampled row that has emitted
+// end_token is fed pad_token and its later words are replaced by it (a per-row flag in shared memory); a finished beam
+// contributes the single candidate (k, pad_token) with its score unchanged, the merge ranks by score / L^length_penalty and
+// carries the raw score beside that key, and each row's frozen length persists in the workspace.  Every block sees every
+// row's state (greedy / sampled: pick_words runs everywhere; beam: the lengths are read behind the merge barrier), so all
+// blocks leave the time loop at the same step once every row has finished, without another barrier.
 #include "../../include/pcdarts_sm100.h"
 #include "pcd_launch.cuh"
 #include "pcd_philox.cuh"
@@ -42,6 +48,9 @@ static inline bool beam_ok(int B, int K, int V) { return K >= 1 && K <= kMaxK &&
 static inline bool sample_args_ok(float temperature, const unsigned long long* seed, int row_offset) {
     return seed && row_offset >= 0 && isfinite(temperature) && temperature > 0.f;
 }
+static inline bool stop_args_ok(const pcd_decode_stop* s, int V) {
+    return s && s->end_token >= 0 && s->end_token < V && s->pad_token >= 0 && s->pad_token < V && isfinite(s->length_penalty);
+}
 }  // namespace decode
 }  // namespace pcd
 
@@ -50,10 +59,10 @@ extern "C" size_t pcd_decode_work_floats(int B, int H, int V) {
 }
 
 // hbuf [2][rows][H] | tbuf [rows][H] | cbuf [2][rows][H] | top-K candidates [rows][ntiles][K] float2 |
-// tile (max, sum exp) [rows][ntiles] float2 | beam scores [rows]
+// tile (max, sum exp) [rows][ntiles] float2 | beam scores [rows] | finished lengths [rows] int (end-of-sequence decode)
 extern "C" size_t pcd_decode_beam_work_floats(int B, int K, int H, int V) {
     const size_t rows = (size_t)B * K;
-    return 5 * rows * H + 2 * rows * pcd::decode::tiles_of(V) * (K + 1) + rows;
+    return 5 * rows * H + 2 * rows * pcd::decode::tiles_of(V) * (K + 1) + 2 * rows;
 }
 
 #if PCD_CUDA
@@ -80,6 +89,10 @@ struct Args {
     float2* bstat;        // [B][ntiles]     (max, sum exp(logit - max)) of a row's tile
     float* bscore;        // [B]  cumulative log-probability of each beam
     float* scores;        // [B]  output
+    // end-of-sequence decode only (kStop)
+    int end_token, pad_token;
+    float length_penalty; // beam: candidates ranked by score / L^length_penalty (0: by score)
+    int* blen;            // [B]  beam: length of a finished beam counting end_token, 0 while it is live
 };
 
 enum { kGreedy = 0, kSampled = 1, kBeam = 2 };
@@ -169,70 +182,137 @@ __device__ __forceinline__ void warp_pop(float (&ls)[kMaxK], int (&lk)[kMaxK], f
     }
 }
 
+// the same two with a third value carried beside each entry (the end-of-sequence merge ranks by key, returns raw scores)
+__device__ __forceinline__ void list_insert(float (&ls)[kMaxK], int (&lk)[kMaxK], float (&lr)[kMaxK], float sc, int key, float raw) {
+#pragma unroll
+    for (int q = 0; q < kMaxK; ++q)
+        if (better(sc, key, ls[q], lk[q])) {
+            const float ts = ls[q], tr = lr[q]; const int tk = lk[q];
+            ls[q] = sc; lk[q] = key; lr[q] = raw; sc = ts; key = tk; raw = tr;
+        }
+}
+
+__device__ __forceinline__ void warp_pop(float (&ls)[kMaxK], int (&lk)[kMaxK], float (&lr)[kMaxK], float& best, int& bk,
+                                         float& braw) {
+    best = ls[0]; bk = lk[0]; braw = lr[0];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+        const int ok = __shfl_xor_sync(0xffffffffu, bk, o);
+        const float orw = __shfl_xor_sync(0xffffffffu, braw, o);
+        if (better(ov, ok, best, bk)) { best = ov; bk = ok; braw = orw; }
+    }
+    if (bk != INT_MAX && lk[0] == bk) {
+#pragma unroll
+        for (int q = 0; q < kMaxK - 1; ++q) { ls[q] = ls[q + 1]; lk[q] = lk[q + 1]; lr[q] = lr[q + 1]; }
+        ls[kMaxK - 1] = -INFINITY; lk[kMaxK - 1] = INT_MAX; lr[kMaxK - 1] = -INFINITY;
+    }
+}
+
+// ranking key of a hypothesis of length L with raw score s: s / L^alpha (s itself for alpha = 0)
+__device__ __forceinline__ float rank_key(float s, int L, float alpha) { return alpha != 0.f ? s / powf((float)L, alpha) : s; }
+
 // step t of the beam decode, behind a grid barrier: block i merges items i, i + gridDim.x, ...  S is free shared memory.
 // Every reduction runs in a fixed order, so the result does not change from run to run.
+// kStop: a finished beam k (FL[k] = its frozen length) skips its tile candidates and its log-sum-exp and contributes the one
+// candidate (k, pad_token) with its score unchanged; candidates are ranked by rank_key, the raw score travels beside the key.
+template <bool kStop>
 __device__ __forceinline__ void merge_beams(const Args& a, int t, float* S) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, K = a.K, nt = a.ntiles, per_row = nt * K;
     float* LSE = S;                                      // [kMaxK]
     float* SC = S + kMaxK;                               // [kMaxK] scores of the beams at step t - 1
     float* WS = S + 2 * kMaxK;                           // [8 warps][kMaxK] each warp's top K
     int* WK = reinterpret_cast<int*>(WS + 8 * kMaxK);
+    float* WR = reinterpret_cast<float*>(WK + 8 * kMaxK);   // kStop: [8 warps][kMaxK] raw scores beside the keys WS
+    int* FL = reinterpret_cast<int*>(WR + 8 * kMaxK);       // kStop: [kMaxK] frozen length of a finished beam, 0 while live
     for (int item = blockIdx.x; item < a.B / K; item += gridDim.x) {
         const int r0 = item * K;
         if (warp < K) {                                  // warp k: log-sum-exp of row r0 + k over its tiles
+            int fl = 0;
+            if constexpr (kStop) fl = t ? __ldcg(a.blen + r0 + warp) : 0;
             const float2* st = a.bstat + (long long)(r0 + warp) * nt;
             float m = -INFINITY;
-            for (int l = lane; l < nt; l += 32) m = fmaxf(m, __ldcg(st + l).x);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
             float s = 0.f;
-            for (int l = lane; l < nt; l += 32) { const float2 p = __ldcg(st + l); s += p.y * expf(p.x - m); }
+            if (!fl) {
+                for (int l = lane; l < nt; l += 32) m = fmaxf(m, __ldcg(st + l).x);
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-            s = __shfl_sync(0xffffffffu, s, 0);
+                for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+                for (int l = lane; l < nt; l += 32) { const float2 p = __ldcg(st + l); s += p.y * expf(p.x - m); }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+                s = __shfl_sync(0xffffffffu, s, 0);
+            }
             if (lane == 0) {
                 LSE[warp] = m + logf(s);
                 SC[warp] = t ? __ldcg(a.bscore + r0 + warp) : (warp ? -INFINITY : 0.f);   // t = 0: only beam 0 is live
+                if constexpr (kStop) FL[warp] = fl;
             }
         }
         __syncthreads();
         // the item's K rows x ntiles x K candidates are contiguous; each thread keeps its best kMaxK
-        float ls[kMaxK];
+        float ls[kMaxK], lr[kMaxK];
         int lk[kMaxK];
 #pragma unroll
-        for (int q = 0; q < kMaxK; ++q) { ls[q] = -INFINITY; lk[q] = INT_MAX; }
+        for (int q = 0; q < kMaxK; ++q) { ls[q] = -INFINITY; lk[q] = INT_MAX; lr[q] = -INFINITY; }
         const float2* cb = a.bcand + (long long)r0 * per_row;
-        for (int i = threadIdx.x; i < K * per_row; i += kT) {
-            const float2 c = __ldcg(cb + i);
-            const int v = __float_as_int(c.y), k = i / per_row;
-            if (v < a.V) list_insert(ls, lk, SC[k] + (c.x - LSE[k]), k * a.V + v);
+        if constexpr (kStop) {
+            const float alpha = a.length_penalty;
+            for (int i = threadIdx.x; i < K * per_row; i += kT) {
+                const int k = i / per_row;
+                if (FL[k]) continue;
+                const float2 c = __ldcg(cb + i);
+                const int v = __float_as_int(c.y);
+                if (v < a.V) {
+                    const float raw = SC[k] + (c.x - LSE[k]);
+                    list_insert(ls, lk, lr, rank_key(raw, t + 1, alpha), k * a.V + v, raw);
+                }
+            }
+            const int k = threadIdx.x;
+            if (k < K && FL[k]) list_insert(ls, lk, lr, rank_key(SC[k], FL[k], alpha), k * a.V + a.pad_token, SC[k]);
+        } else {
+            for (int i = threadIdx.x; i < K * per_row; i += kT) {
+                const float2 c = __ldcg(cb + i);
+                const int v = __float_as_int(c.y), k = i / per_row;
+                if (v < a.V) list_insert(ls, lk, SC[k] + (c.x - LSE[k]), k * a.V + v);
+            }
         }
         for (int j = 0; j < K; ++j) {
             float best; int bk;
-            warp_pop(ls, lk, best, bk);
+            if constexpr (kStop) {
+                float braw;
+                warp_pop(ls, lk, lr, best, bk, braw);
+                if (lane == 0) WR[warp * kMaxK + j] = braw;
+            } else warp_pop(ls, lk, best, bk);
             if (lane == 0) { WS[warp * kMaxK + j] = best; WK[warp * kMaxK + j] = bk; }
         }
         __syncthreads();
         if (warp == 0) {                                 // the 8 warps' lists -> the item's top K, best first
 #pragma unroll
-            for (int q = 0; q < kMaxK; ++q) { ls[q] = -INFINITY; lk[q] = INT_MAX; }
+            for (int q = 0; q < kMaxK; ++q) { ls[q] = -INFINITY; lk[q] = INT_MAX; lr[q] = -INFINITY; }
             for (int e = lane; e < 8 * kMaxK; e += 32)
-                if (e % kMaxK < K) list_insert(ls, lk, WS[e], WK[e]);
+                if (e % kMaxK < K) {
+                    if constexpr (kStop) list_insert(ls, lk, lr, WS[e], WK[e], WR[e]);
+                    else list_insert(ls, lk, WS[e], WK[e]);
+                }
             for (int j = 0; j < K; ++j) {
-                float best; int bk;
-                warp_pop(ls, lk, best, bk);
+                float best, braw; int bk;
+                if constexpr (kStop) warp_pop(ls, lk, lr, best, bk, braw);
+                else warp_pop(ls, lk, best, bk);
                 if (lane == 0) {
                     const int k = bk / a.V, v = bk - k * a.V;
                     a.tokens[(long long)(r0 + j) * a.T + t] = (long long)v | ((long long)(r0 + k) << 32);
-                    a.bscore[r0 + j] = best;
+                    if constexpr (kStop) {
+                        a.bscore[r0 + j] = braw;
+                        a.blen[r0 + j] = FL[k] ? FL[k] : (v == a.end_token ? t + 1 : 0);
+                    } else a.bscore[r0 + j] = best;
                 }
             }
         }
-        __syncthreads();                                 // LSE / SC / WS reused by the next item
+        __syncthreads();                                 // LSE / SC / WS / FL reused by the next item
     }
 }
 
-template <int kMode>
+template <int kMode, bool kStop>
 __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
     constexpr bool kSample = kMode == kSampled, kBeamMode = kMode == kBeam;
     cg::grid_group grid = cg::this_grid();
@@ -245,6 +325,7 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
     int* TOK = reinterpret_cast<int*>(U + u_floats(H));            // [64]
     float* XP = reinterpret_cast<float*>(TOK + kMaxB);             // [4 quarters][16 gate rows][64] input-projection partials
     int* PAR = reinterpret_cast<int*>(XP + 64 * kMaxB);            // [64]  beam: the row whose state a row continues
+    int* FIN = PAR;                                                // [64]  greedy / sampled kStop: the row emitted end_token
     const int tid = threadIdx.x;
     const bool gate_block = (int)blockIdx.x < H / kUnits;
     const int u0 = blockIdx.x * kUnits;
@@ -269,12 +350,14 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
         }
     }
     const int nk = H / kKC;
+    int t_run = a.T;                      // kStop: steps run before every row had finished
     for (int t = 0; t < a.T; ++t) {
         // ---- the word chosen at the previous step ------------------------------------------------------------------------
         if (t == 0) {
             if (tid < kMaxB) {
                 TOK[tid] = a.start;
                 if constexpr (kBeamMode) PAR[tid] = tid / a.K;             // every beam of item b starts from h0[b], c0[b]
+                else if constexpr (kStop) FIN[tid] = 0;
             }
         } else if constexpr (kBeamMode) {
             if (tid < B) {
@@ -283,9 +366,25 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
                 PAR[tid] = (int)(p >> 32);
             }
         } else pick_words(a, TOK);
-        __syncthreads();
+        if constexpr (kStop && kBeamMode) {
+            // every block reads every row's finished length behind the merge barrier, so all of them leave at the same step
+            if (!__syncthreads_count(t == 0 || (tid < B && __ldcg(a.blen + tid) == 0))) { t_run = t; break; }
+        } else __syncthreads();
+        if constexpr (kStop && !kBeamMode)
+            if (t > 0) {
+                // word t - 1 of a finished row is pad_token, and so is its next input; every block picked the same words, so
+                // all of them see the last row finish at the same step
+                int live = 0;
+                if (tid < B) {
+                    if (FIN[tid]) TOK[tid] = a.pad_token;
+                    else live = !(FIN[tid] = TOK[tid] == a.end_token);
+                }
+                if (!__syncthreads_count(live)) t_run = t;
+            }
         if constexpr (!kBeamMode)
             if (t > 0 && blockIdx.x == 0 && tid < B) a.tokens[(long long)tid * a.T + t - 1] = TOK[tid];
+        if constexpr (kStop && !kBeamMode)
+            if (t_run == t) break;
         // ---- phase A: one LSTM step for this block's 4 hidden units ----------------------------------------------------------
         if (gate_block) {
             const float* hprev = t ? a.hbuf + (long long)((t - 1) & 1) * B * H : a.h0;
@@ -495,7 +594,7 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
         }
         grid.sync();
         if constexpr (kBeamMode) {
-            merge_beams(a, t, U);
+            merge_beams<kStop>(a, t, U);
             grid.sync();
         }
     }
@@ -503,7 +602,7 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
         // backtrack: column t of every row's (word, parent) is read before any thread overwrites it with the word of the path
         if (blockIdx.x == 0) {
             int cur = tid;
-            for (int t = a.T - 1; t >= 0; --t) {
+            for (int t = (kStop ? t_run : a.T) - 1; t >= 0; --t) {
                 long long p = 0;
                 if (tid < B) p = __ldcg(a.tokens + (long long)cur * a.T + t);
                 __syncthreads();
@@ -513,11 +612,24 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
                 }
             }
             if (tid < B) a.scores[tid] = __ldcg(a.bscore + tid);
+            if constexpr (kStop)
+                if (tid < B)
+                    for (int t = t_run; t < a.T; ++t) a.tokens[(long long)tid * a.T + t] = a.pad_token;
         }
     } else if (blockIdx.x == 0) {
-        pick_words(a, TOK);
-        __syncthreads();
-        if (tid < B) a.tokens[(long long)tid * a.T + a.T - 1] = TOK[tid];
+        if constexpr (kStop) {
+            if (t_run == a.T) {
+                pick_words(a, TOK);
+                __syncthreads();
+                if (tid < B) a.tokens[(long long)tid * a.T + a.T - 1] = FIN[tid] ? a.pad_token : TOK[tid];
+            } else if (tid < B) {
+                for (int t = t_run; t < a.T; ++t) a.tokens[(long long)tid * a.T + t] = a.pad_token;
+            }
+        } else {
+            pick_words(a, TOK);
+            __syncthreads();
+            if (tid < B) a.tokens[(long long)tid * a.T + a.T - 1] = TOK[tid];
+        }
     }
 }
 
@@ -527,25 +639,25 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
 namespace pcd {
 namespace decode {
 
-// B counts rows: items x K for the beam decode
-template <int kMode>
+// B counts rows: items x K for the beam decode; stop is non-null exactly for the kStop instantiations
+template <int kMode, bool kStop = false>
 static int run(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
                const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
                const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
-               float* work, void* stream, int K = 1, float* scores = nullptr) {
+               float* work, void* stream, int K = 1, float* scores = nullptr, const pcd_decode_stop* stop = nullptr) {
     if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
     if (!shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
     if ((((uintptr_t)emb) | ((uintptr_t)w_ih) | ((uintptr_t)w_hh) | ((uintptr_t)h0) | ((uintptr_t)w_out) | ((uintptr_t)work)) & 15) return PCD_ERR_ALIGN;
     if (((uintptr_t)seed) & 7) return PCD_ERR_ALIGN;
     LaunchState& L = launch_state();
     const size_t smem = ((size_t)16 * (H + 4) + (size_t)16 * (E + 4) + (size_t)u_floats(H) + kMaxB + 64 * kMaxB +
-                         (kMode == kBeam ? kMaxB : 0)) * sizeof(float);
+                         (kMode == kBeam || kStop ? kMaxB : 0)) * sizeof(float);
     if (smem > 227 * 1024) return PCD_ERR_UNSUPPORTED;
     static int sms = 0;                                     // per instantiation: each one sets its own smem attribute
     if (!sms) {
         int dev = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-            cudaFuncSetAttribute(decode_kernel<kMode>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            cudaFuncSetAttribute(decode_kernel<kMode, kStop>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
             sms = 0;
             snprintf(L.last_err, sizeof L.last_err, "decode setup: %s", cudaGetErrorString(cudaGetLastError()));
             return PCD_ERR_CUDA;
@@ -569,8 +681,13 @@ static int run(int T, int B, int H, int E, int V, int start_token, int row_offse
     a.bstat = a.bcand + (size_t)B * ntiles * K;
     a.bscore = reinterpret_cast<float*>(a.bstat + (size_t)B * ntiles);
     a.scores = scores;
+    a.end_token = stop ? stop->end_token : -1;
+    a.pad_token = stop ? stop->pad_token : 0;
+    a.length_penalty = stop ? stop->length_penalty : 0.f;
+    a.blen = reinterpret_cast<int*>(a.bscore + B);
     void* args[] = {&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)decode_kernel<kMode>, dim3(grid), dim3(kT), args, smem, (cudaStream_t)stream);
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)decode_kernel<kMode, kStop>, dim3(grid), dim3(kT), args, smem,
+                                                (cudaStream_t)stream);
     count_launch(L);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) {
@@ -610,6 +727,37 @@ extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int sta
                                                 c0, w_out, b_out, tokens, work, stream, K, scores);
 }
 
+extern "C" int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                                      const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                                      const float* w_out, const float* b_out, long long* tokens, float* work,
+                                      const pcd_decode_stop* stop, void* stream) {
+    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    return pcd::decode::run<pcd::decode::kGreedy, true>(T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh,
+                                                        h0, c0, w_out, b_out, tokens, work, stream, 1, nullptr, stop);
+}
+
+extern "C" int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                                      const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop,
+                                      void* stream) {
+    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset) || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    return pcd::decode::run<pcd::decode::kSampled, true>(T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih,
+                                                         w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, work, stream, 1,
+                                                         nullptr, stop);
+}
+
+extern "C" int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb,
+                                    const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* h0,
+                                    const float* c0, const float* w_out, const float* b_out, long long* tokens, float* scores,
+                                    float* work, const pcd_decode_stop* stop, void* stream) {
+    if (!scores || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    if (!pcd::decode::beam_ok(B, K, V)) return emb && w_ih && w_hh && b_ih && b_hh && h0 && c0 && w_out && b_out && tokens && work
+                                                   ? PCD_ERR_UNSUPPORTED : PCD_ERR_ARG;
+    return pcd::decode::run<pcd::decode::kBeam, true>(T, B * K, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh,
+                                                      h0, c0, w_out, b_out, tokens, work, stream, K, scores, stop);
+}
+
 #else   // ---- CPU emulation build (tests only) ----------------------------------------------------------------------
 
 #include <math.h>
@@ -619,11 +767,12 @@ extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int sta
 static inline float sigm_(float x) { return 1.f / (1.f + expf(-x)); }
 
 // the kernel's arithmetic per row and step: fp64 gate and vocabulary sums rounded to fp32, argmax of the fp32 logit (greedy)
-// or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go to the lowest index
+// or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go to the lowest index.  stop: after end_token a row's
+// remaining positions are pad_token (rows are independent, so the row simply ends there)
 static int decode_emu(bool sample, int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
                       const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
                       const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
-                      float* work) {
+                      float* work, const pcd_decode_stop* stop = nullptr) {
     if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
     if (!pcd::decode::shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
     const unsigned long long key = sample ? *seed : 0ull;
@@ -657,6 +806,10 @@ static int decode_emu(bool sample, int T, int B, int H, int E, int V, int start_
             }
             word = bi;
             tokens[(long long)b * T + t] = bi;
+            if (stop && bi == stop->end_token) {
+                for (int tt = t + 1; tt < T; ++tt) tokens[(long long)b * T + tt] = stop->pad_token;
+                break;
+            }
         }
     }
     return PCD_OK;
@@ -679,24 +832,30 @@ extern "C" int pcd_decode_sample(int T, int B, int H, int E, int V, int start_to
 }
 
 // beam decode with the kernel's semantics: fp64 gate and vocabulary sums rounded to fp32, lambda = logit - lse in fp32
-// (lse from fp64 sums), candidate score s_k + lambda in fp32, ties to the lower beam, then the lower word
-extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                               const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                               const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void*) {
+// (lse from fp64 sums), candidate score s_k + lambda in fp32, ties to the lower beam, then the lower word.  stop: the
+// candidates of pcd_decode_beam_stop ranked by key, raw scores beside them, and the loop ends once every row has finished
+static int beam_emu(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                    const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                    const float* b_out, long long* tokens, float* scores, float* work, const pcd_decode_stop* stop) {
     if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !scores || !work) return PCD_ERR_ARG;
     if (!pcd::decode::beam_ok(B, K, V) || !pcd::decode::shape_ok(T, B * K, H, E, V) || start_token < 0 || start_token >= V)
         return PCD_ERR_UNSUPPORTED;
     const int R = B * K;
+    const float alpha = stop ? stop->length_penalty : 0.f;
+    auto rank_key = [alpha](float sc, int L) { return alpha != 0.f ? sc / powf((float)L, alpha) : sc; };
     std::vector<float> h((size_t)R * H), c((size_t)R * H), hn((size_t)R * H), cn((size_t)R * H), x((size_t)E), s((size_t)H);
     std::vector<float> lam((size_t)R * V), score((size_t)R), nscore((size_t)R);
     std::vector<int> word((size_t)R, start_token), hist_w((size_t)T * R), hist_p((size_t)T * R);
+    std::vector<int> len((size_t)R, 0), nlen((size_t)R, 0);     // stop: frozen length of a finished beam, 0 while live
     for (int r = 0; r < R; ++r) {
         std::copy(h0 + (size_t)(r / K) * H, h0 + (size_t)(r / K + 1) * H, h.begin() + (size_t)r * H);
         std::copy(c0 + (size_t)(r / K) * H, c0 + (size_t)(r / K + 1) * H, c.begin() + (size_t)r * H);
         score[r] = r % K ? -INFINITY : 0.f;
     }
+    int t_run = T;
     for (int t = 0; t < T; ++t) {
         for (int r = 0; r < R; ++r) {
+            if (len[r]) continue;                         // finished: its state is never used again
             for (int k = 0; k < E; ++k) x[k] = t ? emb[(long long)word[r] * E + k] : tanhf(emb[(long long)word[r] * E + k]);
             const float* hr = h.data() + (size_t)r * H;
             for (int j = 0; j < H; ++j) {
@@ -725,37 +884,83 @@ extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int sta
             const float lse = (float)(mx + log(se));
             for (int v = 0; v < V; ++v) lr[v] = lr[v] - lse;
         }
-        for (int b = 0; b < B; ++b) {                     // top K of the item's K x V candidates, best first
-            std::vector<float> bs(K, -INFINITY);
+        for (int b = 0; b < B; ++b) {                     // top K of the item's candidates by key, best first
+            std::vector<float> bs(K, -INFINITY), braw(K, -INFINITY);
             std::vector<int> bk(K, INT_MAX);
-            for (int k = 0; k < K; ++k)
-                for (int v = 0; v < V; ++v) {
-                    float sc = score[b * K + k] + lam[(size_t)(b * K + k) * V + v];
-                    int key = k * V + v;
-                    for (int q = 0; q < K; ++q)
-                        if (sc > bs[q] || (sc == bs[q] && key < bk[q])) { std::swap(sc, bs[q]); std::swap(key, bk[q]); }
+            auto insert = [&](float sc, int key, float raw) {
+                for (int q = 0; q < K; ++q)
+                    if (sc > bs[q] || (sc == bs[q] && key < bk[q])) {
+                        std::swap(sc, bs[q]); std::swap(key, bk[q]); std::swap(raw, braw[q]);
+                    }
+            };
+            for (int k = 0; k < K; ++k) {
+                const int r = b * K + k;
+                if (len[r]) {                             // a finished beam: the one candidate (k, pad_token), score unchanged
+                    insert(rank_key(score[r], len[r]), k * V + stop->pad_token, score[r]);
+                    continue;
                 }
+                for (int v = 0; v < V; ++v) {
+                    const float raw = score[r] + lam[(size_t)r * V + v];
+                    insert(stop ? rank_key(raw, t + 1) : raw, k * V + v, raw);
+                }
+            }
             for (int j = 0; j < K; ++j) {
-                const int r = b * K + j, parent = b * K + bk[j] / V;
-                hist_w[(size_t)t * R + r] = bk[j] % V;
+                const int r = b * K + j, parent = b * K + bk[j] / V, v = bk[j] % V;
+                hist_w[(size_t)t * R + r] = v;
                 hist_p[(size_t)t * R + r] = parent;
-                word[r] = bk[j] % V;
-                nscore[r] = bs[j];
+                word[r] = v;
+                nscore[r] = braw[j];
+                nlen[r] = len[parent] ? len[parent] : (stop && v == stop->end_token ? t + 1 : 0);
                 std::copy(hn.begin() + (size_t)parent * H, hn.begin() + (size_t)(parent + 1) * H, h.begin() + (size_t)r * H);
                 std::copy(cn.begin() + (size_t)parent * H, cn.begin() + (size_t)(parent + 1) * H, c.begin() + (size_t)r * H);
             }
         }
         score.swap(nscore);
+        len.swap(nlen);
+        if (std::all_of(len.begin(), len.end(), [](int l) { return l > 0; })) { t_run = t + 1; break; }
     }
     for (int r = 0; r < R; ++r) {
         int cur = r;
-        for (int t = T - 1; t >= 0; --t) {
+        for (int t = t_run - 1; t >= 0; --t) {
             tokens[(long long)r * T + t] = hist_w[(size_t)t * R + cur];
             cur = hist_p[(size_t)t * R + cur];
         }
+        for (int t = t_run; t < T; ++t) tokens[(long long)r * T + t] = stop->pad_token;
         scores[r] = score[r];
     }
     return PCD_OK;
+}
+
+extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                               const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                               const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void*) {
+    return beam_emu(T, B, K, H, E, V, start_token, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, scores, work, nullptr);
+}
+
+extern "C" int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
+                                      const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
+                                      const float* w_out, const float* b_out, long long* tokens, float* work,
+                                      const pcd_decode_stop* stop, void*) {
+    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    return decode_emu(false, T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens,
+                      work, stop);
+}
+
+extern "C" int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
+                                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
+                                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
+                                      const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop, void*) {
+    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset) || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    return decode_emu(true, T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out,
+                      b_out, tokens, work, stop);
+}
+
+extern "C" int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb,
+                                    const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* h0,
+                                    const float* c0, const float* w_out, const float* b_out, long long* tokens, float* scores,
+                                    float* work, const pcd_decode_stop* stop, void*) {
+    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
+    return beam_emu(T, B, K, H, E, V, start_token, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, scores, work, stop);
 }
 
 #endif

@@ -32,13 +32,15 @@ class ImgEncoder(nn.Module):
 
 class QstEncoder(nn.Module):
     def __init__(self, qst_vocab_size, word_embed_size, embed_size, num_layers, hidden_size, deterministic=True,
-                 temperature=0.1, max_length=30, beam_size=1):
+                 temperature=0.1, max_length=30, beam_size=1, end_token=None, length_penalty=0.0):
         super().__init__()
         self.hidden_size = hidden_size
         self.deterministic = deterministic
         self.temperature = temperature
         self.max_length = max_length
         self.beam_size = beam_size          # > 1: deterministic decoding by beam search; generate() returns the best beam
+        self.end_token = end_token          # set (<end> = 3): words after it are <pad> = 0, and the decode stops early
+        self.length_penalty = length_penalty    # beams with end_token: ranked by log-probability / length^length_penalty
         self.word2vec = nn.Embedding(qst_vocab_size, word_embed_size)
         self.tanh = nn.Tanh()
         self.lstm = nn.LSTM(word_embed_size, hidden_size, num_layers)
@@ -83,12 +85,17 @@ class QstEncoder(nn.Module):
         if self.beam_size > 1:       # beam search runs on the decode kernel only: no stock loop outside its envelope
             if not self.deterministic:
                 raise ValueError(f"beam_size = {self.beam_size} needs deterministic=True (beam search is not sampled)")
-            return decode_beam(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.beam_size)[0][:, 0].contiguous()
-        if self.deterministic and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
-            return decode_greedy(h0, self.lstm, self.word2vec, self.fc2, self.max_length)      # one persistent kernel
-        if self.deterministic is False and decode_supported(h0, self.lstm, self.word2vec, self.fc2):
+            return decode_beam(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.beam_size,
+                               end_token=self.end_token, length_penalty=self.length_penalty)[0][:, 0].contiguous()
+        # end-of-sequence decoding runs on the decode kernel only: decode_greedy / decode_sample raise outside its envelope
+        stop = self.end_token is not None
+        if self.deterministic and (stop or decode_supported(h0, self.lstm, self.word2vec, self.fc2)):
+            return decode_greedy(h0, self.lstm, self.word2vec, self.fc2, self.max_length,      # one persistent kernel
+                                 end_token=self.end_token)
+        if self.deterministic is False and (stop or decode_supported(h0, self.lstm, self.word2vec, self.fc2)):
             # the same kernel, words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
-            return decode_sample(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.temperature)
+            return decode_sample(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.temperature,
+                                 end_token=self.end_token)
         if self.deterministic:       # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
             pcd_ops._stock(f"greedy decode with hidden size {self.hidden_size}")
         # sampled decoding outside the kernel's envelope: the reference's module loop (torch.multinomial)
@@ -163,6 +170,6 @@ class VqaModel(nn.Module):
         twin.img_encoder.darts = self.img_encoder.darts.new()
         _copy_dropout(self, twin)
         # the unrolled twin generates ArchitectLct's pseudo questions: it decodes the way this model was configured to
-        for name in ("deterministic", "temperature", "max_length", "beam_size"):
+        for name in ("deterministic", "temperature", "max_length", "beam_size", "end_token", "length_penalty"):
             setattr(twin.qst_encoder, name, getattr(self.qst_encoder, name))
         return twin.to(config.DEVICE)

@@ -1007,28 +1007,62 @@ def _decode_operands(h0, lstm, word2vec, proj, max_length, tokens=True):
     return lib, (max_length, B, H, E, V), ptrs, ops + [h0c, wout, bout, work], tokens
 
 
-def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2):
+def _decode_stop(V, end_token, pad_token, length_penalty=0.0):
+    """The pcd_decode_stop of an end-of-sequence decode (None for end_token=None: the call without _stop).  ValueError for an
+    end or pad word outside [0, V) or a length penalty that is not finite."""
+    if end_token is None:                               # every hypothesis has max_length words: length_penalty is not used
+        return None
+    a32 = C.c_float(float(length_penalty)).value        # what the kernel divides by
+    if not math.isfinite(a32):
+        raise ValueError(f"decode: length_penalty must be finite, got {length_penalty}")
+    for name, w in (("end_token", end_token), ("pad_token", pad_token)):
+        if isinstance(w, bool) or int(w) != w or not 0 <= w < V:
+            raise ValueError(f"decode: {name} must be an integer in [0, vocabulary size {V}), got {w}")
+    return N.DecodeStop(int(end_token), int(pad_token), a32)
+
+
+def _check_envelope(what, h0, lstm, word2vec, proj):
+    """Modes that exist on the decode kernel only (beams, end-of-sequence decoding): no stock loop outside its envelope."""
+    if not decode_supported(h0, lstm, word2vec, proj):
+        raise RuntimeError(f"{what}: LSTM(layers={lstm.num_layers}, H={lstm.hidden_size}) with E = "
+                           f"{word2vec.embedding_dim} is outside the decode kernel's envelope (PCD_ERR_UNSUPPORTED)")
+
+
+def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2, end_token=None, pad_token=0):
     """tokens (B, max_length) int64 of the greedy decode that starts from `start_token` with h0 = c0 = `h0` (B, H).
+    end_token: once a row has emitted it, its later positions are `pad_token` (pcd_decode_greedy_stop): the unstopped decode
+    truncated after the first end_token, and the kernel stops when every row of a launch has finished.
     Not differentiable (neither is the reference's argmax): parameters are read detached."""
+    stop = _decode_stop(proj.out_features, end_token, pad_token)
+    if stop is not None:
+        _check_envelope("decode_greedy", h0, lstm, word2vec, proj)
     if h0.shape[0] > _LSTM_BATCH:          # independent rows: ceil(B / 64) launches of the persistent kernel
-        return torch.cat([decode_greedy(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length, start_token)
-                          for b0 in range(0, h0.shape[0], _LSTM_BATCH)], 0)
+        return torch.cat([decode_greedy(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length, start_token, end_token,
+                                        pad_token) for b0 in range(0, h0.shape[0], _LSTM_BATCH)], 0)
     lib, dims, ptrs, _keep, tokens = _decode_operands(h0, lstm, word2vec, proj, max_length)
-    N.check(lib, lib.pcd_decode_greedy(*dims, start_token, *ptrs), "pcd_decode_greedy")
+    if stop is None:
+        N.check(lib, lib.pcd_decode_greedy(*dims, start_token, *ptrs), "pcd_decode_greedy")
+    else:
+        N.check(lib, lib.pcd_decode_greedy_stop(*dims, start_token, *ptrs[:-1], C.byref(stop), ptrs[-1]),
+                "pcd_decode_greedy_stop")
     return tokens
 
 
-def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None):
+def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None, end_token=None, pad_token=0):
     """tokens (B, max_length) int64 of the sampled decode (QstEncoder.sample with deterministic=False): every word is drawn from
     softmax(logits / temperature), by the Gumbel-max trick on counter-based Philox noise (pcd_decode_sample).
 
     seed: None draws one 64-bit seed per call on h0's device from torch's generator (so torch.manual_seed reproduces a run, and
     a call captured in a CUDA graph draws a fresh seed on every replay); a Python int, or a 1-element int64 tensor on h0's
     device read when the kernel runs, fixes the words.  Batches above 64 are decoded in slices of 64 with one seed: the noise
-    of a row depends on its index in the whole batch, so the words do not depend on the slicing.  Not differentiable."""
+    of a row depends on its index in the whole batch, so the words do not depend on the slicing.  end_token / pad_token as
+    decode_greedy (pcd_decode_sample_stop): the same words up to the first end_token.  Not differentiable."""
     t32 = C.c_float(float(temperature)).value           # what the kernel divides by
     if not math.isfinite(t32) or t32 <= 0.0:
         raise ValueError(f"decode_sample: temperature must be finite and > 0, got {temperature}")
+    stop = _decode_stop(proj.out_features, end_token, pad_token)
+    if stop is not None:
+        _check_envelope("decode_sample", h0, lstm, word2vec, proj)
     if seed is None:
         seed = torch.empty(1, dtype=torch.int64, device=h0.device).random_(-2 ** 63, None)
     elif not torch.is_tensor(seed):
@@ -1039,7 +1073,11 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
     out = []
     for b0 in range(0, h0.shape[0], _LSTM_BATCH):
         lib, dims, ptrs, _keep, tokens = _decode_operands(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length)
-        N.check(lib, lib.pcd_decode_sample(*dims, start_token, b0, t32, N.ptr(seed), *ptrs), "pcd_decode_sample")
+        if stop is None:
+            N.check(lib, lib.pcd_decode_sample(*dims, start_token, b0, t32, N.ptr(seed), *ptrs), "pcd_decode_sample")
+        else:
+            N.check(lib, lib.pcd_decode_sample_stop(*dims, start_token, b0, t32, N.ptr(seed), *ptrs[:-1], C.byref(stop),
+                                                    ptrs[-1]), "pcd_decode_sample_stop")
         out.append(tokens)
     return out[0] if len(out) == 1 else torch.cat(out, 0)
 
@@ -1047,10 +1085,15 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
 _MAX_BEAM = 8
 
 
-def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2):
+def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2, end_token=None, pad_token=0,
+                length_penalty=0.0):
     """Beam search over exactly `max_length` words from `start_token` with h0 = c0 = `h0` (B, H) (pcd_decode_beam): at every
     step each item keeps the `beam_size` = K paths of highest cumulative log-probability.  Returns (tokens (B, K, max_length)
     int64, scores (B, K) float32), beams best first; beam_size = 1 is the greedy decode scored by its log-probability.
+    end_token (pcd_decode_beam_stop): a beam whose last word is end_token is finished and continues with `pad_token` at no
+    cost; beams are ranked by score / length^length_penalty (length counting end_token), scores are the log-probabilities of
+    the paths up to end_token, and the kernel stops once every beam of a launch has finished.  Without end_token every
+    hypothesis has max_length words and length_penalty is not used.
     Batches are decoded in slices of floor(64 / K) items (the kernel takes 64 rows); items are independent, so the result does
     not depend on the slicing.  Not differentiable: parameters are read detached."""
     V = proj.out_features
@@ -1058,9 +1101,8 @@ def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2):
         raise ValueError(f"decode_beam: beam_size must be an integer in [1, min({_MAX_BEAM}, vocabulary size {V})], "
                          f"got {beam_size}")
     K = int(beam_size)
-    if not decode_supported(h0, lstm, word2vec, proj):
-        raise RuntimeError(f"decode_beam: LSTM(layers={lstm.num_layers}, H={lstm.hidden_size}) with E = "
-                           f"{word2vec.embedding_dim} is outside the decode kernel's envelope (PCD_ERR_UNSUPPORTED)")
+    stop = _decode_stop(V, end_token, pad_token, length_penalty)
+    _check_envelope("decode_beam", h0, lstm, word2vec, proj)
     per = _LSTM_BATCH // K
     tokens, scores = [], []
     for b0 in range(0, h0.shape[0], per):
@@ -1069,8 +1111,12 @@ def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2):
         tok = torch.empty((B, K, T), dtype=torch.long, device=h0.device)
         sc = torch.empty((B, K), dtype=torch.float32, device=h0.device)
         work = torch.empty(int(lib.pcd_decode_beam_work_floats(B, K, H, V)), dtype=torch.float32, device=h0.device)
-        N.check(lib, lib.pcd_decode_beam(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
-                                         N.stream_for(h0)), "pcd_decode_beam")
+        if stop is None:
+            N.check(lib, lib.pcd_decode_beam(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
+                                             N.stream_for(h0)), "pcd_decode_beam")
+        else:
+            N.check(lib, lib.pcd_decode_beam_stop(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
+                                                  C.byref(stop), N.stream_for(h0)), "pcd_decode_beam_stop")
         tokens.append(tok); scores.append(sc)
     if len(tokens) == 1:
         return tokens[0], scores[0]
