@@ -451,57 +451,40 @@ int pcd_lstm_backward(int T, int B, int H, const float* dhs, const float* dhT, c
                       float* pbuf, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Greedy question decode: replaces QstEncoder.generate's 30-iteration loop of embedding -> nn.LSTM step -> tanh -> Linear(H, V)
- * -> argmax (darts_vqa/vqa_model.py:103-136, basic_vqa/models_lct.py:124-157, deterministic sampling) with one persistent
- * cooperative kernel.  The first input is tanh(emb[start_token]), later inputs emb[previous word] (no tanh: vqa_model.py:133);
- * gate order i, f, g, o; ties in the argmax go to the lowest index.  tokens: [B][T] int64.  B <= 64, H a multiple of 32 up to
- * 512, E a multiple of 4.  work: pcd_decode_work_floats(B, H, V) floats, 16-byte aligned.
- * ---------------------------------------------------------------------------------------------- */
-size_t pcd_decode_work_floats(int B, int H, int V);
-int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                      const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                      const float* w_out, const float* b_out, long long* tokens, float* work, void* stream);
-
-/* Sampled question decode (QstEncoder.generate with deterministic=False: every word drawn from softmax(logits / temperature),
- * darts_vqa/vqa_model.py:87-92) in the same kernel, by the Gumbel-max trick: word t of row b is
- *     argmax_v ( logit_v / temperature + G(seed, t, row_offset + b, v) )
- * with G a standard Gumbel variable from Philox4x32-10:  key = {seed & 0xffffffff, seed >> 32}, counter = {v >> 2, t, row, 0},
- * x = word (v & 3) of the block, u = ((float)(x >> 9) + 0.5f) * 2^-23, G = -logf(-logf(u)).  The noise depends only on
- * (seed, t, row, v): a batch decoded in slices (row_offset = first row of the slice) draws what one call would.  `seed` is a
- * DEVICE pointer to one 8-byte-aligned uint64, read by the kernel (the call is CUDA-graph capturable; a graph replays the
- * seed the buffer holds at replay time).  Envelope, token layout and workspace as pcd_decode_greedy.  PCD_ERR_ARG for a null
- * seed, a negative row_offset or a temperature that is not finite and > 0.  The distribution equals torch.multinomial's;
- * the random stream does not. */
-int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                      const float* b_out, long long* tokens, float* work, void* stream);
-
-/* Beam-search question decode (QstEncoder.generate with deterministic=True and beam_size = K > 1) in the same kernel.
- * Items b = 0..B-1, beams k = 0..K-1, rows r = b*K + k, exactly T words (no end-of-sequence handling, no length penalty:
- * pcd_decode_beam_stop below adds both).
- *   t = 0:     every row of item b starts from h = h0[b], c = c0[b] with input tanh(emb[start_token]); the beam scores start
- *              at (0, -inf, ..., -inf), so only beam 0 of an item contributes candidates.
- *   each step: per row one LSTM step gives (h_t, c_t); logits l_r = tanh(h_t) w_out^T + b_out; log-probabilities
- *              lambda_r = l_r - logsumexp(l_r) (temperature 1).  The candidates of item b are the pairs (k, v) scored
- *              s_{b,k} + lambda_{b,k}[v]; the K highest become the new beams j = 0..K-1 in descending order, exact ties going
- *              to the lower k, then the lower v.  Beam j takes over the (h_t, c_t) of its parent row, and its next input is
- *              emb[v_j] (no tanh, as the greedy decode after the start token).
- *   output:    tokens [B][K][T] int64, the words on beam j's path (backtracked through the parent pointers); scores [B][K]
- *              fp32, the cumulative log-probability of that path; beams best first.
- * Envelope: H, E and V as pcd_decode_greedy, 1 <= K <= 8, K <= V, B*K <= 64 rows; PCD_ERR_UNSUPPORTED outside it, PCD_ERR_ARG
- * for a null pointer, PCD_ERR_ALIGN as pcd_decode_greedy.  work: pcd_decode_beam_work_floats(B, K, H, V) floats, 16-byte
- * aligned; tokens is also used as scratch until the kernel ends.  The call only uses caller-owned memory and neither
- * synchronises nor allocates (CUDA-graph capturable).  All reductions run in a fixed order: equal inputs give bit-equal
- * outputs. */
-size_t pcd_decode_beam_work_floats(int B, int K, int H, int V);
-int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                    const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                    const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void* stream);
-
-/* End-of-sequence decoding: the three decodes above with a stop word E = end_token, a padding word P = pad_token and, for
- * beams, a length penalty alpha = length_penalty.  Arguments, envelope, workspace and capturability as the call without
- * _stop; `stop` is a HOST pointer read at the call.
+ * Question decode: replaces QstEncoder.generate's 30-iteration loop of embedding -> nn.LSTM step -> tanh -> Linear(H, V)
+ * -> argmax (darts_vqa/vqa_model.py:103-136, basic_vqa/models_lct.py:124-157) with one persistent cooperative kernel, in
+ * one of three modes, each with or without end-of-sequence decoding.  One pcd_decode_args describes a call; the struct is
+ * a HOST pointer read at the call, every pointer in it is device memory.
+ *
+ * Every mode: h = h0[row], c = c0[row]; the first input is tanh(emb[start_token]), later inputs emb[previous word] (no tanh:
+ * vqa_model.py:133); gate order i, f, g, o; logits l = tanh(h_t) w_out^T + b_out.
+ *   PCD_DECODE_GREEDY (deterministic sampling): word t of row b is argmax_v l_v, ties to the lowest index.
+ *              tokens: [B][T] int64.
+ *   PCD_DECODE_SAMPLED (QstEncoder.generate with deterministic=False: every word drawn from softmax(logits / temperature),
+ *              darts_vqa/vqa_model.py:87-92), by the Gumbel-max trick: word t of row b is
+ *                  argmax_v ( logit_v / temperature + G(seed, t, row_offset + b, v) )
+ *              with G a standard Gumbel variable from Philox4x32-10:  key = {seed & 0xffffffff, seed >> 32}, counter =
+ *              {v >> 2, t, row, 0}, x = word (v & 3) of the block, u = ((float)(x >> 9) + 0.5f) * 2^-23, G = -logf(-logf(u)).
+ *              The noise depends only on (seed, t, row, v): a batch decoded in slices (row_offset = first row of the slice)
+ *              draws what one call would.  `seed` is a DEVICE pointer to one 8-byte-aligned uint64, read by the kernel (a
+ *              CUDA graph replays the seed the buffer holds at replay time).  The distribution equals torch.multinomial's;
+ *              the random stream does not.  tokens: [B][T] int64.
+ *   PCD_DECODE_BEAM (QstEncoder.generate with deterministic=True and beam_size = K > 1): items b = 0..B-1, beams
+ *              k = 0..K-1, rows r = b*K + k.
+ *     t = 0:     every row of item b starts from h = h0[b], c = c0[b] with input tanh(emb[start_token]); the beam scores start
+ *                at (0, -inf, ..., -inf), so only beam 0 of an item contributes candidates.
+ *     each step: per row one LSTM step gives (h_t, c_t) and the logits l_r; log-probabilities lambda_r = l_r - logsumexp(l_r)
+ *                (temperature 1).  The candidates of item b are the pairs (k, v) scored s_{b,k} + lambda_{b,k}[v]; the K
+ *                highest become the new beams j = 0..K-1 in descending order, exact ties going to the lower k, then the
+ *                lower v.  Beam j takes over the (h_t, c_t) of its parent row, and its next input is emb[v_j] (no tanh, as
+ *                the greedy decode after the start token).
+ *     output:    tokens [B][K][T] int64, the words on beam j's path (backtracked through the parent pointers); scores
+ *                [B][K] fp32, the cumulative log-probability of that path; beams best first.  tokens is also used as
+ *                scratch until the kernel ends.
+ * Without the stop (stop = 0) every row has exactly T words, and beams have no length penalty.
+ *
+ * End-of-sequence decoding (stop = 1): a stop word E = end_token, a padding word P = pad_token and, for beams, a length
+ * penalty alpha = length_penalty.
  *   greedy, sampled: every word is chosen exactly as without the stop; once a row has emitted E, every later position is P
  *              (E itself stays).  A stopped decode therefore equals the unstopped one truncated after the first E and filled
  *              with P, bit for bit (rows are independent, the sampled noise depends on (seed, t, row, v) only).
@@ -509,30 +492,42 @@ int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, c
  *              score s_k + lambda_k[v]; a finished beam contributes exactly one, (k, P), with its raw score s_k unchanged.
  *              Candidates are ranked by the key s / powf((float)L, alpha) in fp32 (s itself when alpha = 0), L the
  *              hypothesis length counting E: t + 1 for a live candidate at step t, the frozen length for a finished beam.
- *              Ties as pcd_decode_beam (lower k, then lower v).  scores returns the raw cumulative log-probability of each
- *              path up to and including E (P adds 0); beams come out best first by key.  With alpha = 0 and E never
- *              emitted the result is bit-equal to pcd_decode_beam.
+ *              Ties as without the stop (lower k, then lower v).  scores returns the raw cumulative log-probability of
+ *              each path up to and including E (P adds 0); beams come out best first by key.  With alpha = 0 and E never
+ *              emitted the result is bit-equal to the decode without the stop.
  *   early exit: once every row of the launch has finished, the kernel leaves its time loop and the remaining positions are
  *              P (beams: the backtrack starts from the last step run).
- * PCD_ERR_ARG for a null `stop`, an E or P outside [0, V) or an alpha that is not finite, and as the call without _stop. */
-typedef struct pcd_decode_stop {
-    int end_token;
-    int pad_token;
-    float length_penalty;     /* beam only */
-} pcd_decode_stop;
+ *
+ * Envelope: H a multiple of 32 up to 512, E a multiple of 4, start_token in [0, V); greedy and sampled: B <= 64 rows; beam:
+ * 1 <= K <= 8, K <= V, B*K <= 64 rows.  PCD_ERR_UNSUPPORTED outside it.
+ * PCD_ERR_ARG, before any shape check: a mode outside the three; K != 1 outside beam mode; a null emb .. b_out, tokens or
+ * work, or a null scores in beam mode; sampled: a null seed, a negative row_offset or a temperature that is not finite and
+ * > 0; stop: an E or P outside [0, V) or an alpha that is not finite.
+ * PCD_ERR_ALIGN: emb, w_ih, w_hh, h0, w_out and work must be 16-byte aligned, the seed 8-byte aligned.
+ * work: pcd_decode_work_floats(a) floats (it reads mode, B, K, H and V).  The call only uses caller-owned memory and
+ * neither synchronises nor allocates (CUDA-graph capturable).  All reductions run in a fixed order: equal inputs give
+ * bit-equal outputs.
+ * ---------------------------------------------------------------------------------------------- */
+enum { PCD_DECODE_GREEDY = 0, PCD_DECODE_SAMPLED = 1, PCD_DECODE_BEAM = 2 };
 
-int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                           const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                           const float* w_out, const float* b_out, long long* tokens, float* work,
-                           const pcd_decode_stop* stop, void* stream);
-int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                           const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                           const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                           const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop, void* stream);
-int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                         const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                         const float* w_out, const float* b_out, long long* tokens, float* scores, float* work,
-                         const pcd_decode_stop* stop, void* stream);
+typedef struct pcd_decode_args {
+    int mode;                         /* PCD_DECODE_* */
+    int T, B, K, H, E, V;             /* B: rows (greedy, sampled) or items (beam); K: beams per item, 1 outside beam mode */
+    int start_token;
+    int stop;                         /* 1: end-of-sequence decoding */
+    int end_token, pad_token;         /* stop only */
+    float length_penalty;             /* beam with stop only */
+    float temperature;                /* sampled only */
+    int row_offset;                   /* sampled only: global index of row 0 */
+    const unsigned long long* seed;   /* sampled only */
+    const float *emb, *w_ih, *w_hh, *b_ih, *b_hh, *h0, *c0, *w_out, *b_out;
+    long long* tokens;                /* [B][T]; beam [B][K][T] */
+    float* scores;                    /* beam only: [B][K] */
+    float* work;
+} pcd_decode_args;
+
+size_t pcd_decode_work_floats(const pcd_decode_args* a);
+int pcd_decode(const pcd_decode_args* a, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Drop-path node sum of the derived network's cells (pcdarts/model.py; DARTS's drop_path on every non-Identity op output):

@@ -37,6 +37,7 @@
 
 namespace pcd {
 namespace decode {
+enum { kGreedy = PCD_DECODE_GREEDY, kSampled = PCD_DECODE_SAMPLED, kBeam = PCD_DECODE_BEAM };
 constexpr int kT = 256, kUnits = 4, kMaxB = 64, kMaxK = 8, kTileN = 128, kKC = 32, kWP = kKC + 4, kStages = 4, kPickJ = 5;
 constexpr int kStageFloats = (kMaxB + kTileN) * kWP;
 PCD_HOSTDEV int u_floats(int H) { return kMaxB * (H + 4) > kStages * kStageFloats ? kMaxB * (H + 4) : kStages * kStageFloats; }
@@ -45,24 +46,52 @@ static inline bool shape_ok(int T, int B, int H, int E, int V) {
     return T > 0 && B > 0 && B <= kMaxB && H >= 32 && H <= 512 && H % 32 == 0 && E > 0 && E % 4 == 0 && V > 0;
 }
 static inline bool beam_ok(int B, int K, int V) { return K >= 1 && K <= kMaxK && K <= V && B >= 1 && B <= kMaxB / K; }
-static inline bool sample_args_ok(float temperature, const unsigned long long* seed, int row_offset) {
-    return seed && row_offset >= 0 && isfinite(temperature) && temperature > 0.f;
+
+// the status of a call before anything device-specific: every PCD_ERR_ARG comes before any shape check, so a beam shape
+// outside the envelope is PCD_ERR_UNSUPPORTED only when every pointer is set
+static int validate(const pcd_decode_args* a) {
+    if (!a || a->mode < kGreedy || a->mode > kBeam || (a->mode != kBeam && a->K != 1)) return PCD_ERR_ARG;
+    if (a->mode == kSampled && !(a->seed && a->row_offset >= 0 && isfinite(a->temperature) && a->temperature > 0.f))
+        return PCD_ERR_ARG;
+    if (a->stop && !(a->end_token >= 0 && a->end_token < a->V && a->pad_token >= 0 && a->pad_token < a->V &&
+                     isfinite(a->length_penalty)))
+        return PCD_ERR_ARG;
+    if (!a->emb || !a->w_ih || !a->w_hh || !a->b_ih || !a->b_hh || !a->h0 || !a->c0 || !a->w_out || !a->b_out || !a->tokens ||
+        !a->work || (a->mode == kBeam && !a->scores))
+        return PCD_ERR_ARG;
+    if (a->mode == kBeam && !beam_ok(a->B, a->K, a->V)) return PCD_ERR_UNSUPPORTED;
+    if (!shape_ok(a->T, a->B * a->K, a->H, a->E, a->V) || a->start_token < 0 || a->start_token >= a->V) return PCD_ERR_UNSUPPORTED;
+    return PCD_OK;
 }
-static inline bool stop_args_ok(const pcd_decode_stop* s, int V) {
-    return s && s->end_token >= 0 && s->end_token < V && s->pad_token >= 0 && s->pad_token < V && isfinite(s->length_penalty);
+
+// workspace offsets in floats, rows = B x K:  hbuf [2][rows][H] | tbuf [rows][H] | then greedy / sampled: candidates
+// [rows][ntiles] float2;  beam: cbuf [2][rows][H] | top-K candidates [rows][ntiles][K] float2 | tile (max, sum exp)
+// [rows][ntiles] float2 | beam scores [rows] | finished lengths [rows] int (end-of-sequence decode)
+struct Work {
+    size_t tbuf, cand, cbuf, bcand, bstat, bscore, blen, floats;
+};
+static Work work_of(int mode, int B, int K, int H, int V) {
+    const size_t rows = (size_t)B * K, nt = tiles_of(V), rh = rows * H;
+    Work w = {};
+    w.tbuf = 2 * rh;
+    if (mode == kBeam) {
+        w.cbuf = 3 * rh;
+        w.bcand = 5 * rh;
+        w.bstat = w.bcand + 2 * rows * nt * K;
+        w.bscore = w.bstat + 2 * rows * nt;
+        w.blen = w.bscore + rows;
+        w.floats = w.blen + rows;
+    } else {
+        w.cand = 3 * rh;
+        w.floats = w.cand + 2 * rows * nt;
+    }
+    return w;
 }
 }  // namespace decode
 }  // namespace pcd
 
-extern "C" size_t pcd_decode_work_floats(int B, int H, int V) {
-    return (size_t)3 * B * H + (size_t)2 * B * pcd::decode::tiles_of(V);
-}
-
-// hbuf [2][rows][H] | tbuf [rows][H] | cbuf [2][rows][H] | top-K candidates [rows][ntiles][K] float2 |
-// tile (max, sum exp) [rows][ntiles] float2 | beam scores [rows] | finished lengths [rows] int (end-of-sequence decode)
-extern "C" size_t pcd_decode_beam_work_floats(int B, int K, int H, int V) {
-    const size_t rows = (size_t)B * K;
-    return 5 * rows * H + 2 * rows * pcd::decode::tiles_of(V) * (K + 1) + 2 * rows;
+extern "C" size_t pcd_decode_work_floats(const pcd_decode_args* a) {
+    return a ? pcd::decode::work_of(a->mode, a->B, a->K, a->H, a->V).floats : 0;
 }
 
 #if PCD_CUDA
@@ -94,8 +123,6 @@ struct Args {
     float length_penalty; // beam: candidates ranked by score / L^length_penalty (0: by score)
     int* blen;            // [B]  beam: length of a finished beam counting end_token, 0 while it is live
 };
-
-enum { kGreedy = 0, kSampled = 1, kBeam = 2 };
 
 __device__ __forceinline__ float sigm(float x) { return 1.f / (1.f + expf(-x)); }
 __device__ __forceinline__ float dot4(float4 a, float4 b, float acc) {
@@ -639,20 +666,9 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
 namespace pcd {
 namespace decode {
 
-// B counts rows: items x K for the beam decode; stop is non-null exactly for the kStop instantiations
-template <int kMode, bool kStop = false>
-static int run(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-               const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
-               const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
-               float* work, void* stream, int K = 1, float* scores = nullptr, const pcd_decode_stop* stop = nullptr) {
-    if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
-    if (!shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
-    if ((((uintptr_t)emb) | ((uintptr_t)w_ih) | ((uintptr_t)w_hh) | ((uintptr_t)h0) | ((uintptr_t)w_out) | ((uintptr_t)work)) & 15) return PCD_ERR_ALIGN;
-    if (((uintptr_t)seed) & 7) return PCD_ERR_ALIGN;
-    LaunchState& L = launch_state();
-    const size_t smem = ((size_t)16 * (H + 4) + (size_t)16 * (E + 4) + (size_t)u_floats(H) + kMaxB + 64 * kMaxB +
-                         (kMode == kBeam || kStop ? kMaxB : 0)) * sizeof(float);
-    if (smem > 227 * 1024) return PCD_ERR_UNSUPPORTED;
+// the kernel of one (mode, stop) pair; its first call reads the SM count and sets the kernel's shared-memory limit
+template <int kMode, bool kStop>
+static const void* kernel_of(int& sms_out, LaunchState& L) {
     static int sms = 0;                                     // per instantiation: each one sets its own smem attribute
     if (!sms) {
         int dev = 0;
@@ -660,34 +676,53 @@ static int run(int T, int B, int H, int E, int V, int start_token, int row_offse
             cudaFuncSetAttribute(decode_kernel<kMode, kStop>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
             sms = 0;
             snprintf(L.last_err, sizeof L.last_err, "decode setup: %s", cudaGetErrorString(cudaGetLastError()));
-            return PCD_ERR_CUDA;
+            return nullptr;
         }
     }
+    sms_out = sms;
+    return (const void*)decode_kernel<kMode, kStop>;
+}
+
+// a call that passed validate(): alignment, shared memory, grid, then one cooperative launch
+static int run(const pcd_decode_args& p, void* stream) {
+    const int B = p.B * p.K, H = p.H, E = p.E, V = p.V;   // B counts rows: items x K for the beam decode
+    if ((((uintptr_t)p.emb) | ((uintptr_t)p.w_ih) | ((uintptr_t)p.w_hh) | ((uintptr_t)p.h0) | ((uintptr_t)p.w_out) | ((uintptr_t)p.work)) & 15) return PCD_ERR_ALIGN;
+    if (p.mode == kSampled && ((uintptr_t)p.seed) & 7) return PCD_ERR_ALIGN;
+    LaunchState& L = launch_state();
+    const size_t smem = ((size_t)16 * (H + 4) + (size_t)16 * (E + 4) + (size_t)u_floats(H) + kMaxB + 64 * kMaxB +
+                         (p.mode == kBeam || p.stop ? kMaxB : 0)) * sizeof(float);
+    if (smem > 227 * 1024) return PCD_ERR_UNSUPPORTED;
+    using KernelOf = const void* (*)(int&, LaunchState&);
+    static const KernelOf kernels[3][2] = {{kernel_of<kGreedy, false>, kernel_of<kGreedy, true>},
+                                           {kernel_of<kSampled, false>, kernel_of<kSampled, true>},
+                                           {kernel_of<kBeam, false>, kernel_of<kBeam, true>}};
+    int sms = 0;
+    const void* kernel = kernels[p.mode][p.stop ? 1 : 0](sms, L);
+    if (!kernel) return PCD_ERR_CUDA;
     const int ntiles = tiles_of(V);
     int grid = ntiles < sms ? ntiles : sms;                 // one block per SM: all of them co-resident (cooperative launch)
     if (grid < H / kUnits) grid = H / kUnits;
     if (grid > sms) return PCD_ERR_UNSUPPORTED;
+    const Work w = work_of(p.mode, p.B, p.K, H, V);
     Args a;
-    a.T = T; a.B = B; a.H = H; a.E = E; a.V = V; a.start = start_token; a.ntiles = ntiles;
-    a.emb = emb; a.w_ih = w_ih; a.w_hh = w_hh; a.b_ih = b_ih; a.b_hh = b_hh; a.h0 = h0; a.c0 = c0; a.w_out = w_out; a.b_out = b_out;
-    a.tokens = tokens;
-    a.hbuf = work;
-    a.tbuf = work + (size_t)2 * B * H;
-    a.cand = reinterpret_cast<float2*>(work + (size_t)3 * B * H);
-    a.seed = seed; a.temperature = temperature; a.row_offset = row_offset;
-    a.K = K;
-    a.cbuf = work + (size_t)3 * B * H;
-    a.bcand = reinterpret_cast<float2*>(work + (size_t)5 * B * H);
-    a.bstat = a.bcand + (size_t)B * ntiles * K;
-    a.bscore = reinterpret_cast<float*>(a.bstat + (size_t)B * ntiles);
-    a.scores = scores;
-    a.end_token = stop ? stop->end_token : -1;
-    a.pad_token = stop ? stop->pad_token : 0;
-    a.length_penalty = stop ? stop->length_penalty : 0.f;
-    a.blen = reinterpret_cast<int*>(a.bscore + B);
+    a.T = p.T; a.B = B; a.H = H; a.E = E; a.V = V; a.start = p.start_token; a.ntiles = ntiles;
+    a.emb = p.emb; a.w_ih = p.w_ih; a.w_hh = p.w_hh; a.b_ih = p.b_ih; a.b_hh = p.b_hh; a.h0 = p.h0; a.c0 = p.c0;
+    a.w_out = p.w_out; a.b_out = p.b_out;
+    a.tokens = p.tokens;
+    a.hbuf = p.work;
+    a.tbuf = p.work + w.tbuf;
+    a.cand = reinterpret_cast<float2*>(p.work + w.cand);
+    a.seed = p.seed; a.temperature = p.temperature; a.row_offset = p.row_offset;
+    a.K = p.K;
+    a.cbuf = p.work + w.cbuf;
+    a.bcand = reinterpret_cast<float2*>(p.work + w.bcand);
+    a.bstat = reinterpret_cast<float2*>(p.work + w.bstat);
+    a.bscore = p.work + w.bscore;
+    a.scores = p.scores;
+    a.end_token = p.end_token; a.pad_token = p.pad_token; a.length_penalty = p.length_penalty;
+    a.blen = reinterpret_cast<int*>(p.work + w.blen);
     void* args[] = {&a};
-    cudaError_t e = cudaLaunchCooperativeKernel((const void*)decode_kernel<kMode, kStop>, dim3(grid), dim3(kT), args, smem,
-                                                (cudaStream_t)stream);
+    cudaError_t e = cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(kT), args, smem, (cudaStream_t)stream);
     count_launch(L);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) {
@@ -700,64 +735,6 @@ static int run(int T, int B, int H, int E, int V, int start_token, int row_offse
 }  // namespace decode
 }  // namespace pcd
 
-extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                 const float* w_out, const float* b_out, long long* tokens, float* work, void* stream) {
-    return pcd::decode::run<pcd::decode::kGreedy>(T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out,
-                                   tokens, work, stream);
-}
-
-extern "C" int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                                 const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                                 const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                                 const float* b_out, long long* tokens, float* work, void* stream) {
-    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset)) return PCD_ERR_ARG;
-    return pcd::decode::run<pcd::decode::kSampled>(T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0,
-                                  w_out, b_out, tokens, work, stream);
-}
-
-extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                               const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                               const float* w_out, const float* b_out, long long* tokens, float* scores, float* work,
-                               void* stream) {
-    if (!scores) return PCD_ERR_ARG;
-    if (!pcd::decode::beam_ok(B, K, V)) return emb && w_ih && w_hh && b_ih && b_hh && h0 && c0 && w_out && b_out && tokens && work
-                                                   ? PCD_ERR_UNSUPPORTED : PCD_ERR_ARG;
-    return pcd::decode::run<pcd::decode::kBeam>(T, B * K, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0,
-                                                c0, w_out, b_out, tokens, work, stream, K, scores);
-}
-
-extern "C" int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                      const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                      const float* w_out, const float* b_out, long long* tokens, float* work,
-                                      const pcd_decode_stop* stop, void* stream) {
-    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    return pcd::decode::run<pcd::decode::kGreedy, true>(T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh,
-                                                        h0, c0, w_out, b_out, tokens, work, stream, 1, nullptr, stop);
-}
-
-extern "C" int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                                      const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop,
-                                      void* stream) {
-    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset) || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    return pcd::decode::run<pcd::decode::kSampled, true>(T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih,
-                                                         w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, work, stream, 1,
-                                                         nullptr, stop);
-}
-
-extern "C" int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb,
-                                    const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* h0,
-                                    const float* c0, const float* w_out, const float* b_out, long long* tokens, float* scores,
-                                    float* work, const pcd_decode_stop* stop, void* stream) {
-    if (!scores || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    if (!pcd::decode::beam_ok(B, K, V)) return emb && w_ih && w_hh && b_ih && b_hh && h0 && c0 && w_out && b_out && tokens && work
-                                                   ? PCD_ERR_UNSUPPORTED : PCD_ERR_ARG;
-    return pcd::decode::run<pcd::decode::kBeam, true>(T, B * K, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh,
-                                                      h0, c0, w_out, b_out, tokens, work, stream, K, scores, stop);
-}
-
 #else   // ---- CPU emulation build (tests only) ----------------------------------------------------------------------
 
 #include <math.h>
@@ -766,48 +743,61 @@ extern "C" int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, in
 
 static inline float sigm_(float x) { return 1.f / (1.f + expf(-x)); }
 
-// the kernel's arithmetic per row and step: fp64 gate and vocabulary sums rounded to fp32, argmax of the fp32 logit (greedy)
-// or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go to the lowest index.  stop: after end_token a row's
-// remaining positions are pad_token (rows are independent, so the row simply ends there)
-static int decode_emu(bool sample, int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh, const float* b_ih,
-                      const float* b_hh, const float* h0, const float* c0, const float* w_out, const float* b_out, long long* tokens,
-                      float* work, const pcd_decode_stop* stop = nullptr) {
-    if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !work) return PCD_ERR_ARG;
-    if (!pcd::decode::shape_ok(T, B, H, E, V) || start_token < 0 || start_token >= V) return PCD_ERR_UNSUPPORTED;
-    const unsigned long long key = sample ? *seed : 0ull;
-    std::vector<float> h(h0, h0 + (size_t)B * H), c(c0, c0 + (size_t)B * H), hn((size_t)H), x((size_t)E), s((size_t)H);
+namespace pcd {
+namespace decode {
+
+// one LSTM step of a row from (h, c) on the input word, and the vocabulary logits of the new state, with the kernel's
+// arithmetic: fp64 gate and vocabulary sums rounded to fp32.  c_out may be c; h_out is not h
+static void step_emu(const pcd_decode_args& a, int word, int t, const float* h, const float* c, float* h_out, float* c_out,
+                     float* logits) {
+    const int H = a.H, E = a.E;
+    std::vector<float> x((size_t)E), s((size_t)H);
+    for (int k = 0; k < E; ++k) x[k] = t ? a.emb[(long long)word * E + k] : tanhf(a.emb[(long long)word * E + k]);
+    for (int j = 0; j < H; ++j) {
+        float g[4];
+        for (int q = 0; q < 4; ++q) {
+            double acc = (double)a.b_ih[q * H + j] + a.b_hh[q * H + j];
+            for (int k = 0; k < E; ++k) acc += (double)x[k] * a.w_ih[(long long)(q * H + j) * E + k];
+            for (int k = 0; k < H; ++k) acc += (double)h[k] * a.w_hh[(long long)(q * H + j) * H + k];
+            g[q] = (float)acc;
+        }
+        const float gi = sigm_(g[0]), gf = sigm_(g[1]), gg = tanhf(g[2]), go = sigm_(g[3]);
+        c_out[j] = gf * c[j] + gi * gg;
+        h_out[j] = go * tanhf(c_out[j]);
+    }
+    for (int j = 0; j < H; ++j) s[j] = tanhf(h_out[j]);
+    for (int v = 0; v < a.V; ++v) {
+        double acc = a.b_out[v];
+        for (int k = 0; k < H; ++k) acc += (double)s[k] * a.w_out[(long long)v * H + k];
+        logits[v] = (float)acc;
+    }
+}
+
+// greedy / sampled: argmax of the fp32 logit (greedy) or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go
+// to the lowest index.  stop: after end_token a row's remaining positions are pad_token (rows are independent, so the row
+// simply ends there)
+static int decode_emu(const pcd_decode_args& a) {
+    const int T = a.T, B = a.B, H = a.H, V = a.V;
+    const bool sample = a.mode == kSampled;
+    const unsigned long long key = sample ? *a.seed : 0ull;
+    std::vector<float> h(a.h0, a.h0 + (size_t)B * H), c(a.c0, a.c0 + (size_t)B * H), hn((size_t)H), logit((size_t)V);
     for (int b = 0; b < B; ++b) {
-        int word = start_token;
+        int word = a.start_token;
+        float* hb = h.data() + (size_t)b * H;
+        float* cb = c.data() + (size_t)b * H;
         for (int t = 0; t < T; ++t) {
-            for (int k = 0; k < E; ++k) x[k] = t ? emb[(long long)word * E + k] : tanhf(emb[(long long)word * E + k]);
-            float* hb = h.data() + (size_t)b * H;
-            float* cb = c.data() + (size_t)b * H;
-            for (int j = 0; j < H; ++j) {
-                float g[4];
-                for (int q = 0; q < 4; ++q) {
-                    double acc = (double)b_ih[q * H + j] + b_hh[q * H + j];
-                    for (int k = 0; k < E; ++k) acc += (double)x[k] * w_ih[(long long)(q * H + j) * E + k];
-                    for (int k = 0; k < H; ++k) acc += (double)hb[k] * w_hh[(long long)(q * H + j) * H + k];
-                    g[q] = (float)acc;
-                }
-                const float gi = sigm_(g[0]), gf = sigm_(g[1]), gg = tanhf(g[2]), go = sigm_(g[3]);
-                cb[j] = gf * cb[j] + gi * gg;
-                hn[j] = go * tanhf(cb[j]);
-            }
-            for (int j = 0; j < H; ++j) { hb[j] = hn[j]; s[j] = tanhf(hn[j]); }
+            step_emu(a, word, t, hb, cb, hn.data(), cb, logit.data());
+            std::copy(hn.begin(), hn.end(), hb);
             float best = -INFINITY;
             int bi = 0;
             for (int v = 0; v < V; ++v) {
-                double acc = b_out[v];
-                for (int k = 0; k < H; ++k) acc += (double)s[k] * w_out[(long long)v * H + k];
-                const float score = sample ? (float)acc / temperature + pcd::decode_gumbel(key, t, row_offset + b, v) : (float)acc;
+                const float score = sample ? logit[v] / a.temperature + decode_gumbel(key, t, a.row_offset + b, v) : logit[v];
                 if (score > best) { best = score; bi = v; }
             }
             word = bi;
-            tokens[(long long)b * T + t] = bi;
-            if (stop && bi == stop->end_token) {
-                for (int tt = t + 1; tt < T; ++tt) tokens[(long long)b * T + tt] = stop->pad_token;
+            a.tokens[(long long)b * T + t] = bi;
+            if (a.stop && bi == a.end_token) {
+                for (int tt = t + 1; tt < T; ++tt) a.tokens[(long long)b * T + tt] = a.pad_token;
                 break;
             }
         }
@@ -815,70 +805,31 @@ static int decode_emu(bool sample, int T, int B, int H, int E, int V, int start_
     return PCD_OK;
 }
 
-extern "C" int pcd_decode_greedy(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                 const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                 const float* w_out, const float* b_out, long long* tokens, float* work, void*) {
-    return decode_emu(false, T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens,
-                      work);
-}
-
-extern "C" int pcd_decode_sample(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                                 const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                                 const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                                 const float* b_out, long long* tokens, float* work, void*) {
-    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset)) return PCD_ERR_ARG;
-    return decode_emu(true, T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out,
-                      b_out, tokens, work);
-}
-
-// beam decode with the kernel's semantics: fp64 gate and vocabulary sums rounded to fp32, lambda = logit - lse in fp32
-// (lse from fp64 sums), candidate score s_k + lambda in fp32, ties to the lower beam, then the lower word.  stop: the
-// candidates of pcd_decode_beam_stop ranked by key, raw scores beside them, and the loop ends once every row has finished
-static int beam_emu(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                    const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                    const float* b_out, long long* tokens, float* scores, float* work, const pcd_decode_stop* stop) {
-    if (!emb || !w_ih || !w_hh || !b_ih || !b_hh || !h0 || !c0 || !w_out || !b_out || !tokens || !scores || !work) return PCD_ERR_ARG;
-    if (!pcd::decode::beam_ok(B, K, V) || !pcd::decode::shape_ok(T, B * K, H, E, V) || start_token < 0 || start_token >= V)
-        return PCD_ERR_UNSUPPORTED;
-    const int R = B * K;
-    const float alpha = stop ? stop->length_penalty : 0.f;
+// beam decode: lambda = logit - lse in fp32 (lse from fp64 sums), candidate score s_k + lambda in fp32, ties to the lower
+// beam, then the lower word.  stop: finished beams contribute (k, pad_token), candidates are ranked by key with the raw
+// scores beside them, and the loop ends once every row has finished
+static int beam_emu(const pcd_decode_args& a) {
+    const int T = a.T, B = a.B, K = a.K, H = a.H, V = a.V, R = B * K;
+    const float alpha = a.stop ? a.length_penalty : 0.f;
     auto rank_key = [alpha](float sc, int L) { return alpha != 0.f ? sc / powf((float)L, alpha) : sc; };
-    std::vector<float> h((size_t)R * H), c((size_t)R * H), hn((size_t)R * H), cn((size_t)R * H), x((size_t)E), s((size_t)H);
+    std::vector<float> h((size_t)R * H), c((size_t)R * H), hn((size_t)R * H), cn((size_t)R * H);
     std::vector<float> lam((size_t)R * V), score((size_t)R), nscore((size_t)R);
-    std::vector<int> word((size_t)R, start_token), hist_w((size_t)T * R), hist_p((size_t)T * R);
+    std::vector<int> word((size_t)R, a.start_token), hist_w((size_t)T * R), hist_p((size_t)T * R);
     std::vector<int> len((size_t)R, 0), nlen((size_t)R, 0);     // stop: frozen length of a finished beam, 0 while live
     for (int r = 0; r < R; ++r) {
-        std::copy(h0 + (size_t)(r / K) * H, h0 + (size_t)(r / K + 1) * H, h.begin() + (size_t)r * H);
-        std::copy(c0 + (size_t)(r / K) * H, c0 + (size_t)(r / K + 1) * H, c.begin() + (size_t)r * H);
+        std::copy(a.h0 + (size_t)(r / K) * H, a.h0 + (size_t)(r / K + 1) * H, h.begin() + (size_t)r * H);
+        std::copy(a.c0 + (size_t)(r / K) * H, a.c0 + (size_t)(r / K + 1) * H, c.begin() + (size_t)r * H);
         score[r] = r % K ? -INFINITY : 0.f;
     }
     int t_run = T;
     for (int t = 0; t < T; ++t) {
         for (int r = 0; r < R; ++r) {
             if (len[r]) continue;                         // finished: its state is never used again
-            for (int k = 0; k < E; ++k) x[k] = t ? emb[(long long)word[r] * E + k] : tanhf(emb[(long long)word[r] * E + k]);
-            const float* hr = h.data() + (size_t)r * H;
-            for (int j = 0; j < H; ++j) {
-                float g[4];
-                for (int q = 0; q < 4; ++q) {
-                    double acc = (double)b_ih[q * H + j] + b_hh[q * H + j];
-                    for (int k = 0; k < E; ++k) acc += (double)x[k] * w_ih[(long long)(q * H + j) * E + k];
-                    for (int k = 0; k < H; ++k) acc += (double)hr[k] * w_hh[(long long)(q * H + j) * H + k];
-                    g[q] = (float)acc;
-                }
-                const float gi = sigm_(g[0]), gf = sigm_(g[1]), gg = tanhf(g[2]), go = sigm_(g[3]);
-                cn[(size_t)r * H + j] = gf * c[(size_t)r * H + j] + gi * gg;
-                hn[(size_t)r * H + j] = go * tanhf(cn[(size_t)r * H + j]);
-            }
-            for (int j = 0; j < H; ++j) s[j] = tanhf(hn[(size_t)r * H + j]);
             float* lr = lam.data() + (size_t)r * V;
+            step_emu(a, word[r], t, h.data() + (size_t)r * H, c.data() + (size_t)r * H, hn.data() + (size_t)r * H,
+                     cn.data() + (size_t)r * H, lr);
             float mx = -INFINITY;
-            for (int v = 0; v < V; ++v) {
-                double acc = b_out[v];
-                for (int k = 0; k < H; ++k) acc += (double)s[k] * w_out[(long long)v * H + k];
-                lr[v] = (float)acc;
-                mx = lr[v] > mx ? lr[v] : mx;
-            }
+            for (int v = 0; v < V; ++v) mx = lr[v] > mx ? lr[v] : mx;
             double se = 0.0;
             for (int v = 0; v < V; ++v) se += exp((double)lr[v] - mx);
             const float lse = (float)(mx + log(se));
@@ -896,12 +847,12 @@ static int beam_emu(int T, int B, int K, int H, int E, int V, int start_token, c
             for (int k = 0; k < K; ++k) {
                 const int r = b * K + k;
                 if (len[r]) {                             // a finished beam: the one candidate (k, pad_token), score unchanged
-                    insert(rank_key(score[r], len[r]), k * V + stop->pad_token, score[r]);
+                    insert(rank_key(score[r], len[r]), k * V + a.pad_token, score[r]);
                     continue;
                 }
                 for (int v = 0; v < V; ++v) {
                     const float raw = score[r] + lam[(size_t)r * V + v];
-                    insert(stop ? rank_key(raw, t + 1) : raw, k * V + v, raw);
+                    insert(a.stop ? rank_key(raw, t + 1) : raw, k * V + v, raw);
                 }
             }
             for (int j = 0; j < K; ++j) {
@@ -910,7 +861,7 @@ static int beam_emu(int T, int B, int K, int H, int E, int V, int start_token, c
                 hist_p[(size_t)t * R + r] = parent;
                 word[r] = v;
                 nscore[r] = braw[j];
-                nlen[r] = len[parent] ? len[parent] : (stop && v == stop->end_token ? t + 1 : 0);
+                nlen[r] = len[parent] ? len[parent] : (a.stop && v == a.end_token ? t + 1 : 0);
                 std::copy(hn.begin() + (size_t)parent * H, hn.begin() + (size_t)(parent + 1) * H, h.begin() + (size_t)r * H);
                 std::copy(cn.begin() + (size_t)parent * H, cn.begin() + (size_t)(parent + 1) * H, c.begin() + (size_t)r * H);
             }
@@ -922,45 +873,23 @@ static int beam_emu(int T, int B, int K, int H, int E, int V, int start_token, c
     for (int r = 0; r < R; ++r) {
         int cur = r;
         for (int t = t_run - 1; t >= 0; --t) {
-            tokens[(long long)r * T + t] = hist_w[(size_t)t * R + cur];
+            a.tokens[(long long)r * T + t] = hist_w[(size_t)t * R + cur];
             cur = hist_p[(size_t)t * R + cur];
         }
-        for (int t = t_run; t < T; ++t) tokens[(long long)r * T + t] = stop->pad_token;
-        scores[r] = score[r];
+        for (int t = t_run; t < T; ++t) a.tokens[(long long)r * T + t] = a.pad_token;
+        a.scores[r] = score[r];
     }
     return PCD_OK;
 }
 
-extern "C" int pcd_decode_beam(int T, int B, int K, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                               const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                               const float* w_out, const float* b_out, long long* tokens, float* scores, float* work, void*) {
-    return beam_emu(T, B, K, H, E, V, start_token, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, scores, work, nullptr);
-}
+static int run(const pcd_decode_args& a, void*) { return a.mode == kBeam ? beam_emu(a) : decode_emu(a); }
 
-extern "C" int pcd_decode_greedy_stop(int T, int B, int H, int E, int V, int start_token, const float* emb, const float* w_ih,
-                                      const float* w_hh, const float* b_ih, const float* b_hh, const float* h0, const float* c0,
-                                      const float* w_out, const float* b_out, long long* tokens, float* work,
-                                      const pcd_decode_stop* stop, void*) {
-    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    return decode_emu(false, T, B, H, E, V, start_token, 0, 1.f, nullptr, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens,
-                      work, stop);
-}
-
-extern "C" int pcd_decode_sample_stop(int T, int B, int H, int E, int V, int start_token, int row_offset, float temperature,
-                                      const unsigned long long* seed, const float* emb, const float* w_ih, const float* w_hh,
-                                      const float* b_ih, const float* b_hh, const float* h0, const float* c0, const float* w_out,
-                                      const float* b_out, long long* tokens, float* work, const pcd_decode_stop* stop, void*) {
-    if (!pcd::decode::sample_args_ok(temperature, seed, row_offset) || !pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    return decode_emu(true, T, B, H, E, V, start_token, row_offset, temperature, seed, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out,
-                      b_out, tokens, work, stop);
-}
-
-extern "C" int pcd_decode_beam_stop(int T, int B, int K, int H, int E, int V, int start_token, const float* emb,
-                                    const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* h0,
-                                    const float* c0, const float* w_out, const float* b_out, long long* tokens, float* scores,
-                                    float* work, const pcd_decode_stop* stop, void*) {
-    if (!pcd::decode::stop_args_ok(stop, V)) return PCD_ERR_ARG;
-    return beam_emu(T, B, K, H, E, V, start_token, emb, w_ih, w_hh, b_ih, b_hh, h0, c0, w_out, b_out, tokens, scores, work, stop);
-}
+}  // namespace decode
+}  // namespace pcd
 
 #endif
+
+extern "C" int pcd_decode(const pcd_decode_args* a, void* stream) {
+    const int rc = pcd::decode::validate(a);
+    return rc != PCD_OK ? rc : pcd::decode::run(*a, stream);
+}

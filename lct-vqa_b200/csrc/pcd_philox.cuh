@@ -1,4 +1,4 @@
-// pcd_philox.cuh — the Gumbel noise of the sampled question decode (pcd_decode_sample), shared by the sm_100a kernel and
+// pcd_philox.cuh — the Gumbel noise of the sampled question decode (sampled pcd_decode), shared by the sm_100a kernel and
 // the -DPCD_EMU build so that both (and the numpy restatement in tests/sample_oracle.py) draw the same numbers.
 //
 // By the Gumbel-max trick, argmax_v (logit_v / T + G_v) with independent standard Gumbel G_v is distributed as

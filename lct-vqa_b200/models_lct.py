@@ -7,7 +7,7 @@ import torch.nn as nn
 
 import config
 import pcd_ops
-from pcd_ops import decode_beam, decode_greedy, decode_sample, decode_supported, linear_3xtf32, lstm_forward, vocab_cross_entropy
+from pcd_ops import decode_question, linear_3xtf32, lstm_forward, vocab_cross_entropy
 from pcdarts.model_search import Network
 
 
@@ -82,22 +82,10 @@ class QstEncoder(nn.Module):
         differentiable."""
         batch = len(image_embedding)
         h0 = image_embedding.reshape(batch, self.hidden_size)
-        if self.beam_size > 1:       # beam search runs on the decode kernel only: no stock loop outside its envelope
-            if not self.deterministic:
-                raise ValueError(f"beam_size = {self.beam_size} needs deterministic=True (beam search is not sampled)")
-            return decode_beam(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.beam_size,
-                               end_token=self.end_token, length_penalty=self.length_penalty)[0][:, 0].contiguous()
-        # end-of-sequence decoding runs on the decode kernel only: decode_greedy / decode_sample raise outside its envelope
-        stop = self.end_token is not None
-        if self.deterministic and (stop or decode_supported(h0, self.lstm, self.word2vec, self.fc2)):
-            return decode_greedy(h0, self.lstm, self.word2vec, self.fc2, self.max_length,      # one persistent kernel
-                                 end_token=self.end_token)
-        if self.deterministic is False and (stop or decode_supported(h0, self.lstm, self.word2vec, self.fc2)):
-            # the same kernel, words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
-            return decode_sample(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.temperature,
-                                 end_token=self.end_token)
-        if self.deterministic:       # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
-            pcd_ops._stock(f"greedy decode with hidden size {self.hidden_size}")
+        qst = decode_question(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.deterministic, self.temperature,
+                              self.beam_size, self.end_token, self.length_penalty)
+        if qst is not None:
+            return qst
         # sampled decoding outside the kernel's envelope: the reference's module loop (torch.multinomial)
         self.lstm.flatten_parameters()
         h = image_embedding.view(1, -1, self.hidden_size)

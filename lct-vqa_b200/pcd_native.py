@@ -99,8 +99,14 @@ class DropPathArgs(C.Structure):
         [(n, vp) for n in ("seed", "keep", "h1", "h2", "out", "grad_out", "grad_h1", "grad_h2")]
 
 
-class DecodeStop(C.Structure):
-    _fields_ = [("end_token", i32), ("pad_token", i32), ("length_penalty", f32)]
+DECODE_GREEDY, DECODE_SAMPLED, DECODE_BEAM = 0, 1, 2         # pcd_decode_args.mode
+
+
+class DecodeArgs(C.Structure):
+    _fields_ = [(n, i32) for n in ("mode", "T", "B", "K", "H", "E", "V", "start_token", "stop", "end_token", "pad_token")] + \
+        [("length_penalty", f32), ("temperature", f32), ("row_offset", i32)] + \
+        [(n, vp) for n in ("seed", "emb", "w_ih", "w_hh", "b_ih", "b_hh", "h0", "c0", "w_out", "b_out", "tokens", "scores",
+                           "work")]
 
 
 class DwConvArgs(C.Structure):
@@ -130,8 +136,7 @@ EXPORTS = ("pcd_launch_count", "pcd_profile_enable", "pcd_profile_num_kernels", 
            "pcd_preprocess_forward", "pcd_preprocess_backward", "pcd_adaptive_avgpool_forward", "pcd_adaptive_avgpool_backward",
            "pcd_gemm_tn_3xtf32", "pcd_set_overlap", "pcd_overlap_join", "pcd_ce_forward", "pcd_ce_backward",
            "pcd_transpose_pad", "pcd_lstm_pbuf_floats", "pcd_lstm_forward", "pcd_lstm_backward",
-           "pcd_decode_work_floats", "pcd_decode_greedy", "pcd_decode_sample", "pcd_decode_beam_work_floats", "pcd_decode_beam",
-           "pcd_decode_greedy_stop", "pcd_decode_sample_stop", "pcd_decode_beam_stop", "pcd_flat_max_runs", "pcd_flat_axpy", "pcd_flat_scale",
+           "pcd_decode_work_floats", "pcd_decode", "pcd_flat_max_runs", "pcd_flat_axpy", "pcd_flat_scale",
            "pcd_flat_sumsq", "pcd_flat_sumsq_work", "pcd_flat_adam", "pcd_gemm_small_f32",
            "pcd_dwconv_forward", "pcd_dwconv_backward", "pcd_pwconv_forward", "pcd_pwconv_backward", "pcd_bn_apply",
            "pcd_bn_backward_stats", "pcd_pool3x3_forward", "pcd_pool3x3_backward", "pcd_channel_affine",
@@ -170,16 +175,8 @@ def _declare(lib):
     lib.pcd_lstm_forward.argtypes = [C.c_int, C.c_int, C.c_int] + [vp] * 8
     lib.pcd_lstm_backward.argtypes = [C.c_int, C.c_int, C.c_int] + [vp] * 12
     lib.pcd_decode_work_floats.restype = C.c_size_t
-    lib.pcd_decode_work_floats.argtypes = [C.c_int, C.c_int, C.c_int]
-    lib.pcd_decode_greedy.argtypes = [C.c_int] * 6 + [vp] * 12
-    lib.pcd_decode_sample.argtypes = [C.c_int] * 7 + [C.c_float] + [vp] * 13
-    lib.pcd_decode_beam_work_floats.restype = C.c_size_t
-    lib.pcd_decode_beam_work_floats.argtypes = [C.c_int] * 4
-    lib.pcd_decode_beam.argtypes = [C.c_int] * 7 + [vp] * 13
-    stop_p = C.POINTER(DecodeStop)
-    lib.pcd_decode_greedy_stop.argtypes = [C.c_int] * 6 + [vp] * 11 + [stop_p, vp]
-    lib.pcd_decode_sample_stop.argtypes = [C.c_int] * 7 + [C.c_float] + [vp] * 12 + [stop_p, vp]
-    lib.pcd_decode_beam_stop.argtypes = [C.c_int] * 7 + [vp] * 12 + [stop_p, vp]
+    lib.pcd_decode_work_floats.argtypes = [C.POINTER(DecodeArgs)]
+    lib.pcd_decode.argtypes = [C.POINTER(DecodeArgs), vp]
     lib.pcd_transpose_pad.argtypes = [vp, C.c_longlong, C.c_int, C.c_int, vp, C.c_longlong, vp]
     lib.pcd_gemm_tn_3xtf32.argtypes = [vp, C.c_longlong, vp, C.c_longlong, vp, C.c_longlong, C.c_int, C.c_int, C.c_int, vp,
                                        C.c_int, vp]

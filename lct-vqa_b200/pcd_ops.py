@@ -980,7 +980,7 @@ def lstm_forward(lstm, x, h0, c0):
 # Question decode (QstEncoder.generate): one persistent cooperative kernel, greedy, sampled or beam search
 # --------------------------------------------------------------------------------------------
 def decode_supported(h0, lstm, word2vec, proj):
-    """Shapes pcd_decode_greedy / pcd_decode_sample take (single-layer LSTM, hidden a multiple of 32 up to 512, E % 4 == 0;
+    """Shapes pcd_decode takes in greedy and sampled mode (single-layer LSTM, hidden a multiple of 32 up to 512, E % 4 == 0;
     any batch: tiled by 64)."""
     H = lstm.hidden_size
     return (h0.is_cuda or N._emu_lib is not None) and lstm.num_layers == 1 and not lstm.bidirectional and lstm.bias and \
@@ -988,28 +988,9 @@ def decode_supported(h0, lstm, word2vec, proj):
         proj.in_features == H and proj.bias is not None and h0.dtype == torch.float32
 
 
-def _decode_operands(h0, lstm, word2vec, proj, max_length, tokens=True):
-    """(lib, leading int arguments, pointer arguments, tensors behind the pointers, tokens) of one decode launch over at most
-    64 rows.  The caller holds the tensors until the launch is enqueued.  tokens=False: the pointer arguments stop after the
-    parameters (the beam decode has outputs and a workspace of its own)."""
-    lib = N.lib_for(h0)
-    B, H = h0.shape
-    V, E = word2vec.weight.shape
-    h0c = _f32c(h0)
-    ops = [_f32c(t) for t in (word2vec.weight, lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0)]
-    wout, bout = _f32c(proj.weight), _f32c(proj.bias)
-    params = [N.ptr(t) for t in ops] + [N.ptr(h0c), N.ptr(h0c), N.ptr(wout), N.ptr(bout)]
-    if not tokens:
-        return lib, (max_length, B, H, E, V), params, ops + [h0c, wout, bout], None
-    tokens = torch.empty((B, max_length), dtype=torch.long, device=h0.device)
-    work = torch.empty(int(lib.pcd_decode_work_floats(B, H, V)), dtype=torch.float32, device=h0.device)
-    ptrs = params + [N.ptr(tokens), N.ptr(work), N.stream_for(h0)]
-    return lib, (max_length, B, H, E, V), ptrs, ops + [h0c, wout, bout, work], tokens
-
-
 def _decode_stop(V, end_token, pad_token, length_penalty=0.0):
-    """The pcd_decode_stop of an end-of-sequence decode (None for end_token=None: the call without _stop).  ValueError for an
-    end or pad word outside [0, V) or a length penalty that is not finite."""
+    """(end_token, pad_token, length_penalty as fp32) of an end-of-sequence decode (None for end_token=None: no stop).
+    ValueError for an end or pad word outside [0, V) or a length penalty that is not finite."""
     if end_token is None:                               # every hypothesis has max_length words: length_penalty is not used
         return None
     a32 = C.c_float(float(length_penalty)).value        # what the kernel divides by
@@ -1018,7 +999,7 @@ def _decode_stop(V, end_token, pad_token, length_penalty=0.0):
     for name, w in (("end_token", end_token), ("pad_token", pad_token)):
         if isinstance(w, bool) or int(w) != w or not 0 <= w < V:
             raise ValueError(f"decode: {name} must be an integer in [0, vocabulary size {V}), got {w}")
-    return N.DecodeStop(int(end_token), int(pad_token), a32)
+    return int(end_token), int(pad_token), a32
 
 
 def _check_envelope(what, h0, lstm, word2vec, proj):
@@ -1028,35 +1009,58 @@ def _check_envelope(what, h0, lstm, word2vec, proj):
                            f"{word2vec.embedding_dim} is outside the decode kernel's envelope (PCD_ERR_UNSUPPORTED)")
 
 
+def _decode(mode, h0, lstm, word2vec, proj, max_length, start_token, K=1, temperature=1.0, seed=None, stop=None):
+    """One pcd_decode per slice of floor(64 / K) items (the kernel takes 64 rows; row_offset = the slice's first item), each
+    with its own outputs and workspace.  Returns (tokens, scores): tokens (B, max_length) and scores None, or for beams
+    tokens (B, K, max_length) and scores (B, K).  The arguments are validated by the caller; stop: _decode_stop's tuple."""
+    lib = N.lib_for(h0)
+    V, E = word2vec.weight.shape
+    beam = mode == N.DECODE_BEAM
+    ops = [_f32c(t) for t in (word2vec.weight, lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0)]
+    wout, bout = _f32c(proj.weight), _f32c(proj.bias)
+    end_token, pad_token, length_penalty = stop or (0, 0, 0.0)
+    per = _LSTM_BATCH // K
+    tokens, scores = [], []
+    for b0 in range(0, max(h0.shape[0], 1), per):       # an empty batch reaches the kernel, which rejects it
+        h0c = _f32c(h0[b0:b0 + per])
+        B, H = h0c.shape
+        tok = torch.empty((B, K, max_length) if beam else (B, max_length), dtype=torch.long, device=h0.device)
+        sc = torch.empty((B, K), dtype=torch.float32, device=h0.device) if beam else None
+        a = N.DecodeArgs(mode=mode, T=max_length, B=B, K=K, H=H, E=E, V=V, start_token=start_token, stop=stop is not None,
+                         end_token=end_token, pad_token=pad_token, length_penalty=length_penalty, temperature=temperature,
+                         row_offset=b0, seed=N.ptr(seed), emb=N.ptr(ops[0]), w_ih=N.ptr(ops[1]), w_hh=N.ptr(ops[2]),
+                         b_ih=N.ptr(ops[3]), b_hh=N.ptr(ops[4]), h0=N.ptr(h0c), c0=N.ptr(h0c), w_out=N.ptr(wout),
+                         b_out=N.ptr(bout), tokens=N.ptr(tok), scores=N.ptr(sc))
+        work = torch.empty(int(lib.pcd_decode_work_floats(C.byref(a))), dtype=torch.float32, device=h0.device)
+        a.work = N.ptr(work)
+        N.check(lib, lib.pcd_decode(C.byref(a), N.stream_for(h0)), "pcd_decode")
+        tokens.append(tok)
+        scores.append(sc)
+    if len(tokens) == 1:
+        return tokens[0], scores[0]
+    return torch.cat(tokens, 0), (torch.cat(scores, 0) if beam else None)
+
+
 def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2, end_token=None, pad_token=0):
     """tokens (B, max_length) int64 of the greedy decode that starts from `start_token` with h0 = c0 = `h0` (B, H).
-    end_token: once a row has emitted it, its later positions are `pad_token` (pcd_decode_greedy_stop): the unstopped decode
-    truncated after the first end_token, and the kernel stops when every row of a launch has finished.
+    end_token: once a row has emitted it, its later positions are `pad_token`: the unstopped decode truncated after the
+    first end_token, and the kernel stops when every row of a launch has finished.
     Not differentiable (neither is the reference's argmax): parameters are read detached."""
     stop = _decode_stop(proj.out_features, end_token, pad_token)
     if stop is not None:
         _check_envelope("decode_greedy", h0, lstm, word2vec, proj)
-    if h0.shape[0] > _LSTM_BATCH:          # independent rows: ceil(B / 64) launches of the persistent kernel
-        return torch.cat([decode_greedy(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length, start_token, end_token,
-                                        pad_token) for b0 in range(0, h0.shape[0], _LSTM_BATCH)], 0)
-    lib, dims, ptrs, _keep, tokens = _decode_operands(h0, lstm, word2vec, proj, max_length)
-    if stop is None:
-        N.check(lib, lib.pcd_decode_greedy(*dims, start_token, *ptrs), "pcd_decode_greedy")
-    else:
-        N.check(lib, lib.pcd_decode_greedy_stop(*dims, start_token, *ptrs[:-1], C.byref(stop), ptrs[-1]),
-                "pcd_decode_greedy_stop")
-    return tokens
+    return _decode(N.DECODE_GREEDY, h0, lstm, word2vec, proj, max_length, start_token, stop=stop)[0]
 
 
 def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None, end_token=None, pad_token=0):
     """tokens (B, max_length) int64 of the sampled decode (QstEncoder.sample with deterministic=False): every word is drawn from
-    softmax(logits / temperature), by the Gumbel-max trick on counter-based Philox noise (pcd_decode_sample).
+    softmax(logits / temperature), by the Gumbel-max trick on counter-based Philox noise (pcd_decode in sampled mode).
 
     seed: None draws one 64-bit seed per call on h0's device from torch's generator (so torch.manual_seed reproduces a run, and
     a call captured in a CUDA graph draws a fresh seed on every replay); a Python int, or a 1-element int64 tensor on h0's
     device read when the kernel runs, fixes the words.  Batches above 64 are decoded in slices of 64 with one seed: the noise
     of a row depends on its index in the whole batch, so the words do not depend on the slicing.  end_token / pad_token as
-    decode_greedy (pcd_decode_sample_stop): the same words up to the first end_token.  Not differentiable."""
+    decode_greedy: the same words up to the first end_token.  Not differentiable."""
     t32 = C.c_float(float(temperature)).value           # what the kernel divides by
     if not math.isfinite(t32) or t32 <= 0.0:
         raise ValueError(f"decode_sample: temperature must be finite and > 0, got {temperature}")
@@ -1070,16 +1074,8 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
         seed = torch.tensor([s - 2 ** 64 if s >= 2 ** 63 else s], dtype=torch.int64, device=h0.device)
     elif seed.dtype != torch.int64 or seed.numel() != 1 or seed.device != h0.device:
         raise ValueError("decode_sample: seed must be an int or a 1-element int64 tensor on the device of h0")
-    out = []
-    for b0 in range(0, h0.shape[0], _LSTM_BATCH):
-        lib, dims, ptrs, _keep, tokens = _decode_operands(h0[b0:b0 + _LSTM_BATCH], lstm, word2vec, proj, max_length)
-        if stop is None:
-            N.check(lib, lib.pcd_decode_sample(*dims, start_token, b0, t32, N.ptr(seed), *ptrs), "pcd_decode_sample")
-        else:
-            N.check(lib, lib.pcd_decode_sample_stop(*dims, start_token, b0, t32, N.ptr(seed), *ptrs[:-1], C.byref(stop),
-                                                    ptrs[-1]), "pcd_decode_sample_stop")
-        out.append(tokens)
-    return out[0] if len(out) == 1 else torch.cat(out, 0)
+    return _decode(N.DECODE_SAMPLED, h0, lstm, word2vec, proj, max_length, start_token, temperature=t32, seed=seed,
+                   stop=stop)[0]
 
 
 _MAX_BEAM = 8
@@ -1087,37 +1083,43 @@ _MAX_BEAM = 8
 
 def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2, end_token=None, pad_token=0,
                 length_penalty=0.0):
-    """Beam search over exactly `max_length` words from `start_token` with h0 = c0 = `h0` (B, H) (pcd_decode_beam): at every
-    step each item keeps the `beam_size` = K paths of highest cumulative log-probability.  Returns (tokens (B, K, max_length)
-    int64, scores (B, K) float32), beams best first; beam_size = 1 is the greedy decode scored by its log-probability.
-    end_token (pcd_decode_beam_stop): a beam whose last word is end_token is finished and continues with `pad_token` at no
-    cost; beams are ranked by score / length^length_penalty (length counting end_token), scores are the log-probabilities of
-    the paths up to end_token, and the kernel stops once every beam of a launch has finished.  Without end_token every
-    hypothesis has max_length words and length_penalty is not used.
+    """Beam search over exactly `max_length` words from `start_token` with h0 = c0 = `h0` (B, H) (pcd_decode in beam mode): at
+    every step each item keeps the `beam_size` = K paths of highest cumulative log-probability.  Returns (tokens (B, K,
+    max_length) int64, scores (B, K) float32), beams best first; beam_size = 1 is the greedy decode scored by its
+    log-probability.
+    end_token: a beam whose last word is end_token is finished and continues with `pad_token` at no cost; beams are ranked
+    by score / length^length_penalty (length counting end_token), scores are the log-probabilities of the paths up to
+    end_token, and the kernel stops once every beam of a launch has finished.  Without end_token every hypothesis has
+    max_length words and length_penalty is not used.
     Batches are decoded in slices of floor(64 / K) items (the kernel takes 64 rows); items are independent, so the result does
     not depend on the slicing.  Not differentiable: parameters are read detached."""
     V = proj.out_features
     if isinstance(beam_size, bool) or int(beam_size) != beam_size or not 1 <= beam_size <= _MAX_BEAM or beam_size > V:
         raise ValueError(f"decode_beam: beam_size must be an integer in [1, min({_MAX_BEAM}, vocabulary size {V})], "
                          f"got {beam_size}")
-    K = int(beam_size)
     stop = _decode_stop(V, end_token, pad_token, length_penalty)
     _check_envelope("decode_beam", h0, lstm, word2vec, proj)
-    per = _LSTM_BATCH // K
-    tokens, scores = [], []
-    for b0 in range(0, h0.shape[0], per):
-        lib, dims, ptrs, _keep, _ = _decode_operands(h0[b0:b0 + per], lstm, word2vec, proj, max_length, tokens=False)
-        T, B, H, E, V = dims
-        tok = torch.empty((B, K, T), dtype=torch.long, device=h0.device)
-        sc = torch.empty((B, K), dtype=torch.float32, device=h0.device)
-        work = torch.empty(int(lib.pcd_decode_beam_work_floats(B, K, H, V)), dtype=torch.float32, device=h0.device)
-        if stop is None:
-            N.check(lib, lib.pcd_decode_beam(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
-                                             N.stream_for(h0)), "pcd_decode_beam")
-        else:
-            N.check(lib, lib.pcd_decode_beam_stop(T, B, K, H, E, V, start_token, *ptrs, N.ptr(tok), N.ptr(sc), N.ptr(work),
-                                                  C.byref(stop), N.stream_for(h0)), "pcd_decode_beam_stop")
-        tokens.append(tok); scores.append(sc)
-    if len(tokens) == 1:
-        return tokens[0], scores[0]
-    return torch.cat(tokens, 0), torch.cat(scores, 0)
+    return _decode(N.DECODE_BEAM, h0, lstm, word2vec, proj, max_length, start_token, K=int(beam_size), stop=stop)
+
+
+def decode_question(h0, lstm, word2vec, proj, max_length, deterministic, temperature, beam_size, end_token, length_penalty):
+    """QstEncoder.generate's decode policy: tokens (B, max_length) of the best beam (beam_size > 1), of the greedy decode
+    (`deterministic` truthy) or of the sampled one (`deterministic is False`), all on the decode kernel.  None when the
+    caller's stock loop decodes: sampled decoding outside the kernel's envelope, any other falsy `deterministic` (an
+    overridden sample()), and greedy decoding outside the envelope once allow_stock_ops(True) lets it.  Beam search and
+    end-of-sequence decoding have no stock loop: outside the envelope they raise, even with allow_stock_ops(True)."""
+    if beam_size > 1:
+        if not deterministic:
+            raise ValueError(f"beam_size = {beam_size} needs deterministic=True (beam search is not sampled)")
+        return decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, end_token=end_token,
+                           length_penalty=length_penalty)[0][:, 0].contiguous()
+    # end-of-sequence decoding: decode_greedy / decode_sample raise outside the envelope
+    stop = end_token is not None
+    if deterministic and (stop or decode_supported(h0, lstm, word2vec, proj)):
+        return decode_greedy(h0, lstm, word2vec, proj, max_length, end_token=end_token)
+    if deterministic is False and (stop or decode_supported(h0, lstm, word2vec, proj)):
+        # words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
+        return decode_sample(h0, lstm, word2vec, proj, max_length, temperature, end_token=end_token)
+    if deterministic:            # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
+        _stock(f"greedy decode with hidden size {h0.shape[1]}")
+    return None

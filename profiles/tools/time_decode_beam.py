@@ -4,7 +4,7 @@ the greedy kernel and a stock-torch beam loop, all in one run on one GPU.  Print
     python profiles/tools/time_decode_beam.py [--calls N] [--out profiles/decode_beam.json]
 
 Arms:
-  greedy_kernel   pcd_decode_greedy (QstEncoder.generate with beam_size = 1): one persistent cooperative launch
+  greedy_kernel   pcd_decode in greedy mode (QstEncoder.generate with beam_size = 1): one persistent cooperative launch
   beam_kernel_K   pcd_ops.decode_beam(..., K): ceil(64 K / 64) launches of the persistent kernel in beam mode
   stock_beam_K    the loop a user would write without the kernel: per word an nn.LSTM step, Linear(H, V) over B K rows,
                   log_softmax, topk over K V candidates per item and a gather of the parents' states; TF32 off
@@ -36,7 +36,7 @@ def card():
 
 @torch.no_grad()
 def stock_beam(q, img, K, T, start_token=2):
-    """(tokens (B, K, T), scores (B, K)) by stock torch ops, the semantics of pcd_decode_beam."""
+    """(tokens (B, K, T), scores (B, K)) by stock torch ops, the semantics of pcd_decode in beam mode."""
     B, H = img.shape
     V = q.fc1.out_features
     R = B * K

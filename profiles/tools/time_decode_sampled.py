@@ -4,8 +4,8 @@ run on one GPU.  Prints one JSON line.
     python profiles/tools/time_decode_sampled.py [--calls N] [--out file.json]
 
 Arms:
-  greedy_kernel   deterministic=True: pcd_decode_greedy, one persistent cooperative launch
-  sampled_kernel  deterministic=False: pcd_decode_sample (the same kernel, Gumbel-max on Philox noise) + the seed draw
+  greedy_kernel   deterministic=True: pcd_decode in greedy mode, one persistent cooperative launch
+  sampled_kernel  deterministic=False: pcd_decode in sampled mode (the same kernel, Gumbel-max on Philox noise) + the seed draw
   stock_sampled   deterministic=None: the reference's module loop (nn.LSTM step, Linear, softmax, torch.multinomial per word),
                   which is what deterministic=False ran before the sampled kernel existed
 Timing: CUDA events around blocks of back-to-back calls, the arms alternating block by block, after warm-up; per-call time

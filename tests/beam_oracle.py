@@ -1,4 +1,5 @@
-"""float64 beam search of the question decoder, written from the semantics of pcd_decode_beam (include/pcdarts_sm100.h).
+"""float64 beam search of the question decoder, written from the semantics of pcd_decode in beam mode
+(include/pcdarts_sm100.h).
 
 Items b, beams k, rows r = b*K + k, exactly T words.  Every row of item b starts from h = c = h0[b] with input
 tanh(emb[start]); beam scores start at (0, -inf, ..., -inf).  Per step and row: one LSTM step, logits

@@ -508,7 +508,7 @@ def architect_lct_case(device):
 
 
 def decode_case(device, B, H, E, V, T, seed=3):
-    """pcd_decode_greedy vs the reference's own loop (vqa_model.py:103-136) in fp64, teacher-forced with the kernel's words so
+    """Greedy pcd_decode vs the reference's own loop (vqa_model.py:103-136) in fp64, teacher-forced with the kernel's words so
     that one rounding-level tie cannot desynchronise the rest: every chosen word must be an argmax of the fp64 logits up to
     fp32 rounding, and (ties being measure-zero) essentially all of them must be THE argmax."""
     from pcd_ops import decode_greedy, decode_supported

@@ -1,4 +1,4 @@
-"""numpy restatement of the sampled question decode (pcd_decode_sample; the noise is lct-vqa_b200/csrc/pcd_philox.cuh).
+"""numpy restatement of the sampled question decode (pcd_decode in sampled mode; the noise is lct-vqa_b200/csrc/pcd_philox.cuh).
 
 By the Gumbel-max trick the kernel draws word t of row b as argmax_v (logit_v / T + G(seed, t, row, v)), which is distributed
 as softmax(logit / T), the distribution QstEncoder.sample draws from with torch.multinomial.  G is a pure function of

@@ -1,5 +1,5 @@
-"""float64 end-of-sequence beam search of the question decoder, written from the semantics of pcd_decode_beam_stop
-(include/pcdarts_sm100.h), on the LSTM step of beam_oracle.py.
+"""float64 end-of-sequence beam search of the question decoder, written from the semantics of pcd_decode in beam
+mode with the stop (include/pcdarts_sm100.h), on the LSTM step of beam_oracle.py.
 
 A beam is finished once its last word is `end`.  A live beam k contributes the candidates (k, v) for every v with raw score
 s_k + lambda_k[v]; a finished beam contributes only (k, pad) with its raw score unchanged.  Candidates are ranked by the key

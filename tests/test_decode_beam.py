@@ -1,5 +1,5 @@
-"""Beam-search question decode (pcd_decode_beam, pcd_ops.decode_beam, QstEncoder(beam_size=K)) against the float64 beam search
-of beam_oracle.py.  CPU cases run the kernel source's -DPCD_EMU build; `gpu` cases run the sm_100a kernel.
+"""Beam-search question decode (pcd_decode in beam mode, pcd_ops.decode_beam, QstEncoder(beam_size=K)) against the float64
+beam search of beam_oracle.py.  CPU cases run the kernel source's -DPCD_EMU build; `gpu` cases run the sm_100a kernel.
 
 Comparison rule.  fp32 can reorder near-ties, so the search is compared margin-aware.  TAU bounds the fp32 error one step adds
 to a cumulative beam score: the score is a running fp32 sum of lambda = logit - lse with |score| < 512 over 30 words, so its
@@ -11,11 +11,14 @@ t + 1 steps two candidate scores can each be off by (t + 1) TAU, so
   - otherwise the kernel's best beam, re-scored in float64, must be no worse than T TAU below the oracle's best.
 Independently of the search, every returned score must equal the float64 teacher-forced log-probability of its sequence
 within T TAU."""
+import ctypes
+
 import pytest
 import torch
 
 import beam_oracle as BO
 import parity_cases as P
+from pcd_native import DECODE_BEAM, DECODE_GREEDY, DECODE_SAMPLED, DecodeArgs
 
 TAU = 5e-5
 
@@ -79,15 +82,27 @@ def beam_case(device, B, K, H, E, V, T, seed=3, items=None):
     return check_beams(tokens, scores, (emb, lstm, proj), h0, T, K, items), (tokens, scores, mods, h0)
 
 
-class _Counting:
-    """Stands in for one ctypes function of the loaded library: counts the calls and forwards them."""
+class _Decodes:
+    """Stands in for lib.pcd_decode: records (mode, stop, K) of every call from the pcd_decode_args passed by reference, and
+    forwards the call."""
 
     def __init__(self, fn):
-        self.fn, self.calls = fn, 0
+        self.fn, self.seen = fn, []
 
-    def __call__(self, *args):
-        self.calls += 1
-        return self.fn(*args)
+    def __call__(self, args, stream):
+        a = args._obj
+        self.seen.append((a.mode, a.stop, a.K))
+        return self.fn(args, stream)
+
+    def count(self, mode, stop=0):
+        """the calls in `mode` without (stop=0) or with (stop=1) end-of-sequence decoding"""
+        return sum(m == mode and s == stop for m, s, _ in self.seen)
+
+
+def _decode_args(ptrs, **fields):
+    """pcd_decode_args with the nine parameter pointers `ptrs` (emb .. b_out) and `fields`."""
+    names = ("emb", "w_ih", "w_hh", "b_ih", "b_hh", "h0", "c0", "w_out", "b_out")
+    return DecodeArgs(**dict(zip(names, ptrs)), **fields)
 
 
 # ---- CPU: the emulated kernel source ---------------------------------------------------------------------------------
@@ -126,26 +141,27 @@ def test_batch_slicing_does_not_change_the_result(emulation):
         assert torch.equal(t1[0], tokens[b]) and torch.equal(s1[0], scores[b])
 
 
-def test_generate_routes_beam_search_to_the_kernel(emulation, monkeypatch):
-    """beam_size = 1 never reaches pcd_decode_beam; beam_size > 1 does (both packages) and returns beam 0 as (B, T)."""
+def test_generate_routes_beam_search_to_the_beam_mode(emulation, monkeypatch):
+    """beam_size = 1 never reaches the beam mode of pcd_decode; beam_size > 1 does (both packages) and returns beam 0 as
+    (B, T)."""
     import models_lct
     import pcd_ops
     import vqa_model
     lib = emulation
-    beam, greedy = _Counting(lib.pcd_decode_beam), _Counting(lib.pcd_decode_greedy)
-    monkeypatch.setattr(lib, "pcd_decode_beam", beam)
-    monkeypatch.setattr(lib, "pcd_decode_greedy", greedy)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
+    beam, greedy = lambda: rec.count(DECODE_BEAM), lambda: rec.count(DECODE_GREEDY)
     torch.manual_seed(3)
     img = 0.3 * torch.randn(3, 32)
     for mod in (vqa_model, models_lct):
         q = mod.QstEncoder(90, 8, 32, 1, 32, max_length=5)
         assert q.beam_size == 1
-        n, g = beam.calls, greedy.calls
+        n, g = beam(), greedy()
         q.generate(img)
-        assert beam.calls == n and greedy.calls == g + 1
+        assert beam() == n and greedy() == g + 1 and rec.seen[-1] == (DECODE_GREEDY, 0, 1)
         q.beam_size = 3
         words = q.generate(img)
-        assert beam.calls == n + 1 and greedy.calls == g + 1
+        assert beam() == n + 1 and greedy() == g + 1 and rec.seen[-1] == (DECODE_BEAM, 0, 3)
         proj = q.fc1 if mod is vqa_model else q.fc2
         tokens, _ = pcd_ops.decode_beam(img, q.lstm, q.word2vec, proj, 5, 3)
         assert words.shape == (3, 5) and words.dtype == torch.long and torch.equal(words, tokens[:, 0])
@@ -163,7 +179,7 @@ def test_generate_routes_beam_search_to_the_kernel(emulation, monkeypatch):
         pcd_ops.allow_stock_ops(prev)
 
 
-def test_bad_arguments(emulation):
+def test_bad_beam_arguments(emulation):
     from pcd_ops import decode_beam
     emb, lstm, proj, h0 = _modules(2, 32, 8, 6)
     for bad in (0, -1, 9, 7, 2.5, True):                           # 7 > V = 6
@@ -174,20 +190,29 @@ def test_bad_arguments(emulation):
     ptrs = [t.detach().data_ptr() for t in ops]
     tokens = torch.empty(64 * 3, dtype=torch.long)
     scores = torch.empty(64)
-    work = torch.empty(int(lib.pcd_decode_beam_work_floats(8, 8, 32, 6)))
+    work = torch.empty(int(lib.pcd_decode_work_floats(ctypes.byref(DecodeArgs(mode=DECODE_BEAM, B=8, K=8, H=32, V=6)))))
 
-    def call(B=2, K=2, V=6, T=3, start=2, ptrs=ptrs, out=(tokens.data_ptr(), scores.data_ptr(), work.data_ptr())):
-        return lib.pcd_decode_beam(T, B, K, 32, 8, V, start, *ptrs, *out, None)
+    def call(B=2, K=2, V=6, T=3, start=2, ptrs=ptrs, out=(tokens.data_ptr(), scores.data_ptr(), work.data_ptr()),
+             mode=DECODE_BEAM):
+        a = _decode_args(ptrs, mode=mode, T=T, B=B, K=K, H=32, E=8, V=V, start_token=start, tokens=out[0], scores=out[1],
+                         work=out[2])
+        return lib.pcd_decode(ctypes.byref(a), None)
 
     assert call() == 0
     for kw in (dict(K=0), dict(K=9), dict(K=7), dict(B=9, K=8), dict(B=33, K=2), dict(B=0), dict(T=0), dict(start=6)):
         assert call(**kw) == -2, kw                  # PCD_ERR_UNSUPPORTED
     for i in range(len(ptrs)):
         assert call(ptrs=ptrs[:i] + [None] + ptrs[i + 1:]) == -1, i         # PCD_ERR_ARG
+        assert call(ptrs=ptrs[:i] + [None] + ptrs[i + 1:], K=9) == -1, i    # before the envelope check
     for i in range(3):
         out = [tokens.data_ptr(), scores.data_ptr(), work.data_ptr()]
         out[i] = None
         assert call(out=tuple(out)) == -1, i
+        assert call(out=tuple(out), K=9) == -1, i
+    for mode in (-1, 3):
+        assert call(mode=mode) == -1, mode           # not a mode
+    for mode in (DECODE_GREEDY, DECODE_SAMPLED):
+        assert call(mode=mode, B=2, K=2) == -1, mode     # K != 1 outside beam mode
 
 
 def test_unrolled_twin_keeps_the_beam_width():
@@ -240,7 +265,7 @@ def test_beam_decode_is_deterministic():
 
 @pytest.mark.gpu
 def test_beam_width_one_against_the_greedy_kernel():
-    """K = 1 runs the same fp32 logits as pcd_decode_greedy; the words agree wherever the oracle's top-2 gap exceeds rounding."""
+    """K = 1 runs the same fp32 logits as the greedy decode; the words agree wherever the oracle's top-2 gap exceeds rounding."""
     from pcd_ops import decode_beam, decode_greedy
     B, T = 64, PROD["T"]
     emb, lstm, proj, h0 = _modules(B, PROD["H"], PROD["E"], PROD["V"], seed=14)
@@ -255,7 +280,7 @@ def test_beam_width_one_against_the_greedy_kernel():
 
 
 @pytest.mark.gpu
-def test_misaligned_operand_is_rejected():
+def test_misaligned_decode_operand_is_rejected():
     import pcd_native
     lib = pcd_native.load_cuda()
     emb, lstm, proj, h0 = _modules(2, 32, 8, 40)
@@ -263,11 +288,13 @@ def test_misaligned_operand_is_rejected():
                                                          lstm.bias_hh_l0, h0, h0, proj.weight, proj.bias)]
     tokens = torch.empty(2 * 2 * 3, dtype=torch.long, device="cuda")
     scores = torch.empty(4, device="cuda")
-    work = torch.empty(int(lib.pcd_decode_beam_work_floats(2, 2, 32, 40)) + 4, device="cuda")
-    ptrs = [t.data_ptr() for t in ops]
-    assert lib.pcd_decode_beam(3, 2, 2, 32, 8, 40, 2, *ptrs, tokens.data_ptr(), scores.data_ptr(), work.data_ptr() + 4,
-                               None) == -4          # PCD_ERR_ALIGN: nothing launched
-    assert lib.pcd_decode_beam(3, 2, 2, 32, 8, 40, 2, *ptrs, tokens.data_ptr(), scores.data_ptr(), work.data_ptr(), None) == 0
+    a = _decode_args([t.data_ptr() for t in ops], mode=DECODE_BEAM, T=3, B=2, K=2, H=32, E=8, V=40, start_token=2,
+                     tokens=tokens.data_ptr(), scores=scores.data_ptr())
+    work = torch.empty(int(lib.pcd_decode_work_floats(ctypes.byref(a))) + 4, device="cuda")
+    a.work = work.data_ptr() + 4
+    assert lib.pcd_decode(ctypes.byref(a), None) == -4          # PCD_ERR_ALIGN: nothing launched
+    a.work = work.data_ptr()
+    assert lib.pcd_decode(ctypes.byref(a), None) == 0
     torch.cuda.synchronize()
 
 
@@ -296,9 +323,10 @@ def test_beam_generate_in_a_cuda_graph():
 
 
 @pytest.mark.gpu
-def test_graphed_lct_step_with_beam_search(monkeypatch):
+def test_graphed_lct_step_decodes_in_beam_mode(monkeypatch):
     """search.GraphedLctStep with beam_size = 4 on the EF model (and so on its unrolled twin): the three generate() calls of
-    ArchitectLct.step run on pcd_decode_beam, the replays give finite losses and the first replay equals the eager step."""
+    ArchitectLct.step run on the beam mode of pcd_decode, the replays give finite losses and the first replay equals the
+    eager step."""
     import math
     import config
     import pcd_native
@@ -315,12 +343,11 @@ def test_graphed_lct_step_with_beam_search(monkeypatch):
         config.ARCH_LEARNING_RATE, config.ARCH_WEIGHT_DECAY = lr0, wd0
     ef1.qst_encoder.beam_size = ef2.qst_encoder.beam_size = 4
     lib = pcd_native.load_cuda()
-    beam, greedy = _Counting(lib.pcd_decode_beam), _Counting(lib.pcd_decode_greedy)
-    monkeypatch.setattr(lib, "pcd_decode_beam", beam)
-    monkeypatch.setattr(lib, "pcd_decode_greedy", greedy)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
     tr, va = P.lct_batch(21, "cuda"), P.lct_batch(22, "cuda")
     graphed = GraphedLctStep(arch2, tr, va, 1e-3, 1e-3, warmup=2)
-    assert beam.calls == 3 * 3 and greedy.calls == 0           # two warm-up steps + the captured step
+    assert rec.count(DECODE_BEAM) == 3 * 3 and rec.count(DECODE_GREEDY) == 0       # two warm-up steps + the captured step
     for _ in range(2):
         eager.step(*tr, *va, 1e-3, 1e-3)
     eager.step(*tr, *va, 1e-3, 1e-3)

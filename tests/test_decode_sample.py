@@ -1,6 +1,7 @@
 """Sampled question decode (QstEncoder.generate with deterministic=False) on the persistent decode kernel: Gumbel-max over
-Philox noise (pcd_decode_sample) against the float64 restatement in sample_oracle.py.  CPU cases run the kernel source's
--DPCD_EMU build; `gpu` cases run the sm_100a kernel."""
+Philox noise (pcd_decode in sampled mode) against the float64 restatement in sample_oracle.py.  CPU cases run the kernel
+source's -DPCD_EMU build; `gpu` cases run the sm_100a kernel."""
+import ctypes
 import math
 
 import numpy as np
@@ -9,6 +10,8 @@ import torch
 
 import parity_cases as P
 import sample_oracle as S
+from pcd_native import DECODE_GREEDY, DECODE_SAMPLED, DecodeArgs
+from test_decode_beam import _Decodes, _decode_args
 
 SEED = 0x0123456789ABCDEF         # both key words non-zero
 
@@ -69,17 +72,6 @@ def sample_case(device, B, H, E, V, T, temperature, seed=SEED):
     return check_against_oracle(tokens, (emb, lstm, proj), h0, T, temperature, seed)
 
 
-class _Counting:
-    """Stands in for one ctypes function of the loaded library: counts the calls and forwards them."""
-
-    def __init__(self, fn):
-        self.fn, self.calls = fn, 0
-
-    def __call__(self, *args):
-        self.calls += 1
-        return self.fn(*args)
-
-
 # ---- CPU: the oracle's noise ----------------------------------------------------------------------------------------
 @pytest.mark.parametrize("counter,key,expect", [
     ((0, 0, 0, 0), (0, 0), (0x6627E8D5, 0xE169C58D, 0xBC57AC4C, 0x9B00DBD8)),
@@ -120,30 +112,31 @@ def test_seed_fixes_the_words(emulation):
     assert torch.equal(b, decode_sample(h0, lstm, emb, proj, 6, 1.0))       # seed=None: torch's generator
 
 
-def test_generate_routes_sampling_to_the_kernel(emulation, monkeypatch):
-    """deterministic=False inside the envelope goes through pcd_decode_sample (both packages); deterministic=None with an
-    overridden sample() (the stock-loop reference arm of the timing tools and GPU tests) and H outside the envelope do not."""
+def test_generate_routes_sampling_to_the_sampled_mode(emulation, monkeypatch):
+    """deterministic=False inside the envelope goes through the sampled mode of pcd_decode (both packages); deterministic=None
+    with an overridden sample() (the stock-loop reference arm of the timing tools and GPU tests) and H outside the envelope
+    do not."""
     import models_lct
     import vqa_model
     lib = emulation
-    sample, greedy = _Counting(lib.pcd_decode_sample), _Counting(lib.pcd_decode_greedy)
-    monkeypatch.setattr(lib, "pcd_decode_sample", sample)
-    monkeypatch.setattr(lib, "pcd_decode_greedy", greedy)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
+    sample, greedy = lambda: rec.count(DECODE_SAMPLED), lambda: rec.count(DECODE_GREEDY)
     torch.manual_seed(3)
     img = 0.3 * torch.randn(3, 32)
     for mod in (vqa_model, models_lct):
         q = mod.QstEncoder(90, 8, 32, 1, 32, deterministic=False, temperature=0.5, max_length=5)
-        n = sample.calls
+        n = sample()
         words = q.generate(img)
-        assert sample.calls == n + 1 and greedy.calls == 0
+        assert sample() == n + 1 and greedy() == 0
         assert words.shape == (3, 5) and words.dtype == torch.long and 0 <= int(words.min()) and int(words.max()) < 90
         q.deterministic = None
         q.sample = lambda prob: torch.argmax(prob, 2)
         assert q.generate(img).shape == (3, 5)
-        assert sample.calls == n + 1 and greedy.calls == 0
+        assert sample() == n + 1 and greedy() == 0
     q48 = vqa_model.QstEncoder(90, 8, 48, 1, 48, deterministic=False, max_length=4)     # H = 48: stock loop, no raise
     assert q48.generate(0.3 * torch.randn(2, 48)).shape == (2, 4)
-    assert sample.calls == 2
+    assert sample() == 2
 
 
 def test_sampled_generate_matches_the_oracle_with_the_drawn_seed(emulation):
@@ -159,7 +152,7 @@ def test_sampled_generate_matches_the_oracle_with_the_drawn_seed(emulation):
     check_against_oracle(words, (q.word2vec, q.lstm, q.fc1), img, 4, 0.7, seed)
 
 
-def test_bad_temperature_and_arguments(emulation):
+def test_bad_temperature_and_decode_args(emulation):
     from pcd_ops import decode_sample
     emb, lstm, proj, h0 = _modules(2, 32, 8, 40)
     for bad in (0.0, -1.0, float("nan"), float("inf"), 1e-50):
@@ -170,16 +163,19 @@ def test_bad_temperature_and_arguments(emulation):
     ops = [emb.weight, lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0, h0, h0, proj.weight, proj.bias]
     ptrs = [t.detach().data_ptr() for t in ops]
     tokens = torch.empty(2, 3, dtype=torch.long)
-    work = torch.empty(int(lib.pcd_decode_work_floats(2, 32, 40)))
+    work = torch.empty(int(lib.pcd_decode_work_floats(ctypes.byref(DecodeArgs(mode=DECODE_SAMPLED, B=2, K=1, H=32, V=40)))))
 
-    def call(row_offset=0, temperature=1.0, seed_ptr=seed.data_ptr()):
-        return lib.pcd_decode_sample(3, 2, 32, 8, 40, 2, row_offset, temperature, seed_ptr, *ptrs, tokens.data_ptr(),
-                                     work.data_ptr(), None)
+    def call(row_offset=0, temperature=1.0, seed_ptr=seed.data_ptr(), T=3, K=1):
+        a = _decode_args(ptrs, mode=DECODE_SAMPLED, T=T, B=2, K=K, H=32, E=8, V=40, start_token=2, row_offset=row_offset,
+                         temperature=temperature, seed=seed_ptr, tokens=tokens.data_ptr(), work=work.data_ptr())
+        return lib.pcd_decode(ctypes.byref(a), None)
 
     assert call() == 0
     for kw in (dict(temperature=0.0), dict(temperature=-2.0), dict(temperature=float("nan")), dict(temperature=float("inf")),
-               dict(seed_ptr=None), dict(row_offset=-1)):
+               dict(seed_ptr=None), dict(row_offset=-1), dict(K=2)):
         assert call(**kw) == -1, kw                  # PCD_ERR_ARG
+        assert call(T=0, **kw) == -1, kw             # before the shape check
+    assert call(T=0) == -2                           # PCD_ERR_UNSUPPORTED
 
 
 def test_unrolled_twin_keeps_the_sampling_configuration():
@@ -268,9 +264,10 @@ def test_sampled_decode_in_a_cuda_graph():
 
 
 @pytest.mark.gpu
-def test_graphed_lct_step_with_sampled_questions(monkeypatch):
+def test_graphed_lct_step_decodes_in_sampled_mode(monkeypatch):
     """search.GraphedLctStep with a sampling EF model: the three generate() calls of ArchitectLct.step run on
-    pcd_decode_sample (counted while capturing: replays do not call the library) and the replays give finite losses."""
+    the sampled mode of pcd_decode (counted while capturing: replays do not call the library) and the replays give finite
+    losses."""
     import pcd_native
     from search import GraphedLctStep
     monkeypatch.setitem(P.LCT_DIMS, "hidden_size", 32)        # inside the decode envelope (embed = hidden: h0 is the image
@@ -278,14 +275,13 @@ def test_graphed_lct_step_with_sampled_questions(monkeypatch):
     ef, _, arch = P.make_lct("cuda")
     ef.qst_encoder.deterministic = False
     lib = pcd_native.load_cuda()
-    sample, greedy = _Counting(lib.pcd_decode_sample), _Counting(lib.pcd_decode_greedy)
-    monkeypatch.setattr(lib, "pcd_decode_sample", sample)
-    monkeypatch.setattr(lib, "pcd_decode_greedy", greedy)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
     tr, va = P.lct_batch(21, "cuda"), P.lct_batch(22, "cuda")
     graphed = GraphedLctStep(arch, tr, va, 1e-3, 1e-3, warmup=1)
-    assert sample.calls == 3 * 2 and greedy.calls == 0           # one warm-up step + the captured step
+    assert rec.count(DECODE_SAMPLED) == 3 * 2 and rec.count(DECODE_GREEDY) == 0       # one warm-up step + the captured step
     losses = []
     for _ in range(2):
         losses.append(float(graphed(tr, va)))
         torch.cuda.synchronize()
-    assert sample.calls == 6 and all(math.isfinite(x) for x in losses), losses
+    assert rec.count(DECODE_SAMPLED) == 6 and all(math.isfinite(x) for x in losses), losses

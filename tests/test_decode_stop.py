@@ -1,11 +1,12 @@
-"""End-of-sequence decoding (pcd_decode_{greedy,sample,beam}_stop, the end_token / pad_token / length_penalty keywords of
-pcd_ops and QstEncoder).  CPU cases run the kernel source's -DPCD_EMU build; `gpu` cases run the sm_100a kernel.
+"""End-of-sequence decoding (pcd_decode with stop = 1, the end_token / pad_token / length_penalty keywords of pcd_ops and
+QstEncoder).  CPU cases run the kernel source's -DPCD_EMU build; `gpu` cases run the sm_100a kernel.
 
 Greedy and sampled rows are independent and choose every word as without the stop, so a stopped decode must equal the
 unstopped one truncated after the first end word and filled with the pad word, bit for bit.  Beams are compared with the
 float64 search of stop_oracle.py under the margin rule of test_decode_beam.py applied to the ranking keys s / L^alpha: the
 key of a hypothesis of length L >= 1 carries at most the error of its raw score (alpha >= 0), so the same TAU bounds it."""
 import copy
+import ctypes
 
 import pytest
 import torch
@@ -13,7 +14,8 @@ import torch
 import beam_oracle as BO
 import parity_cases as P
 import stop_oracle as SO
-from test_decode_beam import PROD, TAU, _Counting, _modules
+from pcd_native import DECODE_BEAM, DECODE_GREEDY, DECODE_SAMPLED
+from test_decode_beam import PROD, TAU, _Decodes, _decode_args, _modules
 
 END, PAD = 3, 0                  # the vocabulary's <end> and <pad>
 
@@ -147,18 +149,15 @@ def test_batch_slicing_does_not_change_the_result(emulation):
         assert torch.equal(t1[0], tokens[b]) and torch.equal(s1[0], scores[b])
 
 
-def test_generate_routes_to_the_stop_entry_points(emulation, monkeypatch):
-    """end_token=None keeps the old entry points; a set end_token reaches the _stop ones (both packages, all three modes)."""
+def test_generate_routes_to_the_stop_mode(emulation, monkeypatch):
+    """end_token=None decodes without the stop; a set end_token decodes with it (both packages, all three modes)."""
     import models_lct
     import pcd_ops
     import vqa_model
     lib = emulation
-    names = ("pcd_decode_greedy", "pcd_decode_sample", "pcd_decode_beam",
-             "pcd_decode_greedy_stop", "pcd_decode_sample_stop", "pcd_decode_beam_stop")
-    stubs = {n: _Counting(getattr(lib, n)) for n in names}
-    for n, s in stubs.items():
-        monkeypatch.setattr(lib, n, s)
-    calls = lambda: tuple(stubs[n].calls for n in names)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
+    calls = lambda: tuple(rec.count(mode, stop) for stop in (0, 1) for mode in (DECODE_GREEDY, DECODE_SAMPLED, DECODE_BEAM))
     torch.manual_seed(3)
     img = 0.3 * torch.randn(3, 32)
     for mod in (vqa_model, models_lct):
@@ -199,7 +198,7 @@ def test_outside_the_envelope_raises_even_with_stock_ops(emulation):
         __import__("pcd_ops").allow_stock_ops(prev)
 
 
-def test_bad_arguments(emulation):
+def test_bad_stop_arguments(emulation):
     from pcd_ops import decode_beam, decode_greedy, decode_sample
     import pcd_native
     emb, lstm, proj, h0 = _modules(2, 32, 8, 6)
@@ -221,20 +220,24 @@ def test_bad_arguments(emulation):
     ptrs = [t.detach().data_ptr() for t in ops]
     tokens = torch.empty(64 * 3, dtype=torch.long)
     scores = torch.empty(64)
-    work = torch.empty(int(lib.pcd_decode_beam_work_floats(8, 8, 32, 6)))
+    work = torch.empty(int(lib.pcd_decode_work_floats(ctypes.byref(pcd_native.DecodeArgs(mode=DECODE_BEAM, B=8, K=8, H=32,
+                                                                                          V=6)))))
     seed = torch.tensor([5], dtype=torch.int64)
 
     def calls(stop):
-        sp = None if stop is None else pcd_native.C.byref(stop)
-        return (lib.pcd_decode_greedy_stop(3, 2, 32, 8, 6, 2, *ptrs, tokens.data_ptr(), work.data_ptr(), sp, None),
-                lib.pcd_decode_sample_stop(3, 2, 32, 8, 6, 2, 0, 1.0, seed.data_ptr(), *ptrs, tokens.data_ptr(),
-                                           work.data_ptr(), sp, None),
-                lib.pcd_decode_beam_stop(3, 2, 2, 32, 8, 6, 2, *ptrs, tokens.data_ptr(), scores.data_ptr(), work.data_ptr(),
-                                         sp, None))
+        """the three modes with the stop (end_token, pad_token, length_penalty); None: a null pcd_decode_args"""
+        if stop is None:
+            return (lib.pcd_decode(None, None),) * 3
+        end, pad, alpha = stop
+        common = dict(T=3, H=32, E=8, V=6, start_token=2, stop=1, end_token=end, pad_token=pad, length_penalty=alpha,
+                      tokens=tokens.data_ptr(), work=work.data_ptr())
+        return tuple(lib.pcd_decode(ctypes.byref(_decode_args(ptrs, **common, **kw)), None) for kw in (
+            dict(mode=DECODE_GREEDY, B=2, K=1),
+            dict(mode=DECODE_SAMPLED, B=2, K=1, temperature=1.0, seed=seed.data_ptr()),
+            dict(mode=DECODE_BEAM, B=2, K=2, scores=scores.data_ptr())))
 
-    S = pcd_native.DecodeStop
-    assert calls(S(3, 0, 0.5)) == (0, 0, 0)
-    for bad in (None, S(6, 0, 0.0), S(-1, 0, 0.0), S(3, 6, 0.0), S(3, -1, 0.0), S(3, 0, float("nan")), S(3, 0, float("inf"))):
+    assert calls((3, 0, 0.5)) == (0, 0, 0)
+    for bad in (None, (6, 0, 0.0), (-1, 0, 0.0), (3, 6, 0.0), (3, -1, 0.0), (3, 0, float("nan")), (3, 0, float("inf"))):
         assert calls(bad) == (-1, -1, -1), bad                       # PCD_ERR_ARG
 
 
@@ -394,9 +397,10 @@ def test_stop_generate_in_a_cuda_graph(beam_size, deterministic):
 
 
 @pytest.mark.gpu
-def test_graphed_lct_step_with_stop_and_beams(monkeypatch):
+def test_graphed_lct_step_decodes_beams_with_the_stop(monkeypatch):
     """search.GraphedLctStep with end_token = 3 and beam_size = 4 on the EF model and its unrolled twin: the three generate()
-    calls of ArchitectLct.step run on pcd_decode_beam_stop, the replays give finite losses and the first equals the eager step."""
+    calls of ArchitectLct.step run on pcd_decode in beam mode with the stop, the replays give finite losses and the first
+    equals the eager step."""
     import math
     import config
     import pcd_native
@@ -414,12 +418,11 @@ def test_graphed_lct_step_with_stop_and_beams(monkeypatch):
     for ef in (ef1, ef2):
         ef.qst_encoder.beam_size, ef.qst_encoder.end_token, ef.qst_encoder.length_penalty = 4, END, 0.7
     lib = pcd_native.load_cuda()
-    stop, beam = _Counting(lib.pcd_decode_beam_stop), _Counting(lib.pcd_decode_beam)
-    monkeypatch.setattr(lib, "pcd_decode_beam_stop", stop)
-    monkeypatch.setattr(lib, "pcd_decode_beam", beam)
+    rec = _Decodes(lib.pcd_decode)
+    monkeypatch.setattr(lib, "pcd_decode", rec)
     tr, va = P.lct_batch(21, "cuda"), P.lct_batch(22, "cuda")
     graphed = GraphedLctStep(arch2, tr, va, 1e-3, 1e-3, warmup=2)
-    assert stop.calls == 3 * 3 and beam.calls == 0             # two warm-up steps + the captured step
+    assert rec.count(DECODE_BEAM, 1) == 3 * 3 and len(rec.seen) == 3 * 3       # two warm-up steps + the captured step
     for _ in range(2):
         eager.step(*tr, *va, 1e-3, 1e-3)
     eager.step(*tr, *va, 1e-3, 1e-3)

@@ -103,7 +103,7 @@ def test_product_refuses_cpu_without_emulation():
 
 @pytest.mark.parametrize("B,H,E,V,T", [(5, 32, 12, 300, 7), (3, 64, 8, 128, 4)])
 def test_greedy_decode(B, H, E, V, T):
-    """Host side of pcd_decode_greedy (argument marshalling, token layout, <start>/tanh convention) on the emulation build."""
+    """Host side of the greedy decode (argument marshalling, token layout, <start>/tanh convention) on the emulation build."""
     P.decode_case("cpu", B, H, E, V, T)
 
 
