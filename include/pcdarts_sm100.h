@@ -498,13 +498,30 @@ int pcd_lstm_backward(int T, int B, int H, const float* dhs, const float* dhT, c
  *   early exit: once every row of the launch has finished, the kernel leaves its time loop and the remaining positions are
  *              P (beams: the backtrack starts from the last step run).
  *
+ * Truncated sampling (sampled mode, truncate = 1; HF-style order: temperature, then top-k, then top-p renormalised over the
+ * top-k set).  l is a row's fp32 logits (as above), T the temperature.
+ *   order:     v precedes w iff l_v > l_w, or l_v = l_w and v < w (ties to the lower word, as the greedy argmax; -0 = +0).
+ *   top-k:     S_k = the first min(top_k, V) words in that order; top_k = 0 (or >= V): all V words.
+ *   nucleus:   q_v = expf((l_v - l_max) / T) in fp32, rounded to an integer multiple of 2^-s with s = 63 - (bit length
+ *              of V); these masses are summed exactly in 64-bit integers, so any summation order gives the same sums.
+ *              Z = sum of q over S_k; the target is ceil(top_p * Z) with Z rounded to fp64 and the product in fp64 (at
+ *              most Z).  S = the shortest prefix of S_k, in order, whose mass reaches the target: never empty (the first
+ *              word has q = 1).  top_p = 1: S = S_k, with no mass computed.
+ *   draw:      word t of row b = argmax over v in S of (l_v / T + G(seed, t, row_offset + b, v)), the score and noise of
+ *              untruncated sampling, ties to the lower word: distributed as softmax(l / T) restricted to S and renormalised.
+ *   So top_k = 0 with top_p = 1 gives the untruncated words bit for bit, and top_k = 1, or a top_p below 1/V, the greedy
+ *   words.  stop = 1 combines as with plain sampling.  The kernel keeps each step's logits in the workspace (rows x V
+ *   floats) and finds S by radix select behind one more grid barrier per step.
+ *
  * Envelope: H a multiple of 32 up to 512, E a multiple of 4, start_token in [0, V); greedy and sampled: B <= 64 rows; beam:
  * 1 <= K <= 8, K <= V, B*K <= 64 rows.  PCD_ERR_UNSUPPORTED outside it.
  * PCD_ERR_ARG, before any shape check: a mode outside the three; K != 1 outside beam mode; a null emb .. b_out, tokens or
  * work, or a null scores in beam mode; sampled: a null seed, a negative row_offset or a temperature that is not finite and
- * > 0; stop: an E or P outside [0, V) or an alpha that is not finite.
+ * > 0; stop: an E or P outside [0, V) or an alpha that is not finite; truncate = 1 outside sampled mode, a negative
+ * top_k, or a top_p that is not finite or lies outside (0, 1].
  * PCD_ERR_ALIGN: emb, w_ih, w_hh, h0, w_out and work must be 16-byte aligned, the seed 8-byte aligned.
- * work: pcd_decode_work_floats(a) floats (it reads mode, B, K, H and V).  The call only uses caller-owned memory and
+ * work: pcd_decode_work_floats(a) floats (it reads mode, B, K, H, V and truncate; truncation adds B x V + B floats).
+ * The call only uses caller-owned memory and
  * neither synchronises nor allocates (CUDA-graph capturable).  All reductions run in a fixed order: equal inputs give
  * bit-equal outputs.
  * ---------------------------------------------------------------------------------------------- */
@@ -519,6 +536,9 @@ typedef struct pcd_decode_args {
     float length_penalty;             /* beam with stop only */
     float temperature;                /* sampled only */
     int row_offset;                   /* sampled only: global index of row 0 */
+    int truncate;                     /* sampled only, 1: top-k / nucleus truncation (0: sample from every word) */
+    int top_k;                        /* truncate only: 0 = no top-k limit */
+    float top_p;                      /* truncate only: in (0, 1], 1 = no nucleus */
     const unsigned long long* seed;   /* sampled only */
     const float *emb, *w_ih, *w_hh, *b_ih, *b_hh, *h0, *c0, *w_out, *b_out;
     long long* tokens;                /* [B][T]; beam [B][K][T] */

@@ -29,6 +29,10 @@
 // carries the raw score beside that key, and each row's frozen length persists in the workspace.  Every block sees every
 // row's state (greedy / sampled: pick_words runs everywhere; beam: the lengths are read behind the merge barrier), so all
 // blocks leave the time loop at the same step once every row has finished, without another barrier.
+// Truncated sampling (kTrunc, sampled mode only: top-k and nucleus): the phase-B epilogue stores the logits into a
+// [rows][V] workspace stash instead of ranking them; behind one more grid barrier each block takes whole rows, finds the
+// kept set by radix select (select_words) and draws the Gumbel argmax over it into a word buffer, which the next step
+// reads in place of pick_words.
 #include "../../include/pcdarts_sm100.h"
 #include "pcd_launch.cuh"
 #include "pcd_philox.cuh"
@@ -56,6 +60,8 @@ static int validate(const pcd_decode_args* a) {
     if (a->stop && !(a->end_token >= 0 && a->end_token < a->V && a->pad_token >= 0 && a->pad_token < a->V &&
                      isfinite(a->length_penalty)))
         return PCD_ERR_ARG;
+    if (a->truncate && !(a->mode == kSampled && a->top_k >= 0 && isfinite(a->top_p) && a->top_p > 0.f && a->top_p <= 1.f))
+        return PCD_ERR_ARG;
     if (!a->emb || !a->w_ih || !a->w_hh || !a->b_ih || !a->b_hh || !a->h0 || !a->c0 || !a->w_out || !a->b_out || !a->tokens ||
         !a->work || (a->mode == kBeam && !a->scores))
         return PCD_ERR_ARG;
@@ -65,12 +71,13 @@ static int validate(const pcd_decode_args* a) {
 }
 
 // workspace offsets in floats, rows = B x K:  hbuf [2][rows][H] | tbuf [rows][H] | then greedy / sampled: candidates
-// [rows][ntiles] float2;  beam: cbuf [2][rows][H] | top-K candidates [rows][ntiles][K] float2 | tile (max, sum exp)
-// [rows][ntiles] float2 | beam scores [rows] | finished lengths [rows] int (end-of-sequence decode)
+// [rows][ntiles] float2 | truncated sampling only: logits [rows][V] | words [rows] int;  beam: cbuf [2][rows][H] | top-K
+// candidates [rows][ntiles][K] float2 | tile (max, sum exp) [rows][ntiles] float2 | beam scores [rows] | finished lengths
+// [rows] int (end-of-sequence decode)
 struct Work {
-    size_t tbuf, cand, cbuf, bcand, bstat, bscore, blen, floats;
+    size_t tbuf, cand, cbuf, bcand, bstat, bscore, blen, stash, words, floats;
 };
-static Work work_of(int mode, int B, int K, int H, int V) {
+static Work work_of(int mode, int B, int K, int H, int V, bool truncate) {
     const size_t rows = (size_t)B * K, nt = tiles_of(V), rh = rows * H;
     Work w = {};
     w.tbuf = 2 * rh;
@@ -84,14 +91,43 @@ static Work work_of(int mode, int B, int K, int H, int V) {
     } else {
         w.cand = 3 * rh;
         w.floats = w.cand + 2 * rows * nt;
+        if (truncate) {
+            w.stash = w.floats;
+            w.words = w.stash + rows * (size_t)V;
+            w.floats = w.words + rows;
+        }
     }
     return w;
+}
+
+// truncated sampling (pcdarts_sm100.h): the order-preserving image of (logit, word), larger logit first and ties to the
+// lower word (-0 counts as +0), and a word's mass q = expf((l - lmax) / T) in fp32 as an integer multiple of 2^-s,
+// s = 63 - bit length of V, so that the masses of a row sum exactly (in any order) below 2^63
+PCD_HOSTDEV unsigned long long order_key(float l, int v) {
+    const float z = l == 0.f ? 0.f : l;
+    uint32_t b;
+    memcpy(&b, &z, sizeof b);
+    b ^= (b & 0x80000000u) ? 0xffffffffu : 0x80000000u;
+    return ((unsigned long long)b << 32) | (0xffffffffu - (uint32_t)v);
+}
+PCD_HOSTDEV int mass_shift(int V) {
+    int bits = 0;
+    while (bits < 31 && (V >> bits)) ++bits;
+    return 63 - bits;
+}
+PCD_HOSTDEV unsigned long long mass_of(float l, float lmax, float T, float scale) {
+    return (unsigned long long)rintf(expf((l - lmax) / T) * scale);      // scale = 2^s: exact
+}
+// the nucleus target: Z rounded to fp64, times top_p, rounded up; never above Z
+PCD_HOSTDEV unsigned long long nucleus_target(unsigned long long Z, float top_p) {
+    const unsigned long long t = (unsigned long long)ceil((double)Z * (double)top_p);
+    return t > Z ? Z : t;
 }
 }  // namespace decode
 }  // namespace pcd
 
 extern "C" size_t pcd_decode_work_floats(const pcd_decode_args* a) {
-    return a ? pcd::decode::work_of(a->mode, a->B, a->K, a->H, a->V).floats : 0;
+    return a ? pcd::decode::work_of(a->mode, a->B, a->K, a->H, a->V, a->mode == pcd::decode::kSampled && a->truncate).floats : 0;
 }
 
 #if PCD_CUDA
@@ -122,6 +158,11 @@ struct Args {
     int end_token, pad_token;
     float length_penalty; // beam: candidates ranked by score / L^length_penalty (0: by score)
     int* blen;            // [B]  beam: length of a finished beam counting end_token, 0 while it is live
+    // truncated sampling only (kTrunc)
+    int top_k;            // 0: no top-k limit
+    float top_p;          // 1: no nucleus
+    float* stash;         // [B][V]  the step's fp32 logits
+    int* words;           // [B]     the step's words
 };
 
 __device__ __forceinline__ float sigm(float x) { return 1.f / (1.f + expf(-x)); }
@@ -339,7 +380,195 @@ __device__ __forceinline__ void merge_beams(const Args& a, int t, float* S) {
     }
 }
 
-template <int kMode, bool kStop>
+// ---- truncated sampling: the select phase ------------------------------------------------------------------------------
+constexpr int kSelFloats = 1536;          // tail of the U region: histograms and reduction scratch of the select phase
+PCD_HOSTDEV int stage_cap(int H) { return u_floats(H) - kSelFloats; }
+
+// the boundary of a row's kept set by radix select on the 64-bit order keys, 8 bits per pass from the top: the returned
+// key C has { v : key_v >= C } = the first `need` words in order (kMass = false), or the shortest prefix whose mass
+// reaches `need` (kMass = true), among the words with key >= lo.  A pass stops early once the bucket that holds the
+// boundary is taken whole (its remaining bits are then 0, so C is the larger of that prefix and lo).  Counts and masses
+// are integers: every pass gives the same histogram whatever the order of its atomics.  The 64-bit shared atomic is a
+// compare-and-swap loop, and most words of a row share a few high buckets, so the lanes of a warp that hit one bucket
+// add their masses once, through the warp's scratch xs[32].
+template <bool kMass, class Load>
+__device__ unsigned long long radix_select(Load load, int V, float lmax, float T, float scale, unsigned long long lo,
+                                           unsigned long long need, unsigned* cnt, unsigned long long* mass,
+                                           unsigned long long* bc, unsigned long long* xs) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    unsigned long long P = 0, M = 0;
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        cnt[tid] = 0u;
+        if constexpr (kMass) mass[tid] = 0ull;
+        __syncthreads();
+        for (int base = 0; base < V; base += kT) {          // uniform trip count: the whole warp reaches the match
+            const int v = base + tid;
+            int d = 256;
+            unsigned long long m = 0;
+            if (v < V) {
+                const float l = load(v);
+                const unsigned long long k = order_key(l, v);
+                if (k >= lo && (k & M) == P) {
+                    d = (int)(k >> shift) & 255;
+                    atomicAdd(cnt + d, 1u);
+                    if constexpr (kMass) m = mass_of(l, lmax, T, scale);
+                }
+            }
+            if constexpr (kMass) {
+                const unsigned peers = __match_any_sync(0xffffffffu, d);
+                xs[lane] = m;
+                __syncwarp();
+                if (d < 256 && lane == __ffs(peers) - 1) {
+                    unsigned long long sum = 0;
+                    for (unsigned r = peers; r; r &= r - 1) sum += xs[__ffs(r) - 1];
+                    atomicAdd(mass + d, sum);
+                }
+                __syncwarp();
+            }
+        }
+        __syncthreads();
+        if (tid < 32) {
+            // lane l holds the buckets 255 - 8l .. 248 - 8l (descending); a warp scan finds the bucket where `need` is met
+            unsigned long long own = 0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) own += kMass ? mass[255 - 8 * lane - j] : cnt[255 - 8 * lane - j];
+            unsigned long long inc = own;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned long long x = __shfl_up_sync(0xffffffffu, inc, o);
+                if (lane >= o) inc += x;
+            }
+            const int first = __ffs(__ballot_sync(0xffffffffu, inc >= need)) - 1;
+            if (lane == first) {
+                unsigned long long acc = inc - own;
+                for (int j = 0; j < 8; ++j) {
+                    const int d = 255 - 8 * lane - j;
+                    const unsigned long long x = kMass ? mass[d] : cnt[d];
+                    if (acc + x >= need) {
+                        const unsigned long long left = need - acc;
+                        bc[0] = P | ((unsigned long long)d << shift);
+                        bc[1] = left;
+                        bc[2] = cnt[d] == 1u || (!kMass && cnt[d] == left) || shift == 0;
+                        break;
+                    }
+                    acc += x;
+                }
+            }
+        }
+        __syncthreads();
+        P = bc[0];
+        need = bc[1];
+        const bool done = bc[2] != 0;
+        M |= 255ull << shift;
+        __syncthreads();                  // bc and the histograms are rewritten by the next pass
+        if (done) break;
+    }
+    return P > lo ? P : lo;
+}
+
+// one row: S = the kept set of pcdarts_sm100.h, then the Gumbel argmax over S -> a.words[row]
+template <class Load>
+__device__ void select_row(const Args& a, int t, int row, Load load, float lmax, unsigned* cnt, unsigned long long* mass,
+                           unsigned long long* bc, float* red, unsigned long long* xs) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, V = a.V;
+    const float T = a.temperature;
+    const int s = mass_shift(V);
+    const float scale = __int_as_float((127 + s) << 23);
+    unsigned long long C = 0;             // every key is >= 0: no truncation
+    if (a.top_k > 0 && a.top_k < V)
+        C = radix_select<false>(load, V, lmax, T, scale, 0ull, (unsigned long long)a.top_k, cnt, mass, bc, xs);
+    if (a.top_p < 1.f) {
+        unsigned long long z = 0;
+        for (int v = tid; v < V; v += kT) {
+            const float l = load(v);
+            if (order_key(l, v) >= C) z += mass_of(l, lmax, T, scale);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) z += __shfl_xor_sync(0xffffffffu, z, o);
+        if (lane == 0) mass[warp] = z;
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long Z = 0;
+            for (int w = 0; w < kT / 32; ++w) Z += mass[w];
+            bc[3] = nucleus_target(Z, a.top_p);
+        }
+        __syncthreads();
+        const unsigned long long tgt = bc[3];
+        __syncthreads();
+        C = radix_select<true>(load, V, lmax, T, scale, C, tgt, cnt, mass, bc, xs);
+    }
+    // Gumbel argmax over S: the score of untruncated sampling, one Philox block per 4 words with a kept word
+    const unsigned long long seed = __ldg(a.seed);
+    const uint32_t grow = (uint32_t)(a.row_offset + row);
+    float best = -INFINITY;
+    int bi = INT_MAX;
+    for (int j = tid; 4 * j < V; j += kT) {
+        float l[4];
+        unsigned in = 0u;
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {
+            const int v = 4 * j + w;
+            l[w] = v < V ? load(v) : 0.f;
+            if (v < V && order_key(l[w], v) >= C) in |= 1u << w;
+        }
+        if (in) {
+            const Philox4 blk = philox4x32_10((uint32_t)j, (uint32_t)t, grow, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
+#pragma unroll
+            for (int w = 0; w < 4; ++w)
+                if ((in >> w) & 1u) {
+                    const float sc = l[w] / T + gumbel_of_bits(blk.w[w]);
+                    if (better(sc, 4 * j + w, best, bi)) { best = sc; bi = 4 * j + w; }
+                }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (better(ov, oi, best, bi)) { best = ov; bi = oi; }
+    }
+    if (lane == 0) { red[warp] = best; red[8 + warp] = __int_as_float(bi); }
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < kT / 32; ++w)
+            if (better(red[w], __float_as_int(red[8 + w]), best, bi)) { best = red[w]; bi = __float_as_int(red[8 + w]); }
+        __stcg(a.words + row, (bi >= 0 && bi < V) ? bi : 0);
+    }
+    __syncthreads();                      // red reused by the next row
+}
+
+// step t of the truncated sampled decode, behind the grid barrier after phase B: block r takes rows r, r + gridDim.x, ...
+// A row's logits are staged in the U region when V fits (it does at V = 17858 for every H), else every pass reads L2.
+__device__ void select_words(const Args& a, int t, float* U) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, V = a.V;
+    float* tail = U + stage_cap(a.H);
+    unsigned long long* mass = reinterpret_cast<unsigned long long*>(tail);          // [256]
+    unsigned* cnt = reinterpret_cast<unsigned*>(tail + 512);                          // [256]
+    unsigned long long* bc = reinterpret_cast<unsigned long long*>(tail + 768);       // [4] pass result
+    float* red = tail + 776;                                                          // [16] reductions
+    unsigned long long* xs = reinterpret_cast<unsigned long long*>(tail + 800) + 32 * warp;   // [8 warps][32]
+    const bool staged = V <= stage_cap(a.H);
+    for (int row = blockIdx.x; row < a.B; row += gridDim.x) {
+        const float* src = a.stash + (long long)row * V;
+        float m = -INFINITY;
+        for (int v = tid; v < V; v += kT) {
+            const float l = __ldcg(src + v);
+            if (staged) U[v] = l;
+            m = fmaxf(m, l);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+        if (lane == 0) red[warp] = m;
+        __syncthreads();
+        float lmax = red[0];
+        for (int w = 1; w < kT / 32; ++w) lmax = fmaxf(lmax, red[w]);
+        __syncthreads();
+        if (staged) select_row(a, t, row, [U](int v) { return U[v]; }, lmax, cnt, mass, bc, red, xs);
+        else select_row(a, t, row, [src](int v) { return __ldcg(src + v); }, lmax, cnt, mass, bc, red, xs);
+    }
+}
+
+template <int kMode, bool kStop, bool kTrunc = false>
 __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
     constexpr bool kSample = kMode == kSampled, kBeamMode = kMode == kBeam;
     cg::grid_group grid = cg::this_grid();
@@ -392,6 +621,8 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
                 TOK[tid] = (int)(p & 0xffffffffll);
                 PAR[tid] = (int)(p >> 32);
             }
+        } else if constexpr (kTrunc) {
+            if (tid < B) TOK[tid] = __ldcg(a.words + tid);
         } else pick_words(a, TOK);
         if constexpr (kStop && kBeamMode) {
             // every block reads every row's finished length behind the merge barrier, so all of them leave at the same step
@@ -569,6 +800,17 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
                         for (int o = 8; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
                         if (tx == 0 && row < B) __stcg(a.bstat + (long long)row * a.ntiles + tile, make_float2(mx, se));
                     }
+                } else if constexpr (kTrunc) {
+                    // the select phase behind the next barrier needs whole rows: the tile's logits go to the stash
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        const int row = 4 * ty + i;
+#pragma unroll
+                        for (int j = 0; j < 8; ++j) {
+                            const int col = col0 + tx + 16 * j;
+                            if (row < B && col < a.V) __stcg(a.stash + (long long)row * a.V + col, acc[i][j] + __ldg(a.b_out + col));
+                        }
+                    }
                 } else {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
@@ -623,6 +865,9 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
         if constexpr (kBeamMode) {
             merge_beams<kStop>(a, t, U);
             grid.sync();
+        } else if constexpr (kTrunc) {
+            select_words(a, t, U);
+            grid.sync();
         }
     }
     if constexpr (kBeamMode) {
@@ -646,14 +891,18 @@ __global__ void __launch_bounds__(kT, 1) decode_kernel(Args a) {
     } else if (blockIdx.x == 0) {
         if constexpr (kStop) {
             if (t_run == a.T) {
-                pick_words(a, TOK);
+                if constexpr (kTrunc) {
+                    if (tid < B) TOK[tid] = __ldcg(a.words + tid);
+                } else pick_words(a, TOK);
                 __syncthreads();
                 if (tid < B) a.tokens[(long long)tid * a.T + a.T - 1] = FIN[tid] ? a.pad_token : TOK[tid];
             } else if (tid < B) {
                 for (int t = t_run; t < a.T; ++t) a.tokens[(long long)tid * a.T + t] = a.pad_token;
             }
         } else {
-            pick_words(a, TOK);
+            if constexpr (kTrunc) {
+                if (tid < B) TOK[tid] = __ldcg(a.words + tid);
+            } else pick_words(a, TOK);
             __syncthreads();
             if (tid < B) a.tokens[(long long)tid * a.T + a.T - 1] = TOK[tid];
         }
@@ -667,20 +916,20 @@ namespace pcd {
 namespace decode {
 
 // the kernel of one (mode, stop) pair; its first call reads the SM count and sets the kernel's shared-memory limit
-template <int kMode, bool kStop>
+template <int kMode, bool kStop, bool kTrunc = false>
 static const void* kernel_of(int& sms_out, LaunchState& L) {
     static int sms = 0;                                     // per instantiation: each one sets its own smem attribute
     if (!sms) {
         int dev = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-            cudaFuncSetAttribute(decode_kernel<kMode, kStop>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
+            cudaFuncSetAttribute(decode_kernel<kMode, kStop, kTrunc>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
             sms = 0;
             snprintf(L.last_err, sizeof L.last_err, "decode setup: %s", cudaGetErrorString(cudaGetLastError()));
             return nullptr;
         }
     }
     sms_out = sms;
-    return (const void*)decode_kernel<kMode, kStop>;
+    return (const void*)decode_kernel<kMode, kStop, kTrunc>;
 }
 
 // a call that passed validate(): alignment, shared memory, grid, then one cooperative launch
@@ -696,14 +945,16 @@ static int run(const pcd_decode_args& p, void* stream) {
     static const KernelOf kernels[3][2] = {{kernel_of<kGreedy, false>, kernel_of<kGreedy, true>},
                                            {kernel_of<kSampled, false>, kernel_of<kSampled, true>},
                                            {kernel_of<kBeam, false>, kernel_of<kBeam, true>}};
+    static const KernelOf truncating[2] = {kernel_of<kSampled, false, true>, kernel_of<kSampled, true, true>};
+    const bool trunc = p.mode == kSampled && p.truncate;
     int sms = 0;
-    const void* kernel = kernels[p.mode][p.stop ? 1 : 0](sms, L);
+    const void* kernel = trunc ? truncating[p.stop ? 1 : 0](sms, L) : kernels[p.mode][p.stop ? 1 : 0](sms, L);
     if (!kernel) return PCD_ERR_CUDA;
     const int ntiles = tiles_of(V);
     int grid = ntiles < sms ? ntiles : sms;                 // one block per SM: all of them co-resident (cooperative launch)
     if (grid < H / kUnits) grid = H / kUnits;
     if (grid > sms) return PCD_ERR_UNSUPPORTED;
-    const Work w = work_of(p.mode, p.B, p.K, H, V);
+    const Work w = work_of(p.mode, p.B, p.K, H, V, trunc);
     Args a;
     a.T = p.T; a.B = B; a.H = H; a.E = E; a.V = V; a.start = p.start_token; a.ntiles = ntiles;
     a.emb = p.emb; a.w_ih = p.w_ih; a.w_hh = p.w_hh; a.b_ih = p.b_ih; a.b_hh = p.b_hh; a.h0 = p.h0; a.c0 = p.c0;
@@ -721,6 +972,9 @@ static int run(const pcd_decode_args& p, void* stream) {
     a.scores = p.scores;
     a.end_token = p.end_token; a.pad_token = p.pad_token; a.length_penalty = p.length_penalty;
     a.blen = reinterpret_cast<int*>(p.work + w.blen);
+    a.top_k = p.top_k; a.top_p = p.top_p;
+    a.stash = p.work + w.stash;
+    a.words = reinterpret_cast<int*>(p.work + w.words);
     void* args[] = {&a};
     cudaError_t e = cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(kT), args, smem, (cudaStream_t)stream);
     count_launch(L);
@@ -773,12 +1027,35 @@ static void step_emu(const pcd_decode_args& a, int word, int t, const float* h, 
     }
 }
 
+// truncated sampling: the smallest order key of the kept set S of a row's logits (pcdarts_sm100.h), by sorting where the
+// kernel runs a radix select; the masses are the kernel's integers
+static unsigned long long kept_boundary(const pcd_decode_args& a, const float* logit) {
+    const int V = a.V;
+    std::vector<unsigned long long> key((size_t)V);
+    float lmax = -INFINITY;
+    for (int v = 0; v < V; ++v) { key[v] = order_key(logit[v], v); lmax = logit[v] > lmax ? logit[v] : lmax; }
+    std::vector<int> order((size_t)V);
+    for (int v = 0; v < V; ++v) order[v] = v;
+    std::sort(order.begin(), order.end(), [&](int x, int y) { return key[x] > key[y]; });
+    int n = a.top_k > 0 && a.top_k < V ? a.top_k : V;
+    if (a.top_p < 1.f) {
+        const float scale = ldexpf(1.f, mass_shift(V));
+        unsigned long long Z = 0, acc = 0;
+        for (int i = 0; i < n; ++i) Z += mass_of(logit[order[i]], lmax, a.temperature, scale);
+        const unsigned long long tgt = nucleus_target(Z, a.top_p);
+        int i = 0;
+        while ((acc += mass_of(logit[order[i]], lmax, a.temperature, scale)) < tgt) ++i;
+        n = i + 1;
+    }
+    return key[order[n - 1]];
+}
+
 // greedy / sampled: argmax of the fp32 logit (greedy) or of logit / T + G(seed, t, row_offset + b, v) (sampled); ties go
-// to the lowest index.  stop: after end_token a row's remaining positions are pad_token (rows are independent, so the row
-// simply ends there)
+// to the lowest index.  truncate: the sampled argmax runs over the kept set only.  stop: after end_token a row's remaining
+// positions are pad_token (rows are independent, so the row simply ends there)
 static int decode_emu(const pcd_decode_args& a) {
     const int T = a.T, B = a.B, H = a.H, V = a.V;
-    const bool sample = a.mode == kSampled;
+    const bool sample = a.mode == kSampled, trunc = sample && a.truncate;
     const unsigned long long key = sample ? *a.seed : 0ull;
     std::vector<float> h(a.h0, a.h0 + (size_t)B * H), c(a.c0, a.c0 + (size_t)B * H), hn((size_t)H), logit((size_t)V);
     for (int b = 0; b < B; ++b) {
@@ -788,9 +1065,11 @@ static int decode_emu(const pcd_decode_args& a) {
         for (int t = 0; t < T; ++t) {
             step_emu(a, word, t, hb, cb, hn.data(), cb, logit.data());
             std::copy(hn.begin(), hn.end(), hb);
+            const unsigned long long lo = trunc ? kept_boundary(a, logit.data()) : 0ull;
             float best = -INFINITY;
             int bi = 0;
             for (int v = 0; v < V; ++v) {
+                if (trunc && order_key(logit[v], v) < lo) continue;
                 const float score = sample ? logit[v] / a.temperature + decode_gumbel(key, t, a.row_offset + b, v) : logit[v];
                 if (score > best) { best = score; bi = v; }
             }

@@ -32,7 +32,8 @@ class ImgEncoder(nn.Module):
 
 class QstEncoder(nn.Module):
     def __init__(self, qst_vocab_size, word_embed_size, embed_size, num_layers, hidden_size, deterministic=True,
-                 temperature=0.1, max_length=30, beam_size=1, end_token=None, length_penalty=0.0):
+                 temperature=0.1, max_length=30, beam_size=1, end_token=None, length_penalty=0.0,
+                 top_k=0, top_p=1.0):
         super().__init__()
         self.hidden_size = hidden_size
         self.deterministic = deterministic
@@ -41,6 +42,8 @@ class QstEncoder(nn.Module):
         self.beam_size = beam_size          # > 1: deterministic decoding by beam search; generate() returns the best beam
         self.end_token = end_token          # set (<end> = 3): words after it are <pad> = 0, and the decode stops early
         self.length_penalty = length_penalty    # beams with end_token: ranked by log-probability / length^length_penalty
+        self.top_k = top_k                  # sampling (deterministic=False) only: draw among the top_k most likely words (0: all)
+        self.top_p = top_p                  # sampling only: draw within the nucleus of probability top_p (1: all)
         self.word2vec = nn.Embedding(qst_vocab_size, word_embed_size)
         self.tanh = nn.Tanh()
         self.lstm = nn.LSTM(word_embed_size, hidden_size, num_layers)
@@ -83,7 +86,7 @@ class QstEncoder(nn.Module):
         batch = len(image_embedding)
         h0 = image_embedding.reshape(batch, self.hidden_size)
         qst = decode_question(h0, self.lstm, self.word2vec, self.fc2, self.max_length, self.deterministic, self.temperature,
-                              self.beam_size, self.end_token, self.length_penalty)
+                              self.beam_size, self.end_token, self.length_penalty, self.top_k, self.top_p)
         if qst is not None:
             return qst
         # sampled decoding outside the kernel's envelope: the reference's module loop (torch.multinomial)
@@ -158,6 +161,6 @@ class VqaModel(nn.Module):
         twin.img_encoder.darts = self.img_encoder.darts.new()
         _copy_dropout(self, twin)
         # the unrolled twin generates ArchitectLct's pseudo questions: it decodes the way this model was configured to
-        for name in ("deterministic", "temperature", "max_length", "beam_size", "end_token", "length_penalty"):
+        for name in ("deterministic", "temperature", "max_length", "beam_size", "end_token", "length_penalty", "top_k", "top_p"):
             setattr(twin.qst_encoder, name, getattr(self.qst_encoder, name))
         return twin.to(config.DEVICE)

@@ -104,7 +104,7 @@ DECODE_GREEDY, DECODE_SAMPLED, DECODE_BEAM = 0, 1, 2         # pcd_decode_args.m
 
 class DecodeArgs(C.Structure):
     _fields_ = [(n, i32) for n in ("mode", "T", "B", "K", "H", "E", "V", "start_token", "stop", "end_token", "pad_token")] + \
-        [("length_penalty", f32), ("temperature", f32), ("row_offset", i32)] + \
+        [("length_penalty", f32), ("temperature", f32), ("row_offset", i32), ("truncate", i32), ("top_k", i32), ("top_p", f32)] + \
         [(n, vp) for n in ("seed", "emb", "w_ih", "w_hh", "b_ih", "b_hh", "h0", "c0", "w_out", "b_out", "tokens", "scores",
                            "work")]
 

@@ -7,6 +7,7 @@ enqueues on torch's current stream.
 """
 import ctypes as C
 import math
+import numbers
 
 import torch
 
@@ -1009,16 +1010,32 @@ def _check_envelope(what, h0, lstm, word2vec, proj):
                            f"{word2vec.embedding_dim} is outside the decode kernel's envelope (PCD_ERR_UNSUPPORTED)")
 
 
-def _decode(mode, h0, lstm, word2vec, proj, max_length, start_token, K=1, temperature=1.0, seed=None, stop=None):
+def _decode_truncation(V, top_k, top_p):
+    """(top_k, top_p as fp32) of a truncated sampled decode, None for the defaults (top_k = 0, top_p = 1: no truncation).
+    ValueError for a top_k that is not a non-negative integer or a top_p outside (0, 1]."""
+    if isinstance(top_k, bool) or not isinstance(top_k, numbers.Integral) or top_k < 0:
+        raise ValueError(f"decode_sample: top_k must be a non-negative integer (0: no limit), got {top_k!r}")
+    p32 = C.c_float(float(top_p)).value                 # what the kernel compares against
+    if not math.isfinite(p32) or not 0.0 < p32 <= 1.0:
+        raise ValueError(f"decode_sample: top_p must lie in (0, 1], got {top_p!r}")
+    if top_k == 0 and p32 == 1.0:
+        return None
+    return min(int(top_k), V), p32                      # any top_k >= V keeps every word
+
+
+def _decode(mode, h0, lstm, word2vec, proj, max_length, start_token, K=1, temperature=1.0, seed=None, stop=None,
+            truncation=None):
     """One pcd_decode per slice of floor(64 / K) items (the kernel takes 64 rows; row_offset = the slice's first item), each
     with its own outputs and workspace.  Returns (tokens, scores): tokens (B, max_length) and scores None, or for beams
-    tokens (B, K, max_length) and scores (B, K).  The arguments are validated by the caller; stop: _decode_stop's tuple."""
+    tokens (B, K, max_length) and scores (B, K).  The arguments are validated by the caller; stop: _decode_stop's tuple,
+    truncation: _decode_truncation's."""
     lib = N.lib_for(h0)
     V, E = word2vec.weight.shape
     beam = mode == N.DECODE_BEAM
     ops = [_f32c(t) for t in (word2vec.weight, lstm.weight_ih_l0, lstm.weight_hh_l0, lstm.bias_ih_l0, lstm.bias_hh_l0)]
     wout, bout = _f32c(proj.weight), _f32c(proj.bias)
     end_token, pad_token, length_penalty = stop or (0, 0, 0.0)
+    top_k, top_p = truncation or (0, 1.0)
     per = _LSTM_BATCH // K
     tokens, scores = [], []
     for b0 in range(0, max(h0.shape[0], 1), per):       # an empty batch reaches the kernel, which rejects it
@@ -1028,7 +1045,8 @@ def _decode(mode, h0, lstm, word2vec, proj, max_length, start_token, K=1, temper
         sc = torch.empty((B, K), dtype=torch.float32, device=h0.device) if beam else None
         a = N.DecodeArgs(mode=mode, T=max_length, B=B, K=K, H=H, E=E, V=V, start_token=start_token, stop=stop is not None,
                          end_token=end_token, pad_token=pad_token, length_penalty=length_penalty, temperature=temperature,
-                         row_offset=b0, seed=N.ptr(seed), emb=N.ptr(ops[0]), w_ih=N.ptr(ops[1]), w_hh=N.ptr(ops[2]),
+                         row_offset=b0, truncate=truncation is not None, top_k=top_k, top_p=top_p, seed=N.ptr(seed),
+                         emb=N.ptr(ops[0]), w_ih=N.ptr(ops[1]), w_hh=N.ptr(ops[2]),
                          b_ih=N.ptr(ops[3]), b_hh=N.ptr(ops[4]), h0=N.ptr(h0c), c0=N.ptr(h0c), w_out=N.ptr(wout),
                          b_out=N.ptr(bout), tokens=N.ptr(tok), scores=N.ptr(sc))
         work = torch.empty(int(lib.pcd_decode_work_floats(C.byref(a))), dtype=torch.float32, device=h0.device)
@@ -1052,9 +1070,16 @@ def decode_greedy(h0, lstm, word2vec, proj, max_length, start_token=2, end_token
     return _decode(N.DECODE_GREEDY, h0, lstm, word2vec, proj, max_length, start_token, stop=stop)[0]
 
 
-def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None, end_token=None, pad_token=0):
+def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token=2, seed=None, end_token=None, pad_token=0,
+                  top_k=0, top_p=1.0):
     """tokens (B, max_length) int64 of the sampled decode (QstEncoder.sample with deterministic=False): every word is drawn from
     softmax(logits / temperature), by the Gumbel-max trick on counter-based Philox noise (pcd_decode in sampled mode).
+
+    top_k > 0 draws only among the top_k most likely words, top_p < 1 only among the smallest set of most likely words whose
+    probability reaches top_p (the nucleus, taken within the top-k words when both are set): the distribution is
+    softmax(logits / temperature) restricted to that set and renormalised, with the same noise (pcd_decode with truncate = 1;
+    pcdarts_sm100.h states the rule exactly).  The defaults keep every word and run the untruncated kernel.  Truncation has
+    no stock loop: outside the decode kernel's envelope it raises, even with allow_stock_ops(True).
 
     seed: None draws one 64-bit seed per call on h0's device from torch's generator (so torch.manual_seed reproduces a run, and
     a call captured in a CUDA graph draws a fresh seed on every replay); a Python int, or a 1-element int64 tensor on h0's
@@ -1065,7 +1090,8 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
     if not math.isfinite(t32) or t32 <= 0.0:
         raise ValueError(f"decode_sample: temperature must be finite and > 0, got {temperature}")
     stop = _decode_stop(proj.out_features, end_token, pad_token)
-    if stop is not None:
+    truncation = _decode_truncation(proj.out_features, top_k, top_p)
+    if stop is not None or truncation is not None:
         _check_envelope("decode_sample", h0, lstm, word2vec, proj)
     if seed is None:
         seed = torch.empty(1, dtype=torch.int64, device=h0.device).random_(-2 ** 63, None)
@@ -1075,7 +1101,7 @@ def decode_sample(h0, lstm, word2vec, proj, max_length, temperature, start_token
     elif seed.dtype != torch.int64 or seed.numel() != 1 or seed.device != h0.device:
         raise ValueError("decode_sample: seed must be an int or a 1-element int64 tensor on the device of h0")
     return _decode(N.DECODE_SAMPLED, h0, lstm, word2vec, proj, max_length, start_token, temperature=t32, seed=seed,
-                   stop=stop)[0]
+                   stop=stop, truncation=truncation)[0]
 
 
 _MAX_BEAM = 8
@@ -1102,12 +1128,17 @@ def decode_beam(h0, lstm, word2vec, proj, max_length, beam_size, start_token=2, 
     return _decode(N.DECODE_BEAM, h0, lstm, word2vec, proj, max_length, start_token, K=int(beam_size), stop=stop)
 
 
-def decode_question(h0, lstm, word2vec, proj, max_length, deterministic, temperature, beam_size, end_token, length_penalty):
+def decode_question(h0, lstm, word2vec, proj, max_length, deterministic, temperature, beam_size, end_token, length_penalty,
+                    top_k=0, top_p=1.0):
     """QstEncoder.generate's decode policy: tokens (B, max_length) of the best beam (beam_size > 1), of the greedy decode
-    (`deterministic` truthy) or of the sampled one (`deterministic is False`), all on the decode kernel.  None when the
-    caller's stock loop decodes: sampled decoding outside the kernel's envelope, any other falsy `deterministic` (an
-    overridden sample()), and greedy decoding outside the envelope once allow_stock_ops(True) lets it.  Beam search and
-    end-of-sequence decoding have no stock loop: outside the envelope they raise, even with allow_stock_ops(True)."""
+    (`deterministic` truthy) or of the sampled one (`deterministic is False`, truncated by top_k / top_p), all on the decode
+    kernel.  None when the caller's stock loop decodes: sampled decoding outside the kernel's envelope, any other falsy
+    `deterministic` (an overridden sample()), and greedy decoding outside the envelope once allow_stock_ops(True) lets it.
+    Beam search, end-of-sequence decoding and top-k / nucleus truncation have no stock loop: outside the envelope they raise,
+    even with allow_stock_ops(True)."""
+    truncated = top_k != 0 or top_p != 1.0
+    if truncated and deterministic is not False:
+        raise ValueError(f"top_k = {top_k!r} / top_p = {top_p!r} need deterministic=False (they truncate sampling)")
     if beam_size > 1:
         if not deterministic:
             raise ValueError(f"beam_size = {beam_size} needs deterministic=True (beam search is not sampled)")
@@ -1117,9 +1148,10 @@ def decode_question(h0, lstm, word2vec, proj, max_length, deterministic, tempera
     stop = end_token is not None
     if deterministic and (stop or decode_supported(h0, lstm, word2vec, proj)):
         return decode_greedy(h0, lstm, word2vec, proj, max_length, end_token=end_token)
-    if deterministic is False and (stop or decode_supported(h0, lstm, word2vec, proj)):
+    if deterministic is False and (stop or truncated or decode_supported(h0, lstm, word2vec, proj)):
         # words drawn from softmax(logits / temperature) by Gumbel-max on a seed from torch's generator
-        return decode_sample(h0, lstm, word2vec, proj, max_length, temperature, end_token=end_token)
+        return decode_sample(h0, lstm, word2vec, proj, max_length, temperature, end_token=end_token, top_k=top_k,
+                             top_p=top_p)
     if deterministic:            # greedy decode outside the kernel's envelope: loud unless stock ops were opted in
         _stock(f"greedy decode with hidden size {h0.shape[1]}")
     return None
